@@ -5,6 +5,10 @@ adjoint + regulariser pullback, gradient all-reduce, Adam) on synthetic data.
 
     python bench.py --gpus N --steps K --warmup W            # this repo (libLRNDE.so)
     python bench.py --impl reference --gpus N --steps K ...  # CPU restatement of the reference
+    python bench.py --steps K --dump-outputs DIR             # also write the last timed step's results as DIR/*.npy
+
+The native arms load libLRNDE.so as `python -c 'import __graft_entry__ as g; g.build()'` left it and write
+nothing into the tree.
 
 Metric (BASELINE.json): MNIST neural-ODE train samples/s (+ NFE/s).  Workload: the
 "mnist_ode batch-scaling sweep" config at 8192 samples per GPU (weak scaling: 8192 x N, i.e.
@@ -28,6 +32,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark runs from the tree build() left, which may be read-only: no __pycache__
 
 D, H, NCLS = 784, 100, 10
 TOL = 1.4e-8
@@ -171,9 +176,32 @@ def workload_config(args, n):
 
 
 # ---------------------------------------------------------------------------------- this repo
-def _native_loop(pkg, torch, dist, args, B, world, rank, dev, ctx, steps, warmup, e2e_steps):
+DUMP_BYTES = 64 * 10**6     # cap on what --dump-outputs writes in all
+
+
+def dump_outputs(path, outputs, per_sample):
+    """Writes every entry of `outputs` as path/<name>.npy: tensors in float32, Python numbers as float64 scalars.  The
+    arrays named in `per_sample` carry one row per sample; when everything together would exceed DUMP_BYTES, they are
+    cut to a fixed seeded choice of rows (the same rows in every run with the same batch size)."""
+    import torch
+    arrs = {k: v.detach().float() if isinstance(v, torch.Tensor) else np.float64(v) for k, v in outputs.items()}
+    fixed = 128 * len(arrs) + sum(4 * v.numel() if isinstance(v, torch.Tensor) else v.nbytes   # 128: .npy header
+                                  for k, v in arrs.items() if k not in per_sample)
+    n = arrs[per_sample[0]].shape[0]
+    rows = min(n, (DUMP_BYTES - fixed) // sum(4 * arrs[k][0].numel() for k in per_sample))
+    if rows < n:
+        pick = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, rows, replace=False)))
+        for k in per_sample:
+            arrs[k] = arrs[k].index_select(0, pick.to(arrs[k].device))
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrs.items():
+        np.save(os.path.join(path, k + ".npy"), v.cpu().numpy() if isinstance(v, torch.Tensor) else v)
+
+
+def _native_loop(pkg, torch, dist, args, B, world, rank, dev, ctx, steps, warmup, e2e_steps, keep_step=None):
     """The training iteration at batch B per GPU: returns (ms per step device-resident, ms per step through host
-    buffers, info of the last step, kernel launches inside the timed region, nfe sum)."""
+    buffers, info of the last step, kernel launches inside the timed region, nfe sum).  keep_step: index of the
+    device-resident step whose results are returned under "outputs" (u(t2), gradients, updated parameters, loss)."""
     lib = pkg.lib()
     chk = pkg._lib.check
     chain = pkg.TDChain(pkg.Chain(pkg.Dense(D, H, "tanh"), pkg.Dense(H, D)))
@@ -210,6 +238,7 @@ def _native_loop(pkg, torch, dist, args, B, world, rank, dev, ctx, steps, warmup
     loss = C.c_float()
     launches = {"n": 0}
     info = {}
+    kept = {}
     # host side of the e2e leg: page-locked buffers, as a host application (the Julia caller) would keep
     hb = {"ps": pin((P,)), "Wc": pin((Wc.numel(),)), "dps": pin((P,)), "dwc": pin((Wc.numel(),))}
     hb["ps"].copy_(ps)
@@ -242,6 +271,9 @@ def _native_loop(pkg, torch, dist, args, B, world, rank, dev, ctx, steps, warmup
             adam(i, d_ps, d_Wc)
             fs, bs = sol.stats, sol.bwd_stats
             nfe, reg, retcode = st2["nfe"], float(st2["reg_val"]), sol.retcode
+            if i == keep_step:       # u_last, d_x and d_ps are fresh per step; d_Wc, ps and Wc are rewritten in place
+                kept.update(u_final=u_last, d_x=d_x.t(), d_ps=d_ps, d_wc=d_Wc.clone(), ps=ps.clone(), wc=Wc.clone(),
+                            loss=float(loss.value), reg_val=reg, nfe=float(nfe))
             sol.free()
         else:
             # t1 is host-sampled exactly as the layer functor does (neural_ode.jl:69-71)
@@ -345,14 +377,13 @@ def _native_loop(pkg, torch, dist, args, B, world, rank, dev, ctx, steps, warmup
     h2d = 4 * (B * D + B + P + PW) + 4 * (P + PW)            # x, labels, ps, Wc in; the host gradients back up for the optimiser
     d2h = 4 * (P + PW + 1) + 4 * (P + PW)                    # d_ps, d_Wc, loss out; the updated parameters
     return dict(ms=ms_total / steps, ms_total=ms_total, ms_e2e=ms_e, info=fwd_info, e2e_info=e2e_info, launches=n_launch, nfe_sum=nfe_sum,
-                per_step_ms=per_step_ms,
+                per_step_ms=per_step_ms, outputs=kept,
                 h2d=h2d, d2h=d2h, node=node, chain=chain, ps=ps, xb=xb, P=P)
 
 
 def run_native(args):
     import torch
     import __graft_entry__ as entry
-    entry.build()
     pkg = entry.load_package()
     lib = pkg.lib()
     chk = pkg._lib.check
@@ -387,8 +418,13 @@ def run_native(args):
         clocks.start()         # before the warm-up: nvidia-smi's own start-up (~1 s of driver calls) must not
                                # land inside the timed region; it keeps sampling every 200 ms through it
     e2e_steps = max(0, min(args.steps, args.e2e_steps))
-    r = _native_loop(pkg, torch, dist, args, B, world, rank, dev, ctx, args.steps, args.warmup, e2e_steps)
-    clk = clocks.stop() if rank == 0 else None
+    try:
+        r = _native_loop(pkg, torch, dist, args, B, world, rank, dev, ctx, args.steps, args.warmup, e2e_steps,
+                         keep_step=args.warmup + args.steps - 1 if args.dump_outputs else None)
+    finally:                   # the nvidia-smi sampler must not outlive a failed run
+        clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r["outputs"], per_sample=("u_final", "d_x"))
     ms, ms_e, fwd_info = r["ms"], r["ms_e2e"], r["info"]
     value = B * world / (ms / 1e3)
     e2e = {"value": B * world / (ms_e / 1e3), "unit": "samples/s", "h2d_bytes_per_step": r["h2d"],
@@ -540,7 +576,6 @@ def sde_setup(B, use_oracle):
         ps = np.concatenate([orc.glorot_uniform_params(od, rng), orc.glorot_uniform_params(og, rng)])
     else:
         import __graft_entry__ as entry
-        entry.build()
         pkg = entry.load_package()
         layer = pkg.NeuralDSDE(pkg.Chain(pkg.Dense(Ds, Hs, "tanh"), pkg.Dense(Hs, Ds)), pkg.Chain(pkg.Dense(Ds, Ds)), **kw)
         ps = layer.initialparameters(rng)
@@ -712,7 +747,6 @@ def run_physionet(args):
         return
     import torch
     import __graft_entry__ as entry
-    entry.build()
     pkg = entry.load_package()
     dev = torch.device("cuda", 0)
     cell = pkg.LatentGRUCell(S["in_dim"], S["H"], S["Lg"])
@@ -803,7 +837,6 @@ def cifar10_setup(B, use_oracle, W=32, loop_mode=0):
         D = net.state_dims
     else:
         import __graft_entry__ as entry
-        entry.build()
         pkg = entry.load_package()
         chain = pkg.TDConvChain(pkg.ConvChain(pkg.Conv(8, 64, True, "gelu"), pkg.Conv(64, 64, True, "gelu"),
                                               pkg.Conv(64, 8), width=W, height=W))
@@ -1018,7 +1051,14 @@ def main():
     ap.add_argument("--sde-batch", type=int, default=128)
     ap.add_argument("--cifar-batch", type=int, default=256)
     ap.add_argument("--cifar-ref-batch", type=int, default=4, help="bounded sample for the CPU oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (u(t2) and d_x per sample, "
+                         "d_ps, d_wc, the updated ps and wc, loss, reg_val, nfe) as DIR/<name>.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "mnist_ode" or args.impl != "native"):
+        ap.error("--dump-outputs covers the default workload (--workload mnist_ode --impl native)")
     if args.workload == "mnist_sde":
         run_sde(args)
     elif args.workload == "physionet":

@@ -98,7 +98,7 @@ def build(name):
     t1_index = 1 if kw.get("regularize") == "biased" else None
     sol, st2, aux, cots, d_x, d_ps = _run(model, kw, seed, name, x, ps, cots_in, d_reg, np.float32, t1_index)
     # Float64 twin: the size of the Float32 rounding noise in every compared quantity
-    sol64, st64, aux64, _, d_x64, d_ps64 = _run(model, kw, seed, name, x, ps, cots_in, d_reg, np.float64, t1_index)
+    _, st64, aux64, _, d_x64, d_ps64 = _run(model, kw, seed, name, x, ps, cots_in, d_reg, np.float64, t1_index)
     s = aux["sol"]
     s64 = aux64["sol"]
     log64 = np.array([(t, dt, e, a) for (t, dt, e, a) in s64.step_log], dtype=np.float64)
@@ -114,7 +114,6 @@ def build(name):
         t1=np.float32(aux.get("t1", 0.0)), dt_reg=np.float32(aux.get("dt_reg", 0.0)),
         step_log64=log64, reg_val64=np.float64(st64["reg_val"]),
         n_bwd64=np.int64(len(aux64["bsol"].step_log)),
-        u_last64=np.asarray(sol64.u[-1], np.float64), d_x64=d_x64.astype(np.float64),
         d_ps_rel64=np.float64(np.abs(d_ps64 - d_ps).max() / np.abs(d_ps64).max()),
         d_x_rel64=np.float64(np.abs(d_x64 - d_x).max() / (np.abs(d_x64).max() + 1e-300)),
     )

@@ -48,28 +48,7 @@ def rel(a, b):
     return float(np.abs(a - b).max() / (np.abs(b).max() + 1e-30))
 
 
-# ------------------------------------------------------------------ f(u, p, t)
-@pytest.mark.parametrize("prec", PRECS_SMALL)
-@pytest.mark.parametrize("layers,td,input_act,B", [
-    ([(2, 4, "gelu"), (4, 2, "identity")], True, None, 1),
-    ([(3, 5, "tanh"), (5, 3, "tanh")], False, "tanh", 7),
-    ([(20, 40, "tanh"), (40, 20, "tanh"), (20, 40, "sigmoid"), (40, 20, "relu")], True, None, 130),
-    ([(784, 100, "tanh"), (100, 784, "identity")], True, None, 128),
-    ([(784, 100, "tanh"), (100, 784, "identity")], True, None, 77),
-    ([(33, 70, "gelu"), (70, 33, "identity")], True, None, 65),
-])
-def test_dynamics_matches_oracle(pkg, prec, layers, td, input_act, B):
-    if prec == "smem" and layers[0][0] > 256:
-        pytest.skip("the mnist network (158 K parameters) does not fit shared memory: tcgen05 path only")
-    rng = np.random.default_rng(0)
-    om = _omodel(layers, td, input_act)
-    ps = orc.glorot_uniform_params(om, rng) + (0.05 * rng.standard_normal(om.nparams)).astype(np.float32)
-    x = rng.standard_normal((layers[0][0], B)).astype(np.float32)
-    layer = pkg.NeuralODE(_chain(pkg, layers, td, input_act), precision=prec)
-    got = layer.dynamics(x, ps, 0.37)
-    want = om.f(x, ps, np.float32(0.37))
-    assert got.shape == want.shape
-    assert rel(got, want) < 2e-5, rel(got, want)
+# f(u, p, t) and its pullback, call by call against Float64: tests/test_gpu_dense_rhs.py
 
 
 def _check_controller_replay(pkg, t, dt, eest, acc, t0, tend, stops, maxiters):

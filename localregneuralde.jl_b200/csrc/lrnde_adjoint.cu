@@ -50,12 +50,86 @@ __device__ __forceinline__ void act_pair(float x, float& h, float& s) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// (0) interpolant kernel: c_j = C_n + dt_n sum_i b_i(theta_j) H(k_i), the dense interpolant of the forward solution in
+// hidden space at every stage time of the attempt, written as the stored copy of c_j (rows Kaug, Kaug + 1 = tau_j, 1,
+// the rest 0).  It does not depend on lambda, so it runs ahead of the chain kernel over the whole batch, and the
+// stages that fall in the same forward interval share one read of that interval's 8 tape arrays.
+// Thread = 4 hidden rows of one sample (a warp reads one sample's row of 512 bytes).
+// ---------------------------------------------------------------------------------------------------------
+struct AInterpP {
+  SolveDev* S;
+  int single;            // 1: c_1 of the current state (time / interpolant yint[0])
+  float* ws;
+  size_t zlen;
+  int B, Kaug, nunit;    // nunit = padded samples x LR_ZROW / 4
+};
+
+__global__ void __launch_bounds__(256) adj_interp_kernel(AInterpP p) {
+  SolveDev* S = p.S;
+  if (p.single ? S->failed : S->done) return;
+  __shared__ float s_cf[6][8], s_sc[6][8], s_tau[6];
+  __shared__ const float* s_hb[6];
+  __shared__ float* s_dst[6];
+  const int nst = p.single ? 1 : 6;
+  if (threadIdx.x < nst) {
+    const int j = threadIdx.x;
+    const LinComb& yd = S->yint[p.single ? 0 : j + 1];
+    const size_t slotn = (size_t)(yd.base - S->ftape) / ((size_t)7 * S->flen);
+    s_hb[j] = S->fhtape + slotn * 7 * S->fzlen;
+    for (int s = 0; s < 8; ++s) {
+      s_cf[j][s] = (s < 7) ? yd.coef[s] : 1.0f;
+      s_sc[j][s] = (s < 7) ? 1.0f : yd.scale;
+    }
+    s_tau[j] = yd.t;
+    const int slot = S->slot, next = (S->slot + 1) % S->cap;
+    const int arr = p.single ? LA_S1 + 3 * slot + 2 : (j == 5 ? LA_S1 + 3 * next + 2 : LA_CC + j);
+    s_dst[j] = p.ws + (size_t)arr * p.zlen;
+  }
+  __syncthreads();
+  const int u = blockIdx.x * blockDim.x + threadIdx.x;
+  if (u >= p.nunit) return;
+  const int b = u / (LR_ZROW / 4), r0 = (u % (LR_ZROW / 4)) * 4;
+  const size_t e = (size_t)b * LR_ZROW + r0;
+  const bool any = (b < p.B) && (r0 < p.Kaug);
+  float4 tp[8];
+  const float* cur = nullptr;
+  for (int j = 0; j < nst; ++j) {
+    if (any && s_hb[j] != cur) {   // tiles in the order the coefficients take them: H(k_1..7), then C_n
+      cur = s_hb[j];
+#pragma unroll
+      for (int s = 0; s < 8; ++s) {
+        const float* src = (s == 7) ? cur : cur + (size_t)(s < 6 ? s + 1 : 8) * S->fzlen;   // H(k_7) = H(k_1) of the next slot
+        tp[s] = __ldcg(reinterpret_cast<const float4*>(src + e));
+      }
+    }
+    float c[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+    if (any) {
+#pragma unroll
+      for (int s = 0; s < 8; ++s) {
+        const float cf = s_cf[j][s], sc = s_sc[j][s];
+        c[0] = fmaf(cf, tp[s].x, __fmul_rn(sc, c[0]));
+        c[1] = fmaf(cf, tp[s].y, __fmul_rn(sc, c[1]));
+        c[2] = fmaf(cf, tp[s].z, __fmul_rn(sc, c[2]));
+        c[3] = fmaf(cf, tp[s].w, __fmul_rn(sc, c[3]));
+      }
+    }
+    float o[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int r = r0 + k;
+      o[k] = (r < p.Kaug) ? c[k] : ((r == p.Kaug) ? s_tau[j] : ((r == p.Kaug + 1) ? 1.0f : 0.0f));
+    }
+    *reinterpret_cast<float4*>(s_dst[j] + e) = make_float4(o[0], o[1], o[2], o[3]);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // (1) chain kernel: one CTA = 64 samples as two independent halves of 32 (while the tensor core works for one half
 // the other half's warps do their element-wise arithmetic).  Thread of a compute warp = one hidden row x 16 samples.
 // TMEM: [Mz hi | Mz lo | Mh^T hi | Mh^T lo] as A operands (8 KS columns each), then one 32-column accumulator per half
-// (p = Mz c first, Mh^T eps once p has been read).
+// (p = Mz c first, Mh^T eps once p has been read).  c_j comes from adj_interp_kernel's stored copy.
 // ---------------------------------------------------------------------------------------------------------
-constexpr int kTapeBufs = 3;                       // ring of [64 samples][LR_ZROW] tiles of the forward hidden tape
+constexpr int kTapeBufs = 3;                       // ring of [64 samples][LR_ZROW] tiles of c_j
 constexpr int kTapeBufBytes = kNT * LR_ZROW * 4;   // 32 KB
 struct AChainP {
   SolveDev* S;
@@ -111,9 +185,6 @@ __global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
   __shared__ uint32_t tmem_slot;
   __shared__ LinComb sd[6], sy[7];
   __shared__ float s_bt[7];
-  __shared__ const float* s_fh;
-  __shared__ const float* s_ftape;
-  __shared__ size_t s_flen, s_fzlen;
   __shared__ int s_slot, s_next;
 
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
@@ -136,7 +207,6 @@ __global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
       mbar_init(&xdone[c], 1u);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    s_fh = S->fhtape; s_ftape = S->ftape; s_flen = S->flen; s_fzlen = S->fzlen;
     s_slot = S->slot; s_next = (S->slot + 1) % S->cap;
   }
   if (threadIdx.x >= 64 && threadIdx.x < 70) sd[threadIdx.x - 64] = S->st[threadIdx.x - 64];
@@ -157,26 +227,20 @@ __global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
   if (tr) ATRACE(0, 0);
 
   if (warp == 0) {
-    // ---------------- forward hidden tape in: per stage the 7 H(k_i) tiles then the C_n tile of the interval that
-    // holds the stage time, bulk-copied onto a ring (the interpolant does not depend on lambda: it runs ahead)
+    // ---------------- c_j in: the stored copy adj_interp_kernel wrote, one tile per stage, bulk-copied onto a ring
+    // (it does not depend on lambda: it runs ahead)
     {
       const int nvalid = min(kNT, p.B - n0);
       const uint32_t bytes = (uint32_t)nvalid * LR_ZROW * 4u;
-      int it = 0;
-      for (int jj = 0; jj < nst; ++jj) {
-        const LinComb& yd = SINGLE ? sy[0] : sy[jj + 1];
-        const size_t slotn = (size_t)(yd.base - s_ftape) / ((size_t)7 * s_flen);
-        const float* hb = s_fh + slotn * 7 * s_fzlen;
-        for (int s = 0; s < 8; ++s, ++it) {
-          const int b = it % kTapeBufs;
-          const float* src = (s == 7) ? hb : hb + (size_t)(s < 6 ? s + 1 : 8) * s_fzlen;   // H(k_7) = H(k_1) of the next slot
-          mbar_wait(&tempty[b], (uint32_t)(((it / kTapeBufs) & 1) ^ 1));
-          if (elect_one_sync()) {
-            mbar_arrive_expect_tx(&tfull[b], bytes);
-            bulk_g2s(tbuf + (size_t)b * kTapeBufBytes, src + (size_t)n0 * LR_ZROW, bytes, &tfull[b]);
-          }
-          __syncwarp();
+      for (int it = 0; it < nst; ++it) {
+        const int b = it % kTapeBufs;
+        const float* src = SINGLE ? arr(LA_S1 + 3 * s_slot + 2) : (it == 5 ? arr(LA_S1 + 3 * s_next + 2) : arr(LA_CC + it));
+        mbar_wait(&tempty[b], (uint32_t)(((it / kTapeBufs) & 1) ^ 1));
+        if (elect_one_sync()) {
+          mbar_arrive_expect_tx(&tfull[b], bytes);
+          bulk_g2s(tbuf + (size_t)b * kTapeBufBytes, src + (size_t)n0 * LR_ZROW, bytes, &tfull[b]);
         }
+        __syncwarp();
       }
     }
     // ---------------- Delta_b / Delta_bt operand images out (units of 16 samples for the lambda GEMM)
@@ -318,7 +382,7 @@ __global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
     const size_t e0 = (size_t)nb * LR_ZROW + hrow;
     uint8_t* const tCc = tC[cg];
     uint8_t* const tEc = tE[cg];
-    const float* tape_row = reinterpret_cast<const float*>(tbuf) + (cg * 32 + rbase) * LR_ZROW + hrow;
+    const float* ring_row = reinterpret_cast<const float*>(tbuf) + (cg * 32 + rbase) * LR_ZROW + hrow;
 
     float c[16], ep[16], dprev[16];
 #pragma unroll
@@ -330,22 +394,27 @@ __global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
     }
     float v[16], ss[16];
     // software pipeline: iteration jj runs the front of stage jj (operand tiles), then the lambda-independent part of
-    // stage jj + 1 (interpolant c from the tape ring, known part of eps) while the tensor core works, then the back of
-    // stage jj (p, activation, alpha, delta).  jj = -1 only prefetches.
+    // stage jj + 1 (known part of eps) while the tensor core works, then the back of stage jj (p, activation, alpha,
+    // delta).  jj = -1 only prefetches.
     for (int jj = -1; jj < nst; ++jj) {
       const LinComb& yd = SINGLE ? sy[0] : sy[jj < 0 ? 1 : jj + 1];
       const float tau = yd.t;
       const bool last = (!SINGLE && jj == 5);
       float* dst_del = SINGLE ? arr(LA_S1 + 3 * slot + 0) : (last ? arr(LA_S1 + 3 * next + 0) : arr(LA_DEL + max(jj, 0)));
       float* dst_hh = SINGLE ? arr(LA_S1 + 3 * slot + 1) : (last ? arr(LA_S1 + 3 * next + 1) : arr(LA_HH + max(jj, 0)));
-      float* dst_cc = SINGLE ? arr(LA_S1 + 3 * slot + 2) : (last ? arr(LA_S1 + 3 * next + 2) : arr(LA_CC + max(jj, 0)));
       if (jj >= 0) {
         if (tr) ATRACE(1, jj);
-        // ---- operand tiles: c_j (rows Kaug, Kaug + 1 of the stored copy = tau_j, 1) and
-        //      eps_j = (partial sum prefetched during the previous stage) + a_{j,j-1} delta_{j-1}
-        const float cextra = (hrow == p.Kaug) ? tau : ((hrow == p.Kaug + 1) ? 1.0f : 0.0f);
+        // ---- operand tiles: c_j (dense interpolant of the forward solution in hidden space, adj_interp_kernel) from
+        //      the ring, and eps_j = (partial sum prefetched during the previous stage) + a_{j,j-1} delta_{j-1}
+        {
+          const int b = jj % kTapeBufs;
+          mbar_wait(&tfull[b], (uint32_t)((jj / kTapeBufs) & 1));
+          const float* tb = ring_row + (size_t)b * (kTapeBufBytes / 4);
 #pragma unroll
-        for (int i = 0; i < 16; ++i) dst_cc[e0 + (size_t)i * LR_ZROW] = rowc ? c[i] : cextra;
+          for (int i = 0; i < 16; ++i) c[i] = rowc ? tb[i * LR_ZROW] : 0.0f;
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&tempty[b]);
+        }
         tile_put16(tCc, c);
         if (!SINGLE) {
           const float cl = sd[jj].coef[jj];
@@ -361,24 +430,6 @@ __global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
         if (tr) ATRACE(2, jj);
       }
       if (jj + 1 < nst) {
-        // ---- c_{j+1} = C_n + dt_n sum_i b_i(theta) H(k_i): dense interpolant of the forward solution in hidden space,
-        //      from the tape ring (the 7 H(k_i) tiles, then the C_n tile)
-        const LinComb& yn = SINGLE ? sy[0] : sy[jj + 2];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) c[i] = 0.0f;
-        for (int s = 0; s < 8; ++s) {
-          const int it = (jj + 1) * 8 + s;
-          const int b = it % kTapeBufs;
-          mbar_wait(&tfull[b], (uint32_t)((it / kTapeBufs) & 1));
-          if (rowc) {
-            const float* tb = tape_row + (size_t)b * (kTapeBufBytes / 4);
-            const float cf = (s < 7) ? yn.coef[s] : 1.0f, sc = (s < 7) ? 1.0f : yn.scale;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) c[i] = fmaf(cf, tb[i * LR_ZROW], sc * c[i]);
-          }
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&tempty[b]);
-        }
         if (!SINGLE && jj >= 0) {   // known part of eps_{j+1}: delta_1 .. delta_j (the newest one is in registers)
 #pragma unroll
           for (int i = 0; i < 16; ++i) ep[i] = sd[jj + 1].coef[jj] * dprev[i];
@@ -1019,6 +1070,11 @@ static void lra_launch_chain(LatentAdjoint& E, SolveDev* S, int single) {
   cp.passes = E.passes;
   const size_t smem_c = 4 * ((size_t)sh.nfull * 8192 + (size_t)sh.ntail * 2048) + ladj::kTapeBufs * ladj::kTapeBufBytes + 1024;
   cudaStream_t st = E.ctx->stream;
+  ladj::AInterpP ip;
+  ip.S = S; ip.single = single; ip.ws = E.ws; ip.zlen = E.zlen; ip.B = (int)E.B; ip.Kaug = sh.Kaug;
+  ip.nunit = E.ntiles * fused::kNT * (LR_ZROW / 4);
+  ladj::adj_interp_kernel<<<(ip.nunit + 255) / 256, 256, 0, st>>>(ip);
+  LRA_COUNT(E.ctx);
 #define LRA_CHAIN(A) do { if (single) ladj::adj_chain_kernel<A, true><<<E.ntiles, fused::kThreads, smem_c, st>>>(cp); \
                          else ladj::adj_chain_kernel<A, false><<<E.ntiles, fused::kThreads, smem_c, st>>>(cp); } while (0)
   switch (sh.act) {

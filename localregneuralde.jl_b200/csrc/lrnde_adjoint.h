@@ -12,7 +12,9 @@
 //   mu block          mu' = -J_p^T lambda:  sum_j w_j dW1_j = Delta_w x^T + (sum_j w_j delta_j c_j^T) W2a^T,
 //                     sum_j w_j dW2a_j = lambda_n (sum_j w_j [h_j;tau_j;1])^T - dt W1^T (sum_j w_j eps_j [h_j;tau_j;1]^T)
 // so an attempt touches D-dimensional data only to read lambda_n and x and to write lambda_{n+1}:
-//   (1) adj_chain_kernel   the six stages in hidden space (tcgen05, Mz / Mh^T as TMEM A operands)
+//   (0) adj_interp_kernel  c_j of the six stages from the forward hidden tape (lambda-independent: one pass over the
+//                          whole batch, one read of each forward interval's tape per attempt), stored for (1) and (3)
+//   (1) adj_chain_kernel   the six stages in hidden space (tcgen05, Mz / Mh^T as TMEM A operands; c_j from (0))
 //   (2) kgemm_kernel<2,1>  [W1^T Delta_b, W1^T Delta_bt] with the lambda_{n+1} / residual epilogue (lrnde_fused.cu)
 //   (3) pairacc_kernel     every batch contraction of the mu block (tcgen05, MN-major operands, split over the batch)
 //   (4) adj_reduce_kernel + adj_mu_kernel   fixed-order reduction, mu_{n+1}, residual of the mu block
@@ -50,8 +52,8 @@ struct LatentAdjoint {
   void prepare(const float* mz_plain = nullptr);
   // stage-1 quantities (delta_1, [h_1;t;1], c_1) of the current state from alpha_in and S->yint[0]
   void begin(SolveDev* S);
-  // one Tsit5 attempt of the adjoint from the descriptors of S (st, yint, err): launches (1) - (4)
+  // one Tsit5 attempt of the adjoint from the descriptors of S (st, yint, err): launches (0) - (4)
   void attempt(SolveDev* S);
-  // profiling: the launches of attempt() one by one (0 chain, 1 lambda GEMM, 2 pairacc, 3 reduce + mu)
+  // profiling: the launches of attempt() one by one (0 interpolant + chain, 1 lambda GEMM, 2 pairacc, 3 reduce + mu)
   void attempt_part(SolveDev* S, int which);
 };

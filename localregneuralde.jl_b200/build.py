@@ -3,8 +3,8 @@
     python localregneuralde.jl_b200/build.py [--force]
 
 The CUDA library is the product; the host-check library only re-exports the scalar
-step-size logic of csrc/lrnde_controller.h so the CPU test-suite can pin it bit-for-bit
-against the oracle without a GPU.
+step-size logic of csrc/lrnde_controller.h and the save plan of csrc/lrnde_saveplan.h so
+the CPU test-suite can pin them against the oracle without a GPU.
 """
 from __future__ import annotations
 

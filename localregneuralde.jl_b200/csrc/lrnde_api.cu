@@ -25,8 +25,7 @@
 #include "lrnde_fused.h"
 #include "lrnde_adjoint.h"
 #include "lrnde_regrev.cuh"
-
-static bool lr_reg_hidden_eligible(const lrnde_model* m, int reg_type);
+#include "lrnde_saveplan.h"
 
 // ------------------------------------------------------------------------------------------
 // errors
@@ -736,6 +735,92 @@ struct ConvEval {
 };
 
 // ------------------------------------------------------------------------------------------
+// Engine route of one call: which engines evaluate f, its pullback and the regulariser's reverse pass.  lr_ode_route
+// decides it once per call and is the only reader of LRNDE_NO_FUSED, LRNDE_NO_SMEM, LRNDE_NO_LATENT_ADJ,
+// LRNDE_FULL_TAPE and LRNDE_NO_HIDDEN_REG; a kept tape stores the route of its forward call and the pullback follows it.
+// The shared-memory engine is sized for the reverse pass (small_smem_bytes(bwd = true)) even without a pullback, so a
+// forward and its pullback agree on small and umma.  lean => latent_adj => fused => umma; umma excludes small.
+// ------------------------------------------------------------------------------------------
+struct OdeRoute {
+  bool conv = false;        // conv dynamics: ConvEval, which keeps its own switches
+  bool small = false;       // the shared-memory engine (lrnde_smem_mlp.cuh): the whole network in one launch
+  bool umma = false;        // per-layer tcgen05 kernels, else FP32 SIMT
+  bool fused = false;       // forward attempts on FusedEngine; an MlpEval built for pullbacks (vjp) does not use it
+  bool latent_adj = false;  // the pullback runs on LatentAdjoint: the forward keeps its hidden tape
+  bool lean = false;        // the forward does not store k_2..k_6 (saves and the pullback read the hidden tape)
+  bool reg_hidden = false;  // the regulariser's reverse pass runs in hidden space (lrnde_regrev.cuh)
+  bool fused_model = false; // FusedEngine accepts the model at this precision (whether or not the call runs it)
+  int passes = 3;           // tf32 hi/lo products of the tensor-core engines: 1 = single-pass TF32
+};
+
+// Shared-memory engine: the padded network (twice, for the reverse pass) and the tile buffers must fit one SM.  Fills
+// *net and returns the samples per tile, 0 when the network does not fit.
+static int lr_small_tile(lrnde_ctx* ctx, const lrnde_model* m, int64_t B, SdeNet* net) {
+  if ((int)m->layers.size() > SDE_MAXL) return 0;
+  SdeNet& snet = *net;
+  memset(&snet, 0, sizeof(snet));
+  snet.nl = (int)m->layers.size(); snet.td = m->td; snet.D = m->D; snet.nparams = (int)m->nparams;
+  int woff = 0, hoff = 0, md = m->D;
+  for (int l = 0; l < snet.nl; ++l) {
+    const LayerInfo& L = m->layers[l];
+    snet.in[l] = L.in; snet.out[l] = L.out; snet.outp[l] = (L.out + 3) & ~3; snet.act[l] = L.act;
+    snet.ps_w[l] = L.w_off; snet.ps_b[l] = L.b_off;
+    snet.w_off[l] = woff; woff += (L.in + m->td + 1) * snet.outp[l];
+    snet.hid_off[l] = hoff; hoff += snet.outp[l];
+    md = std::max(md, std::max(L.in, snet.outp[l]));
+  }
+  snet.wfloats = woff; snet.hid_rows = hoff; snet.maxdim = md;
+  int n_sm = 0;
+  size_t smem_optin = 0;
+  sde_device_limits(ctx->device, &n_sm, &smem_optin);
+  int S = 32;
+  while (S > 8 && ((B + S - 1) / S) < n_sm / 2) S >>= 1;
+  for (;; S >>= 1) {
+    if (small_smem_bytes(snet, m->D, S + 1, true) + 2048 <= smem_optin) return S;   // 2 KB of static shared memory
+    if (S <= 4) return 0;
+  }
+}
+
+// Hidden-space reverse pass of the regulariser step (lrnde_regrev.cuh): 2-layer TD-MLP with tanh,
+// regularize_type = :error_estimate
+static bool lr_reg_hidden_eligible(const lrnde_model* m, int reg_type) {
+  FusedShape sh;
+  if (reg_type != LRNDE_REGTYPE_ERROR || !lrf_shape(m, &sh)) return false;
+  if (m->layers.size() != 2 || m->layers[0].act != ACT_TANH || m->layers[1].act != ACT_IDENTITY) return false;
+  if (m->input_act != ACT_IDENTITY) return false;
+  const LayerInfo &L1 = m->layers[0], &L2 = m->layers[1];
+  // the layer blocks must be [weight | bias] back to back (ComponentArray order), D a multiple of 4 (16-byte rows)
+  if (L1.b_off != L1.w_off + (int64_t)L1.out * (L1.in + m->td) || L2.b_off != L2.w_off + (int64_t)L2.out * (L2.in + m->td)) return false;
+  return sh.D % 4 == 0 && sh.H % 4 == 0 && sh.Kaug + m->td + 1 <= 104;
+}
+
+// o == NULL: precision 0 (auto), no tape
+static OdeRoute lr_ode_route(lrnde_ctx* ctx, const lrnde_model* m, const lrnde_opts* o, int64_t B) {
+  OdeRoute r;
+  if (!m->conv.empty()) { r.conv = true; return r; }
+  const int prec = o ? o->precision : LRNDE_PREC_AUTO;
+  const bool keep_tape = o && o->keep_tape;
+  r.passes = (prec == LRNDE_PREC_TF32) ? 1 : 3;
+  // LRNDE_PREC_SMEM asks for the shared-memory engine; LRNDE_PREC_AUTO picks it for batches the per-layer tcgen05
+  // kernels cannot fill (their cost is per-CTA latency, ~25 us per layer launch)
+  if (prec == LRNDE_PREC_SMEM || prec == LRNDE_PREC_AUTO) {
+    const bool want = (prec == LRNDE_PREC_SMEM);
+    if (want && (int)m->layers.size() > SDE_MAXL) lr_fail(LRNDE_EINVAL, "precision smem: at most %d layers", SDE_MAXL);
+    SdeNet net;
+    const bool fits = lr_small_tile(ctx, m, B, &net) > 0;
+    if (want && !fits) lr_fail(LRNDE_EINVAL, "precision smem: the network does not fit shared memory");
+    r.small = fits && (want || (B <= 4096 && !getenv("LRNDE_NO_SMEM")));
+  }
+  r.umma = prec != LRNDE_PREC_FP32_SIMT && !r.small;
+  r.fused_model = prec != LRNDE_PREC_FP32_SIMT && FusedEngine::eligible(m);
+  r.fused = r.fused_model && r.umma && !getenv("LRNDE_NO_FUSED");
+  r.latent_adj = r.fused && keep_tape && LatentAdjoint::eligible(m) && !getenv("LRNDE_NO_LATENT_ADJ");
+  r.lean = r.latent_adj && !getenv("LRNDE_FULL_TAPE");
+  r.reg_hidden = r.fused && keep_tape && lr_reg_hidden_eligible(m, o->reg_type) && !getenv("LRNDE_NO_HIDDEN_REG");
+  return r;
+}
+
+// ------------------------------------------------------------------------------------------
 // MLP evaluator: f(u, ps, t) and its VJP as sequences of kernels reading device descriptors
 // ------------------------------------------------------------------------------------------
 struct MlpEval {
@@ -743,7 +828,6 @@ struct MlpEval {
   const lrnde_model* m;
   const float* ps;
   int64_t B;
-  int prec;
   bool with_vjp;
   std::vector<float*> act;  // act[l]: [out_l x B]
   std::vector<float*> pre;  // pre[l]: [out_l x B] (vjp only)
@@ -771,22 +855,22 @@ struct MlpEval {
   std::vector<int> wS, wChunk;    // SIMT weight-gradient split
   std::vector<int> uS, uChunk;    // tcgen05 weight-gradient split (0 = layer not eligible)
 
-  MlpEval(lrnde_ctx* c, const lrnde_model* mm, const float* p, int64_t b, int precision, bool vjp)
-      : ctx(c), m(mm), ps(p), B(b), prec(precision), with_vjp(vjp) {
-    if (!m->conv.empty()) {
+  // vjp: the evaluator of a pullback, which never runs the fused forward (route.fused is ignored)
+  MlpEval(lrnde_ctx* c, const lrnde_model* mm, const float* p, int64_t b, const OdeRoute& route, bool vjp)
+      : ctx(c), m(mm), ps(p), B(b), with_vjp(vjp) {
+    if (route.conv) {
       conv = std::make_unique<ConvEval>(c, mm, p, b, vjp);
       return;
     }
     const int L = (int)m->layers.size();
-    use_umma = (precision != LRNDE_PREC_FP32_SIMT);
-    setup_small(precision);
-    if (use_small) use_umma = false;
+    use_umma = route.umma;
+    if (route.small) setup_small();
     use_cluster = (getenv("LRNDE_NO_CLUSTER") == nullptr);
     if (const char* e = getenv("LRNDE_NACC")) nacc_max = std::max(1, std::min(8, atoi(e)));
     use_lean = (getenv("LRNDE_NO_LEAN") == nullptr);
     use_wide = (getenv("LRNDE_NO_WIDE") == nullptr);
-    passes = (precision == LRNDE_PREC_TF32) ? 1 : 3;
-    if (use_umma && !vjp && FusedEngine::eligible(m) && !getenv("LRNDE_NO_FUSED")) {
+    passes = route.passes;
+    if (route.fused && !vjp) {
       fe = std::make_unique<FusedEngine>(ctx, m, ps, B, passes);
       packW1x = (float*)ctx->alloc(sizeof(float) * 2 * umma::kAChunkFloats * umma::kReplicas *
                                    (size_t)tiles_m(m->layers[0].out) * chunks_k(m->layers[0].in));
@@ -858,38 +942,12 @@ struct MlpEval {
     ctx->release(packW1x);
   }
 
-  // once per call: transposed weights for the data-gradient GEMMs, and (tcgen05 path) the
-  // tf32 hi/lo shared-memory images of every weight matrix
-  // Eligibility of the shared-memory engine: the padded network (twice, for the reverse pass) and the tile
-  // buffers fit one SM.  LRNDE_PREC_SMEM asks for it explicitly; LRNDE_PREC_AUTO picks it for batches the
-  // per-layer tcgen05 kernels cannot fill (their cost is per-CTA latency, ~25 us per layer launch).
-  void setup_small(int precision) {
-    use_small = false;
-    if (precision != LRNDE_PREC_SMEM && precision != LRNDE_PREC_AUTO) return;
-    const bool want = (precision == LRNDE_PREC_SMEM);
-    if ((int)m->layers.size() > SDE_MAXL) { if (want) lr_fail(LRNDE_EINVAL, "precision smem: at most %d layers", SDE_MAXL); return; }
-    memset(&snet, 0, sizeof(snet));
-    snet.nl = (int)m->layers.size(); snet.td = m->td; snet.D = m->D; snet.nparams = (int)m->nparams;
-    int woff = 0, hoff = 0, md = m->D;
-    for (int l = 0; l < snet.nl; ++l) {
-      const LayerInfo& L = m->layers[l];
-      snet.in[l] = L.in; snet.out[l] = L.out; snet.outp[l] = (L.out + 3) & ~3; snet.act[l] = L.act;
-      snet.ps_w[l] = L.w_off; snet.ps_b[l] = L.b_off;
-      snet.w_off[l] = woff; woff += (L.in + m->td + 1) * snet.outp[l];
-      snet.hid_off[l] = hoff; hoff += snet.outp[l];
-      md = std::max(md, std::max(L.in, snet.outp[l]));
-    }
-    snet.wfloats = woff; snet.hid_rows = hoff; snet.maxdim = md;
+  // the shared-memory engine's network image, tile size and grid (the route chose it, so lr_small_tile fits)
+  void setup_small() {
     int n_sm = 0;
     size_t smem_optin = 0;
     sde_device_limits(ctx->device, &n_sm, &smem_optin);
-    int S = 32;
-    while (S > 8 && ((B + S - 1) / S) < n_sm / 2) S >>= 1;
-    for (;; S >>= 1) {
-      if (small_smem_bytes(snet, m->D, S + 1, true) + 2048 <= smem_optin) break;   // 2 KB of static shared memory
-      if (S <= 4) { if (want) lr_fail(LRNDE_EINVAL, "precision smem: the network does not fit shared memory"); return; }
-    }
-    if (!want && (B > 4096 || getenv("LRNDE_NO_SMEM"))) return;
+    const int S = lr_small_tile(ctx, m, B, &snet);
     use_small = true;
     sS = S;
     const int ntiles = (int)((B + S - 1) / S);
@@ -911,6 +969,8 @@ struct MlpEval {
     return q;
   }
 
+  // once per call: transposed weights for the data-gradient GEMMs, and (tcgen05 path) the
+  // tf32 hi/lo shared-memory images of every weight matrix
   void prepare() {
     if (conv) { conv->prepare(); return; }
     if (use_small) return;
@@ -1511,15 +1571,12 @@ struct lrnde_tape {
   float* ps = nullptr;  // device copy of the parameters the forward used
   float* bn_state = nullptr;  // conv dynamics: device copy of st.model the forward normalised with (testmode)
   float* Mz = nullptr;        // latent-space engines: W1 W2a of the parameters the forward used ([128][128])
-  int reg_hidden = 0;         // the regulariser integrator kept its hidden images: its reverse pass runs in hidden space
+  OdeRoute route;             // the engines of the forward call; its pullback runs on the same ones
   std::unique_ptr<Solver> fwd;
   std::unique_ptr<Solver> reg;  // regulariser integrator (2-slot ring), reg modes only
   std::vector<float> fts;       // host copy of accepted times
-  std::vector<float> save_ts;   // times of the FULL saved solution (incl. t1 when appended)
-  std::vector<int> save_out;    // index of the output block for each save_ts entry, -1 if dropped
+  SavePlan saves;               // the saved solution of the forward call, t1
   int reg_mode = 0;
-  int lean = 0;                 // lean tape: k_2..k_6 of the forward steps were not stored (latent-space adjoint only)
-  float t1 = 0.f;
   // step logs (host copies)
   std::vector<float> log_t[2], log_dt[2], log_eest[2];
   std::vector<unsigned char> log_acc[2];
@@ -1641,10 +1698,6 @@ static void lr_grow_tape(Solver& S) {
   LR_CUDA(cudaMemcpyAsync(&S.dev->cap, &S.h.cap, sizeof(int), cudaMemcpyHostToDevice, st));
 }
 
-// forward declaration: y(t) of the kept forward solution (defined after lr_host_interp)
-static void lr_sol_at(lrnde_ctx* ctx, lrnde_tape* T, FusedEngine* fe, float tq, float* dst, LinComb* host_desc,
-                      const LinComb* dev_desc);
-
 static size_t lr_tape_budget(lrnde_ctx* ctx) {
   if (ctx->tape_budget) return (size_t)ctx->tape_budget;
   // cudaMemGetInfo takes a driver lock (measured 0.08 ... 60 ms per call on a shared host), so the
@@ -1695,8 +1748,9 @@ static LinComb lr_host_interp(const Solver& F, const std::vector<float>& fts, fl
 }
 
 // y(t) of the forward solution into dst (device): the stored state on an exact hit, else the dense interpolant --
-// from the D-dimensional tape, or (lean tape) from the hidden tape: y(t) = x + W2a c(t) (FusedEngine::dense_output)
-static void lr_sol_at(lrnde_ctx* ctx, lrnde_tape* T, FusedEngine* fe, float tq, float* dst, LinComb* host_desc,
+// from the D-dimensional tape, or (lean tape, lean_fe: an engine of the forward's model) from the hidden tape:
+// y(t) = x + W2a c(t) (FusedEngine::dense_output)
+static void lr_sol_at(lrnde_ctx* ctx, lrnde_tape* T, FusedEngine* lean_fe, float tq, float* dst, LinComb* host_desc,
                       const LinComb* dev_desc) {
   Solver& F = *T->fwd;
   cudaStream_t st = ctx->stream;
@@ -1704,14 +1758,13 @@ static void lr_sol_at(lrnde_ctx* ctx, lrnde_tape* T, FusedEngine* fe, float tq, 
   *host_desc = lr_host_interp(F, T->fts, tq);
   host_desc->dst = dst;
   LR_CUDA(cudaMemcpyAsync((void*)dev_desc, host_desc, sizeof(LinComb), cudaMemcpyHostToDevice, st));
-  if (T->lean && host_desc->n > 0) {
-    if (!fe) lr_fail(LRNDE_ESTATE, "lean tape without the latent-space engine");
+  if (lean_fe && host_desc->n > 0) {
     const size_t n = (size_t)(host_desc->base - F.tape) / ((size_t)7 * DB);
     const size_t zl = F.h.zlen;
     const float* harr[8];
     for (int i = 0; i < 7; ++i) harr[i] = F.htape + (n * 7 + i) * zl;
     harr[7] = F.htape + ((n + 1) * 7 + 1) * zl;
-    fe->dense_output(F.dev, harr, host_desc->coef, host_desc->scale, F.tape, dev_desc);
+    lean_fe->dense_output(F.dev, harr, host_desc->coef, host_desc->scale, F.tape, dev_desc);
   } else {
     lincomb_kernel<<<lr_ew_blocks(DB), 256, 0, st>>>(dev_desc, dst, DB, nullptr);
     LR_COUNT(ctx);
@@ -1737,6 +1790,32 @@ struct DevBuf {  // pooled device scratch with RAII
   DevBuf(lrnde_ctx* c, size_t nfloat) : ctx(c), p((float*)c->alloc(sizeof(float) * nfloat)) {}
   ~DevBuf() { ctx->release(p); }
 };
+
+// The returned blocks of the saved solution into u_save (may be NULL) and their times into save_times (host, may be
+// NULL).  u_save is a HOST pointer when the forward call had host_buffers.
+static void lr_write_saves(lrnde_ctx* ctx, lrnde_tape* T, FusedEngine* lean_fe, float* u_save, float* save_times) {
+  const SavePlan& plan = T->saves;
+  for (size_t i = 0; i < plan.times.size(); ++i)
+    if (plan.out[i] >= 0 && save_times) save_times[plan.out[i]] = plan.times[i];
+  if (!u_save || plan.nout == 0) return;
+  cudaStream_t st = ctx->stream;
+  const size_t DB = T->fwd->h.len;
+  const int host = T->opts.host_buffers;
+  DevBuf dd(ctx, (size_t)plan.nout * (sizeof(LinComb) / 4 + 1)), stage(ctx, host ? DB : 1);
+  for (size_t i = 0; i < plan.times.size(); ++i) {
+    const int blk = plan.out[i];
+    if (blk < 0) continue;
+    LinComb hd;
+    float* dst = host ? stage.p : u_save + (size_t)blk * DB;
+    lr_sol_at(ctx, T, lean_fe, std::min(plan.times[i], T->fts.back()), dst, &hd, (const LinComb*)dd.p + blk);
+    if (host) {
+      LR_CUDA(cudaMemcpyAsync(u_save + (size_t)blk * DB, dst, sizeof(float) * DB, cudaMemcpyDeviceToHost, st));
+      LR_CUDA(cudaStreamSynchronize(st));   // stage is reused by the next block
+    }
+  }
+  LR_CHECK_LAUNCH();
+  LR_CUDA(cudaStreamSynchronize(st));
+}
 
 // ------------------------------------------------------------------------------------------
 // f(u, ps, t) once (parity hook)
@@ -1764,7 +1843,7 @@ extern "C" int lrnde_dynamics_eval(lrnde_ctx* ctx, const lrnde_model* m, const l
   memset(&d, 0, sizeof(d));
   d.base = ud; d.t = t; d.dst = outd;
   LR_CUDA(cudaMemcpyAsync(ddesc.p, &d, sizeof(d), cudaMemcpyHostToDevice, st));
-  MlpEval ev(ctx, m, psd, B, o ? o->precision : 0, false);
+  MlpEval ev(ctx, m, psd, B, lr_ode_route(ctx, m, o, B), false);
   ev.prepare();
   DevBuf dstate(ctx, ev.conv ? std::max<int64_t>(1, ev.conv->nstate) : 1);
   if (ev.conv) ev.conv->attach_state(o, dstate.p);
@@ -1813,7 +1892,7 @@ extern "C" int lrnde_dynamics_vjp(lrnde_ctx* ctx, const lrnde_model* m, const lr
   d[1].base = ld; d[1].t = t;
   LinComb* dd = (LinComb*)ddesc.p;
   LR_CUDA(cudaMemcpyAsync(dd, d, sizeof(d), cudaMemcpyHostToDevice, st));
-  MlpEval ev(ctx, m, psd, B, o ? o->precision : 0, true);
+  MlpEval ev(ctx, m, psd, B, lr_ode_route(ctx, m, o, B), true);
   ev.prepare();
   DevBuf dstate(ctx, ev.conv ? std::max<int64_t>(1, ev.conv->nstate) : 1);
   if (ev.conv) { ev.conv->attach_state(o, dstate.p); ev.conv->bn_update = false; }
@@ -1859,10 +1938,12 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
   LR_CUDA(cudaMemcpyAsync(T->ps, ps, sizeof(float) * P, in_kind, st));
   const bool timing = getenv("LRNDE_TIMING") != nullptr;
   const long tq0 = lr_now_us();
+  T->route = lr_ode_route(ctx, m, o, B);
+  const OdeRoute& route = T->route;
 
   // ---- dense tape
   size_t slot_bytes = sizeof(float) * 7 * DB;
-  if (FusedEngine::eligible(m) && o->precision != LRNDE_PREC_FP32_SIMT)   // latent (+ hidden) tape of the fused engine
+  if (route.fused_model)   // latent (+ hidden) tape of the fused engine
     slot_bytes += sizeof(float) * 7 * (size_t)LR_ZROW * (size_t)B * (o->keep_tape ? 2 : 1);
   size_t budget_slots = std::max<size_t>(3, lr_tape_budget(ctx) / slot_bytes);
   const long tq1 = lr_now_us();
@@ -1877,7 +1958,7 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
   const long tq2 = lr_now_us();
 
   const bool need_vjp = false;
-  MlpEval ev(ctx, m, T->ps, B, o->precision, need_vjp);
+  MlpEval ev(ctx, m, T->ps, B, route, need_vjp);
   if (ev.fe && o->keep_tape) {
     T->Mz = (float*)ctx->alloc(sizeof(float) * 128 * 128);
     ev.mz_plain_out = T->Mz;
@@ -1899,12 +1980,7 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
   const int write_z = o->keep_tape ? 1 : 0;
   // lean tape: when the pullback will run in hidden space nothing reads k_2..k_6 of the D-dimensional tape (saves and
   // the regulariser's start state come from the hidden tape: FusedEngine::dense_output), so they are not stored
-  const bool lean = fe && write_z && LatentAdjoint::eligible(m) && !getenv("LRNDE_NO_LATENT_ADJ") && !getenv("LRNDE_FULL_TAPE");
-  T->lean = lean ? 1 : 0;
-  if (fe) fe->lean = lean ? 1 : 0;
-  auto sol_at = [&](float tq, float* dst, LinComb* host_desc, const LinComb* dev_desc) {
-    lr_sol_at(ctx, T.get(), fe, tq, dst, host_desc, dev_desc);
-  };
+  if (fe) fe->lean = route.lean ? 1 : 0;
   if (fe) {
     F.enable_latent(fe->zlen(), write_z != 0);
     ev.latent_of(F.tape, F.ztape);
@@ -1951,73 +2027,14 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
   lr_copy_log(F, T.get(), 0);
   const float t_last = T->fts.back();
 
-  // ---- which times the returned solution holds (neural_ode.jl:102-116)
-  std::vector<float> times;      // full saved solution
-  std::vector<int> out_index;    // output block per entry, -1 = dropped (_CorrectedDESolution)
-  float t1 = o->t1;
+  // ---- which times the returned solution holds (neural_ode.jl:102-116), and their states
+  T->saves = lr_save_plan(*o, T->fts);
+  const float t1 = T->saves.t1;
   const int mode = o->reg_mode;
-  if (o->nsave > 0) {
-    for (int i = 0; i < o->nsave; ++i) times.push_back(o->saveat[i]);
-    if (o->save_start && std::find(times.begin(), times.end(), o->t0) == times.end())
-      times.insert(times.begin(), o->t0);
-    for (size_t i = 0; i < times.size(); ++i) out_index.push_back((int)i);
-    if (mode == LRNDE_REG_UNBIASED) { times.push_back(t1); out_index.push_back(-1); }
-  } else if (o->nsave == 0 && mode != LRNDE_REG_BIASED) {
-    // solve(...; saveat = [t1, t2] / [t2], save_start) : the reference splats save_start into solve (neural_ode.jl:51)
-    if (o->save_start) { times.push_back(o->t0); out_index.push_back(0); }
-    if (mode == LRNDE_REG_UNBIASED) { times.push_back(t1); out_index.push_back((int)out_index.size()); }
-    times.push_back(o->t2);
-    out_index.push_back((int)out_index.size());
-  } else {  // every accepted step (saveat = [] of the :biased path, or nsave == -1)
-    int start = o->save_start ? 0 : 1;
-    for (int n = start; n <= naccept; ++n) { times.push_back(T->fts[n]); out_index.push_back(n - start); }
-  }
-  if (mode == LRNDE_REG_BIASED) {  // t1 = rand(rng, sol.t[1:end-1])   (neural_ode.jl:92)
-    int ncand = (int)times.size() - 1;
-    if (ncand > 0) {
-      int idx = std::min(ncand - 1, std::max(0, (int)std::floor(o->u01 * (float)ncand)));
-      t1 = times[idx];
-    } else t1 = o->t0;
-  }
-  if (o->last_only) {   // fused diffeqsol_to_array (src/utils.jl:37): only sol.u[end] leaves the library
-    int last = -1, mx = -1;
-    for (size_t i = 0; i < out_index.size(); ++i)
-      if (out_index[i] > mx) { mx = out_index[i]; last = (int)i; }
-    for (size_t i = 0; i < out_index.size(); ++i) out_index[i] = ((int)i == last) ? 0 : -1;
-  }
-  int nout = 0;
-  for (int v : out_index) nout = std::max(nout, v + 1);
+  const int nout = T->saves.nout;
   if (u_save && nout > u_save_cap)
     lr_fail(LRNDE_EINVAL, "u_save holds %lld blocks but the solution has %d", (long long)u_save_cap, nout);
-
-  // ---- write the saved states
-  std::vector<LinComb> descs;
-  std::vector<float> desc_t;
-  std::vector<int> desc_out;
-  for (size_t i = 0; i < times.size(); ++i) {
-    if (out_index[i] < 0) continue;
-    float tq = std::min(times[i], t_last);
-    descs.push_back(LinComb());
-    desc_t.push_back(tq);
-    desc_out.push_back(out_index[i]);
-    if (save_times) save_times[out_index[i]] = times[i];
-  }
-  if (u_save && !descs.empty()) {
-    DevBuf dd(ctx, descs.size() * (sizeof(LinComb) / 4 + 1));
-    DevBuf stage(ctx, host ? DB * descs.size() : 1);
-    for (size_t i = 0; i < descs.size(); ++i) {
-      float* dst = host ? stage.p + i * DB : u_save + (size_t)desc_out[i] * DB;
-      sol_at(desc_t[i], dst, &descs[i], ((const LinComb*)dd.p) + i);
-      if (host)
-        LR_CUDA(cudaMemcpyAsync(u_save + (size_t)desc_out[i] * DB, dst, sizeof(float) * DB,
-                                cudaMemcpyDeviceToHost, st));
-    }
-    LR_CHECK_LAUNCH();
-    LR_CUDA(cudaStreamSynchronize(st));
-  }
-  T->save_ts = times;
-  T->save_out = out_index;
-  T->t1 = t1;
+  lr_write_saves(ctx, T.get(), route.lean ? fe : nullptr, u_save, save_times);
 
   const long t_saves = lr_now_us();
   // ---- local regulariser: integrator at t1 + one differentiable step (neural_ode.jl:75-78)
@@ -2029,13 +2046,11 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
     if (ctx->nranks > 1) R.h.total_len = F.h.total_len;
     R.init_ctrl(t1, o->t2, o->t2, o->maxiters, o->pow_mode, o->abstol, o->reltol);
     // hidden images [h_j ; t_j ; 1] of the regulariser's stages for the hidden-space reverse pass (lrnde_regrev.cuh)
-    const bool reg_hidden = fe && o->keep_tape && T->Mz && lr_reg_hidden_eligible(m, o->reg_type);
-    if (fe) R.enable_latent(fe->zlen(), reg_hidden);
-    T->reg_hidden = reg_hidden ? 1 : 0;
+    if (fe) R.enable_latent(fe->zlen(), route.reg_hidden);
     R.upload();
     LinComb u1;
     DevBuf dd(ctx, sizeof(LinComb) / 4 + 1);
-    sol_at(std::min(t1, t_last), R.tape, &u1, (const LinComb*)dd.p);
+    lr_sol_at(ctx, T.get(), route.lean ? fe : nullptr, std::min(t1, t_last), R.tape, &u1, (const LinComb*)dd.p);
     if (fe) fe->lean = 0;   // the regulariser integrator keeps k_2..k_6 (its reverse pass reads them)
     if (fe) {
       ev.latent_of(R.tape, R.ztape);
@@ -2094,26 +2109,11 @@ extern "C" int lrnde_ode_saved_states(lrnde_ctx* ctx, const lrnde_model* m, lrnd
   if (!ctx || !m || !T || !u_save) lr_fail(LRNDE_EINVAL, "lrnde_ode_saved_states: bad args");
   if (T->ctx != ctx || T->model != m) lr_fail(LRNDE_ESTATE, "tape belongs to another ctx/model");
   LR_CUDA(cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
-  const size_t DB = (size_t)m->D * T->B;
-  const int host = T->opts.host_buffers;
-  int nout = 0;
-  for (int v : T->save_out) nout = std::max(nout, v + 1);
-  if (nout > u_save_cap) lr_fail(LRNDE_EINVAL, "u_save holds %lld blocks but the solution has %d", (long long)u_save_cap, nout);
-  std::unique_ptr<FusedEngine> fe;
-  if (T->lean) fe = std::make_unique<FusedEngine>(ctx, m, T->ps, T->B, T->opts.precision == LRNDE_PREC_TF32 ? 1 : 3);
-  const float t_last = T->fts.back();
-  DevBuf dd(ctx, sizeof(LinComb) / 4 + 1), stage(ctx, host ? DB : 1);
-  for (size_t i = 0; i < T->save_ts.size(); ++i) {
-    if (T->save_out[i] < 0) continue;
-    LinComb hd;
-    float* dst = host ? stage.p : u_save + (size_t)T->save_out[i] * DB;
-    lr_sol_at(ctx, T, fe.get(), std::min(T->save_ts[i], t_last), dst, &hd, (const LinComb*)dd.p);
-    if (host) LR_CUDA(cudaMemcpyAsync(u_save + (size_t)T->save_out[i] * DB, dst, sizeof(float) * DB, cudaMemcpyDeviceToHost, st));
-    if (save_times) save_times[T->save_out[i]] = T->save_ts[i];
-    LR_CUDA(cudaStreamSynchronize(st));   // dd / stage are reused by the next block
-  }
-  LR_CHECK_LAUNCH();
+  if (T->saves.nout > u_save_cap)
+    lr_fail(LRNDE_EINVAL, "u_save holds %lld blocks but the solution has %d", (long long)u_save_cap, T->saves.nout);
+  std::unique_ptr<FusedEngine> lean_fe;
+  if (T->route.lean) lean_fe = std::make_unique<FusedEngine>(ctx, m, T->ps, T->B, T->route.passes);
+  lr_write_saves(ctx, T, lean_fe.get(), u_save, save_times);
   LR_API_END
 }
 
@@ -2155,22 +2155,35 @@ extern "C" int lrnde_profile_adjoint_last(float* us5) {
   return LRNDE_OK;
 }
 
+// the launches of the first attempt, repeated (same descriptors: the controller does not run; they only write the next
+// ring slot, which the real attempt recomputes), timed with CUDA events on the library's stream
+static void lr_profile_adjoint(lrnde_ctx* ctx, LatentAdjoint& la, SolveDev* A, int iters, bool timing) {
+  cudaStream_t st = ctx->stream;
+  cudaEvent_t e[6];
+  for (auto& ev_ : e) LR_CUDA(cudaEventCreate(&ev_));
+  for (int w = 0; w < 2; ++w) la.attempt(A);
+  for (int k = 0; k < 4; ++k) {
+    LR_CUDA(cudaEventRecord(e[k], st));
+    for (int i = 0; i < iters; ++i) la.attempt_part(A, k);
+  }
+  LR_CUDA(cudaEventRecord(e[4], st));
+  for (int i = 0; i < iters; ++i) la.attempt(A);
+  LR_CUDA(cudaEventRecord(e[5], st));
+  LR_CUDA(cudaEventSynchronize(e[5]));
+  const char* nm[5] = {"chain", "lambda gemm", "pairacc", "reduce + mu", "attempt"};
+  for (int k = 0; k < 5; ++k) {
+    float ms = 0.0f;
+    LR_CUDA(cudaEventElapsedTime(&ms, e[k], e[k + 1]));
+    g_adj_profile_us[k] = 1000.0f * ms / (float)iters;
+    if (timing) fprintf(stderr, "[lrnde] adjoint attempt: %-12s %8.1f us\n", nm[k], g_adj_profile_us[k]);
+  }
+  for (auto& ev_ : e) cudaEventDestroy(ev_);
+}
+
 // ------------------------------------------------------------------------------------------
 // Reverse pass of the regulariser step in hidden space (lrnde_regrev.cuh): 2-layer TD-MLP with tanh,
 // regularize_type = :error_estimate.  dps += d_reg * d reg_val / d ps.
 // ------------------------------------------------------------------------------------------
-static bool lr_reg_hidden_eligible(const lrnde_model* m, int reg_type) {
-  if (getenv("LRNDE_NO_HIDDEN_REG")) return false;
-  FusedShape sh;
-  if (reg_type != LRNDE_REGTYPE_ERROR || !lrf_shape(m, &sh)) return false;
-  if (m->layers.size() != 2 || m->layers[0].act != ACT_TANH || m->layers[1].act != ACT_IDENTITY) return false;
-  if (m->input_act != ACT_IDENTITY) return false;
-  const LayerInfo &L1 = m->layers[0], &L2 = m->layers[1];
-  // the layer blocks must be [weight | bias] back to back (ComponentArray order), D a multiple of 4 (16-byte rows)
-  if (L1.b_off != L1.w_off + (int64_t)L1.out * (L1.in + m->td) || L2.b_off != L2.w_off + (int64_t)L2.out * (L2.in + m->td)) return false;
-  return sh.D % 4 == 0 && sh.H % 4 == 0 && sh.Kaug + m->td + 1 <= 104;
-}
-
 static void lr_wgrad_launch(lrnde_ctx* ctx, const umma::WgOperand& P, const umma::WgOperand& Q, int transposed, int ldo, int64_t N,
                             float* part, size_t block, int nsplit, int chunk, int passes, const int* done) {
   static bool attr_set = false;
@@ -2287,6 +2300,40 @@ static void lr_reg_pullback_hidden(lrnde_ctx* ctx, const lrnde_model* m, lrnde_t
   LR_CUDA(cudaStreamSynchronize(st));   // the scratch buffers go back to the pool
 }
 
+// The same reverse pass through the per-layer pullback of f, stage by stage (any model and regularize_type)
+static void lr_reg_pullback_layers(lrnde_ctx* ctx, const lrnde_model* m, lrnde_tape* T, MlpEval& ev, float d_reg,
+                                   float* dps_dev) {
+  cudaStream_t st = ctx->stream;
+  Solver& R = *T->reg;
+  const size_t DB = (size_t)m->D * T->B;
+  DevBuf work(ctx, 9 * DB);
+  RegSeedP sp;
+  sp.R = R.dev; sp.reg_type = T->opts.reg_type; sp.d_reg = d_reg;
+  for (int k = 0; k < 6; ++k) sp.dk[k] = work.p + (size_t)k * DB;
+  sp.du = work.p + 6 * DB;
+  sp.dg6 = work.p + 7 * DB;
+  float* abuf = work.p + 8 * DB;
+  reg_seed_kernel<<<lr_ew_blocks(DB), 256, 0, st>>>(sp);
+  LR_COUNT(ctx);
+  std::vector<LinComb> lam(6);
+  for (int k = 0; k < 6; ++k) { memset(&lam[k], 0, sizeof(LinComb)); lam[k].base = sp.dk[k]; }
+  DevBuf dl(ctx, 6 * (sizeof(LinComb) / 4 + 1));
+  LR_CUDA(cudaMemcpyAsync(dl.p, lam.data(), sizeof(LinComb) * 6, cudaMemcpyHostToDevice, st));
+  const LinComb* lamd = (const LinComb*)dl.p;
+  for (int row = 5; row >= 0; --row) {
+    const LinComb* y = (row == 5) ? &R.dev->st[6] : &R.dev->st[row];
+    ev.vjp(y, lamd + row, abuf, nullptr, 1.0f, dps_dev, nullptr, 0, 1.0f, 1.0f, nullptr);
+    if (row == 0) break;  // k2's input depends on k1 only (constant)
+    RegBwdP bp;
+    bp.R = R.dev; bp.row = row; bp.a = abuf; bp.du = sp.du; bp.dg6 = sp.dg6;
+    for (int k = 0; k < 6; ++k) { bp.dk[k] = sp.dk[k]; bp.coef[k] = lr_tsit5_a(row, k); }
+    reg_bwd_stage_kernel<<<lr_ew_blocks(DB), 256, 0, st>>>(bp);
+    LR_COUNT(ctx);
+  }
+  LR_CHECK_LAUNCH();
+  LR_CUDA(cudaStreamSynchronize(st));
+}
+
 
 extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_tape* T,
                                   const float* d_u_save, float d_reg, float* d_ps, float* d_x,
@@ -2308,10 +2355,10 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
   Solver& F = *T->fwd;
   const int nsteps = (int)T->fts.size() - 1;
   const float t0 = T->fts.front(), t2 = T->fts.back();
+  const OdeRoute& route = T->route;
 
   // cotangent blocks on the device
-  int nout = 0;
-  for (int v : T->save_out) nout = std::max(nout, v + 1);
+  const int nout = T->saves.nout;
   DevBuf dstage(ctx, (host && d_u_save) ? DB * (size_t)std::max(nout, 1) : 1);
   const float* dU = d_u_save;
   if (host && d_u_save) {
@@ -2321,12 +2368,10 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
   auto cot_blocks = [&](float tval, std::vector<const float*>& out) {
     out.clear();
     if (!dU) return;
-    for (size_t i = 0; i < T->save_ts.size(); ++i)
-      if (T->save_out[i] >= 0 && std::min(T->save_ts[i], t2) == tval)
-        out.push_back(dU + (size_t)T->save_out[i] * DB);
+    for (int blk : T->saves.blocks_at(tval, t2)) out.push_back(dU + (size_t)blk * DB);
   };
 
-  MlpEval ev(ctx, m, T->ps, B, o.precision, true);
+  MlpEval ev(ctx, m, T->ps, B, route, true);
   ev.prepare();
   if (ev.conv && o.model_testmode) { ev.conv->bn_state = T->bn_state; ev.conv->testmode = 1; }
 
@@ -2359,9 +2404,7 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
     A.h.ftdir = 1;
     // latent-space adjoint (lrnde_adjoint.h): the forward solve kept its hidden tape
     std::unique_ptr<LatentAdjoint> la;
-    if (T->lean && getenv("LRNDE_NO_LATENT_ADJ"))
-      lr_fail(LRNDE_ESTATE, "the forward solve kept a lean tape (latent-space adjoint); set LRNDE_FULL_TAPE=1 for the forward to use the per-layer adjoint");
-    if (F.htape && ev.use_umma && LatentAdjoint::eligible(m) && !getenv("LRNDE_NO_LATENT_ADJ")) {
+    if (route.latent_adj) {
       la = std::make_unique<LatentAdjoint>(ctx, m, T->ps, B, ev.passes);
       la->W1T = ev.WT[0]; la->Zx = F.ztape; la->x = F.tape;
       la->prepare(T->Mz);
@@ -2386,20 +2429,14 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
       A.h.total_len = (unsigned long long)D * (unsigned long long)ctx->total_batch + P;
       A.enable_mu_exchange(P);
     }
-    // interior tstops: saved times strictly inside (t0, t2), descending, unique
-    std::vector<float> stops;
-    for (float s : T->save_ts) {
-      float sc = std::min(s, t2);
-      if (sc > t0 && sc < t2 && std::find(stops.begin(), stops.end(), sc) == stops.end()) stops.push_back(sc);
-    }
-    std::sort(stops.begin(), stops.end(), [](float a, float b) { return a > b; });
+    // tstops: the saved times strictly inside (t0, t2), descending, then t0
+    std::vector<float> stops = T->saves.interior_stops(t0, t2);
     stops.push_back(t0);
     A.init_ctrl(t2, t0, stops[0], o.maxiters, o.pow_mode, o.abstol, o.reltol);
     // lean tape: the per-layer right-hand side (initial-dt probes only) reads y(t) materialised from the hidden tape
     std::unique_ptr<FusedEngine> fe_y;
     std::unique_ptr<DevBuf> ybuf, ydescs;
-    if (T->lean) {
-      if (!la) lr_fail(LRNDE_ESTATE, "lean forward tape but the latent-space adjoint is not available for this call");
+    if (route.lean) {
       fe_y = std::make_unique<FusedEngine>(ctx, m, T->ps, B, ev.passes);
       ybuf = std::make_unique<DevBuf>(ctx, DB);
       ydescs = std::make_unique<DevBuf>(ctx, 2 * (sizeof(LinComb) / 4 + 1));
@@ -2409,7 +2446,7 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
       LR_CUDA(cudaMemcpyAsync(ydescs->p, &od, sizeof(LinComb), cudaMemcpyHostToDevice, st));
     }
     auto rhs = [&](const LinComb* in, const LinComb* y, const int* done, const LinComb*, bool) {
-      if (T->lean) {
+      if (route.lean) {
         LinComb* out_desc = (LinComb*)ydescs->p;       // {dst = ybuf}
         LinComb* y_mat = out_desc + 1;                 // {base = ybuf, t = y->t}, written on the device
         fe_y->dense_output_dev(A.dev, y, F.tape, ybuf->p, y_mat, out_desc);
@@ -2443,30 +2480,7 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
     if (la && A.muglob) LR_CUDA(cudaMemsetAsync(A.muglob, 0, sizeof(float) * P, st));
     if (la) latent_begin();
     mark("latent begin");
-    if (la && getenv("LRNDE_PROFILE_ADJ")) {
-      // the launches of the first attempt, repeated (same descriptors: the controller does not run; they only write
-      // the next ring slot, which the real attempt recomputes), timed with CUDA events on the library's stream
-      const int iters = std::max(1, atoi(getenv("LRNDE_PROFILE_ADJ")));
-      cudaEvent_t e[6];
-      for (auto& ev_ : e) LR_CUDA(cudaEventCreate(&ev_));
-      for (int w = 0; w < 2; ++w) la->attempt(A.dev);
-      for (int k = 0; k < 4; ++k) {
-        LR_CUDA(cudaEventRecord(e[k], st));
-        for (int i = 0; i < iters; ++i) la->attempt_part(A.dev, k);
-      }
-      LR_CUDA(cudaEventRecord(e[4], st));
-      for (int i = 0; i < iters; ++i) la->attempt(A.dev);
-      LR_CUDA(cudaEventRecord(e[5], st));
-      LR_CUDA(cudaEventSynchronize(e[5]));
-      const char* nm[5] = {"chain", "lambda gemm", "pairacc", "reduce + mu", "attempt"};
-      for (int k = 0; k < 5; ++k) {
-        float ms = 0.0f;
-        LR_CUDA(cudaEventElapsedTime(&ms, e[k], e[k + 1]));
-        g_adj_profile_us[k] = 1000.0f * ms / (float)iters;
-        if (timing) fprintf(stderr, "[lrnde] adjoint attempt: %-12s %8.1f us\n", nm[k], g_adj_profile_us[k]);
-      }
-      for (auto& ev_ : e) cudaEventDestroy(ev_);
-    }
+    if (la && getenv("LRNDE_PROFILE_ADJ")) lr_profile_adjoint(ctx, *la, A.dev, std::max(1, atoi(getenv("LRNDE_PROFILE_ADJ"))), timing);
     for (size_t si = 0; si < stops.size(); ++si) {
       A.run_segment();
       mark("segment");
@@ -2508,36 +2522,9 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
 
   const long tb_adj = lr_now_us();
   // ---- reverse pass of the regulariser step: gradient w.r.t. ps only
-  if (T->reg && d_reg != 0.0f && T->reg_hidden && ev.use_umma && !getenv("LRNDE_NO_HIDDEN_REG")) {
-    lr_reg_pullback_hidden(ctx, m, T, ev, d_reg, dps_dev);
-  } else if (T->reg && d_reg != 0.0f) {
-    Solver& R = *T->reg;
-    DevBuf work(ctx, 9 * DB);
-    RegSeedP sp;
-    sp.R = R.dev; sp.reg_type = o.reg_type; sp.d_reg = d_reg;
-    for (int k = 0; k < 6; ++k) sp.dk[k] = work.p + (size_t)k * DB;
-    sp.du = work.p + 6 * DB;
-    sp.dg6 = work.p + 7 * DB;
-    float* abuf = work.p + 8 * DB;
-    reg_seed_kernel<<<lr_ew_blocks(DB), 256, 0, st>>>(sp);
-    LR_COUNT(ctx);
-    std::vector<LinComb> lam(6);
-    for (int k = 0; k < 6; ++k) { memset(&lam[k], 0, sizeof(LinComb)); lam[k].base = sp.dk[k]; }
-    DevBuf dl(ctx, 6 * (sizeof(LinComb) / 4 + 1));
-    LR_CUDA(cudaMemcpyAsync(dl.p, lam.data(), sizeof(LinComb) * 6, cudaMemcpyHostToDevice, st));
-    const LinComb* lamd = (const LinComb*)dl.p;
-    for (int row = 5; row >= 0; --row) {
-      const LinComb* y = (row == 5) ? &R.dev->st[6] : &R.dev->st[row];
-      ev.vjp(y, lamd + row, abuf, nullptr, 1.0f, dps_dev, nullptr, 0, 1.0f, 1.0f, nullptr);
-      if (row == 0) break;  // k2's input depends on k1 only (constant)
-      RegBwdP bp;
-      bp.R = R.dev; bp.row = row; bp.a = abuf; bp.du = sp.du; bp.dg6 = sp.dg6;
-      for (int k = 0; k < 6; ++k) { bp.dk[k] = sp.dk[k]; bp.coef[k] = lr_tsit5_a(row, k); }
-      reg_bwd_stage_kernel<<<lr_ew_blocks(DB), 256, 0, st>>>(bp);
-      LR_COUNT(ctx);
-    }
-    LR_CHECK_LAUNCH();
-    LR_CUDA(cudaStreamSynchronize(st));
+  if (T->reg && d_reg != 0.0f) {
+    if (route.reg_hidden) lr_reg_pullback_hidden(ctx, m, T, ev, d_reg, dps_dev);
+    else lr_reg_pullback_layers(ctx, m, T, ev, d_reg, dps_dev);
   }
   if (host) {
     if (!no_dx) LR_CUDA(cudaMemcpyAsync(d_x, dx_dev, sizeof(float) * DB, cudaMemcpyDeviceToHost, st));
@@ -2570,14 +2557,15 @@ extern "C" int lrnde_profile_step(lrnde_ctx* ctx, const lrnde_model* m, const lr
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const size_t DB = (size_t)m->D * B;
-  MlpEval ev(ctx, m, ps, B, o->precision, false);
-  if (!ev.fe) lr_fail(LRNDE_EINVAL, "lrnde_profile_step: the model / precision does not use the latent-space engine");
+  const OdeRoute route = lr_ode_route(ctx, m, o, B);
+  if (!route.fused) lr_fail(LRNDE_EINVAL, "lrnde_profile_step: the model / precision does not use the latent-space engine");
+  MlpEval ev(ctx, m, ps, B, route, false);
   ev.prepare();
   Solver F(ctx, DB, DB, 3, 0, 8);
   F.init_ctrl(o->t0, o->t2, o->t2, o->maxiters, o->pow_mode, o->abstol, o->reltol);
   F.enable_latent(ev.fe->zlen(), o->keep_tape != 0);   // keep_tape: the training configuration (hidden tape, lean D-tape)
   if (F.htape) LR_CUDA(cudaMemsetAsync(F.htape, 0, sizeof(float) * ev.fe->zlen(), st));
-  ev.fe->lean = (o->keep_tape && LatentAdjoint::eligible(m) && !getenv("LRNDE_FULL_TAPE")) ? 1 : 0;
+  ev.fe->lean = route.lean ? 1 : 0;
   LR_CUDA(cudaMemcpyAsync(F.tape, x, sizeof(float) * DB, cudaMemcpyDeviceToDevice, st));
   F.h.use_cond = 0;
   F.upload();

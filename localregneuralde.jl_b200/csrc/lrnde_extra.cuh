@@ -154,8 +154,8 @@ extern "C" int lrnde_sosri_step(lrnde_ctx* ctx, const lrnde_model* drift,
   }
   LR_CUDA(cudaMemcpyAsync(descs.p, hd.data(), sizeof(LinComb) * 8, cudaMemcpyHostToDevice, st));
   const LinComb* dd = (const LinComb*)descs.p;
-  MlpEval evf(ctx, drift, psd.p, B, o->precision, false);
-  MlpEval evg(ctx, diffusion, psg.p, B, o->precision, false);
+  MlpEval evf(ctx, drift, psd.p, B, lr_ode_route(ctx, drift, o, B), false);
+  MlpEval evg(ctx, diffusion, psg.p, B, lr_ode_route(ctx, diffusion, o, B), false);
   evf.prepare();
   evg.prepare();
   for (int s = 0; s < 4; ++s) {
@@ -577,7 +577,7 @@ extern "C" int lrnde_profile_feval(lrnde_ctx* ctx, const lrnde_model* m, const l
     for (int i = 0; i < nsrc; ++i) { d.src[i] = srcs.p + (size_t)i * len; d.coef[i] = 0.1f * (float)(i + 1); }
   }
   LR_CUDA(cudaMemcpyAsync(ddesc.p, &d, sizeof(d), cudaMemcpyHostToDevice, st));
-  MlpEval ev(ctx, m, ps, B, o ? o->precision : 0, false);
+  MlpEval ev(ctx, m, ps, B, lr_ode_route(ctx, m, o, B), false);
   ev.prepare();
   // LRNDE_PROFILE_LAYERS=k: only the first k layers (k = 1 isolates the layer-1 kernel with the
   // stage combination in its operand prologue)

@@ -1,7 +1,9 @@
-// CPU build of the scalar step-size logic (lrnde_controller.h) for the no-GPU test-suite.
+// CPU build of the scalar step-size logic (lrnde_controller.h) and of the save plan
+// (lrnde_saveplan.h) for the no-GPU test-suite.
 // Not part of the product path: libLRNDE.so runs the same functions inside its controller
-// kernels; this library only lets pytest compare them bit-for-bit with the oracle.
+// kernels and its forward call; this library only lets pytest compare them with the oracle.
 #include "lrnde_controller.h"
+#include "lrnde_saveplan.h"
 
 extern "C" {
 
@@ -43,5 +45,21 @@ int lrhc_replay(float t0, float tend, const float* tstops, int nstops, float dt0
   }
   *retcode = c.retcode;
   return k;
+}
+
+// The save plan of a forward call (lrnde_saveplan.h) whose solve accepted the times fts[0..nfts-1].  Writes up to cap
+// times and output blocks, t1 and the number of output blocks; returns the number of times.
+int lrhc_save_plan(int reg_mode, float t0, float t2, float t1, float u01, const float* saveat, int nsave,
+                   int save_start, int last_only, const float* fts, int nfts, float* times, int* out, int cap,
+                   float* t1_out, int* nout) {
+  lrnde_opts o;
+  memset(&o, 0, sizeof(o));
+  o.reg_mode = reg_mode; o.t0 = t0; o.t2 = t2; o.t1 = t1; o.u01 = u01;
+  o.saveat = saveat; o.nsave = nsave; o.save_start = save_start; o.last_only = last_only;
+  const SavePlan p = lr_save_plan(o, std::vector<float>(fts, fts + nfts));
+  for (int i = 0; i < (int)p.times.size() && i < cap; ++i) { times[i] = p.times[i]; out[i] = p.out[i]; }
+  *t1_out = p.t1;
+  *nout = p.nout;
+  return (int)p.times.size();
 }
 }

@@ -1,6 +1,7 @@
 """CPU suite for the host side of libLRNDE: the scalar step-size logic that the device
 controller runs (csrc/lrnde_controller.h, re-exported by liblrnde_hostcheck.so) is pinned
-bit-for-bit against the oracle, the golden fixtures are re-derived from the oracle, and the
+bit-for-bit against the oracle, so is the save plan of a forward call (csrc/lrnde_saveplan.h),
+the golden fixtures are re-derived from the oracle, and the
 CUDA library loads and exports every symbol include/lrnde.h declares (no compute here)."""
 import ctypes as C
 import os
@@ -39,6 +40,9 @@ def hc():
     L.lrhc_replay.restype = i32
     L.lrhc_replay.argtypes = [f32, f32, C.c_void_p, i32, f32, f32, i32, i32, C.c_void_p, i32,
                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.lrhc_save_plan.restype = i32
+    L.lrhc_save_plan.argtypes = [i32, f32, f32, f32, f32, C.c_void_p, i32, i32, i32, C.c_void_p, i32,
+                                 C.c_void_p, C.c_void_p, i32, C.c_void_p, C.c_void_p]
     return L
 
 
@@ -159,6 +163,97 @@ def test_initdt_matches_oracle(hc):
                                float(dtmax), float(dtmin), tdir, None))
         # 10^x / log10 go through libm here and numpy's own kernels in the oracle: a few ulps
         assert abs(float(got) - float(want)) <= 2e-6 * abs(float(want)), (trial, got, want)
+
+
+# accepted times of a solve on tspan (0, 1): all the save plan reads of the solve
+_FTS = np.array([0.0, 0.05, 0.17, 0.4, 0.63, 0.9, 1.0], np.float32)
+
+
+def _fake_solution(fts=_FTS):
+    """An oracle ODESolution that accepted the steps fts (zero stages: interpolating it is cheap)."""
+    z = np.zeros((2, 1), np.float32)
+    n = len(fts) - 1
+    return orc.ODESolution(ts=list(fts), us=[z + np.float32(i) for i in range(n + 1)], ks=[[z] * 7] * n,
+                           dts=list(np.diff(fts)), step_log=[], nf=0, naccept=n, nreject=0, retcode=0, tdir=1,
+                           dtype=np.dtype(np.float32))
+
+
+def _solve_kwargs(saveat, save_start):
+    kw = {} if saveat is None else dict(saveat=saveat)
+    if save_start is not None:
+        kw["save_start"] = save_start
+    return kw
+
+
+def _oracle_forward(mode, saveat, save_start):
+    """The oracle NeuralODE.forward on _fake_solution: (full saved times, returned times, t1)."""
+    model = orc.MLP([orc.Dense(2, 4, "tanh"), orc.Dense(4, 2)], time_dependent=True)
+    layer = orc.NeuralODE(model, regularize=mode, **_solve_kwargs(saveat, save_start))
+    layer._solve = lambda x, ps: _fake_solution()
+    ps = orc.glorot_uniform_params(model, np.random.default_rng(0))
+    out, _, aux = layer.forward(np.zeros((2, 1), np.float32), ps, layer.initialstates(np.random.default_rng(1)))
+    full = out.t if mode == "none" else aux["out_full"].t
+    return list(full), list(out.t), aux.get("t1")
+
+
+def _save_plan(hc, mode, saveat, save_start, last_only, t1=0.0, u01=0.0, nsave=None):
+    """lrnde_opts as the NeuralODE layer fills them, through lr_save_plan on _FTS: (times, blocks, t1, nout)."""
+    pkg = entry.load_package()
+    layer = pkg.NeuralODE(pkg.Chain(pkg.Dense(2, 4, "tanh"), pkg.Dense(4, 2)), regularize=mode,
+                          return_last_only=last_only, **_solve_kwargs(saveat, save_start))
+    o, _keep = layer._opts(mode, t1, u01, keep_tape=True, host=True)
+    if nsave is not None:
+        o.nsave = nsave
+    cap = len(_FTS) + max(o.nsave, 0) + 3
+    times, out = np.zeros(cap, np.float32), np.zeros(cap, np.int32)
+    t1_out, nout = C.c_float(), C.c_int32()
+    n = hc.lrhc_save_plan(o.reg_mode, o.t0, o.t2, o.t1, o.u01, C.cast(o.saveat, C.c_void_p), o.nsave, o.save_start,
+                          o.last_only, _FTS.ctypes.data, len(_FTS), times.ctypes.data, out.ctypes.data, cap,
+                          C.byref(t1_out), C.byref(nout))
+    assert 0 < n <= cap
+    return times[:n], out[:n], np.float32(t1_out.value), nout.value
+
+
+def _returned(times, out, nout):
+    """The times of the output blocks 0 .. nout-1, in block order (each block written once)."""
+    blocks = sorted((int(b), t) for t, b in zip(times, out) if b >= 0)
+    assert [b for b, _ in blocks] == list(range(nout))
+    return np.array([t for _, t in blocks], np.float32)
+
+
+@pytest.mark.parametrize("last_only", [False, True], ids=["all", "last_only"])
+@pytest.mark.parametrize("save_start", [None, False, True], ids=["start_unset", "start0", "start1"])
+@pytest.mark.parametrize("saveat", [None, [0.25, 0.5, 0.9], [0.0, 0.4, 1.0]], ids=["no_saveat", "saveat", "saveat_t0"])
+@pytest.mark.parametrize("mode", ["none", "unbiased", "biased"])
+def test_save_plan_matches_oracle(hc, mode, saveat, save_start, last_only):
+    """The saved times, the returned blocks and t1 of a forward call (lrnde_saveplan.h) are those of the oracle's
+    NeuralODE.forward; :biased draws t1 with its own RNG there, so the library's rule is checked instead:
+    t1 = times[clamp(floor(u01 * ncand), 0, ncand - 1)] over the ncand = len(times) - 1 candidates times[:-1]."""
+    full, ret, t1_orc = _oracle_forward(mode, saveat, save_start)
+    want_ret = np.array(ret[-1:] if last_only else ret, np.float32)
+    for u01 in ((0.0, 0.37, 0.9999999) if mode == "biased" else (0.0,)):
+        t1_in = t1_orc if mode == "unbiased" else 0.0
+        times, out, t1, nout = _save_plan(hc, mode, saveat, save_start, last_only, t1=t1_in, u01=u01)
+        assert times.tobytes() == np.array(full, np.float32).tobytes(), (times, full)
+        assert _returned(times, out, nout).tobytes() == want_ret.tobytes(), (times, out, ret)
+        if mode == "biased":
+            ncand = len(times) - 1
+            idx = min(ncand - 1, max(0, int(np.floor(np.float32(u01) * np.float32(ncand)))))
+            assert t1 == times[idx] and t1_orc in list(times[:-1])
+        else:
+            assert t1 == np.float32(t1_in)
+
+
+@pytest.mark.parametrize("save_start", [False, True], ids=["start0", "start1"])
+@pytest.mark.parametrize("mode", ["none", "unbiased"])
+def test_save_plan_every_step(hc, mode, save_start):
+    """nsave == -1 saves every accepted step (the oracle's saveat = [] path) in any mode; t1 is not appended."""
+    times, out, t1, nout = _save_plan(hc, mode, None, save_start, False, t1=0.3, nsave=-1)
+    layer = orc.NeuralODE(orc.MLP([orc.Dense(2, 2)]), regularize=mode, save_start=save_start)
+    want = np.array(layer._saves(_fake_solution(), None, all_steps=True).t, np.float32)
+    assert times.tobytes() == want.tobytes()
+    assert _returned(times, out, nout).tobytes() == want.tobytes()
+    assert t1 == np.float32(0.3)
 
 
 def test_library_exports_every_header_symbol():

@@ -117,6 +117,78 @@ static inline int lr_ew_blocks(size_t n) {
   return (int)b;
 }
 
+struct DevBuf {  // pooled device scratch with RAII
+  lrnde_ctx* ctx;
+  float* p;
+  DevBuf(lrnde_ctx* c, size_t nfloat) : ctx(c), p((float*)c->alloc(sizeof(float) * nfloat)) {}
+  ~DevBuf() { ctx->release(p); }
+};
+
+// The caller's arrays of one C entry point: host memory when the call has host_buffers, device memory otherwise.
+// Kernels see only the device pointers this hands out; n counts elements.  Two kinds each way:
+//   in / out            staged: the caller's device array is used in place; a host array goes through a pooled
+//                       buffer (copied in now, or back by finish())
+//   copy_in / copy_out  owned copy: always a pooled buffer (or `dst` / `src`, a device buffer the entry point
+//                       owns), copied from / back to the caller either way.  For arrays the call overwrites,
+//                       arrays a tape keeps past the call, and kernels that want the pool's 256-byte alignment
+//                       or must not alias another argument
+// A NULL array gets no buffer and no copy.  Copies run on ctx->stream; finish() queues the copies back in the order
+// the outputs were declared and does not synchronise.
+struct CallerBufs {
+  lrnde_ctx* ctx;
+  const bool host;
+  CallerBufs(lrnde_ctx* c, int host_buffers) : ctx(c), host(host_buffers != 0) {}
+  ~CallerBufs() { for (void* q : pooled_) ctx->release(q); }
+  CallerBufs(const CallerBufs&) = delete;
+  CallerBufs& operator=(const CallerBufs&) = delete;
+
+  template <class T> const T* in(const T* p, size_t n) { return (p && host) ? copy_in(p, n) : p; }
+  template <class T> T* copy_in(const T* p, size_t n) {
+    if (!p) return nullptr;
+    T* d = pool<T>(n);
+    copy_in(d, p, n);
+    return d;
+  }
+  template <class T> void copy_in(T* dst, const T* p, size_t n) {
+    if (p)
+      LR_CUDA(cudaMemcpyAsync(dst, p, sizeof(T) * n, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice,
+                              ctx->stream));
+  }
+  template <class T> T* out(T* p, size_t n) { return (p && host) ? copy_out(p, n) : p; }
+  template <class T> T* copy_out(T* p, size_t n) {
+    if (!p) return nullptr;
+    T* d = pool<T>(n);
+    copy_out(p, (const T*)d, n);
+    return d;
+  }
+  template <class T> void copy_out(T* p, const T* src, size_t n) {
+    if (p) back_.push_back({p, src, sizeof(T) * n});
+  }
+  // staged input that the call also writes back (BatchNorm running statistics)
+  template <class T> T* inout(T* p, size_t n) {
+    if (!p || !host) return p;
+    T* d = copy_in(p, n);
+    copy_out(p, (const T*)d, n);
+    return d;
+  }
+  void finish() {
+    for (const Back& b : back_)
+      LR_CUDA(cudaMemcpyAsync(b.dst, b.src, b.bytes, host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice,
+                              ctx->stream));
+    back_.clear();
+  }
+
+ private:
+  struct Back { void* dst; const void* src; size_t bytes; };
+  std::vector<void*> pooled_;
+  std::vector<Back> back_;
+  template <class T> T* pool(size_t n) {
+    T* d = (T*)ctx->alloc(sizeof(T) * n);
+    pooled_.push_back(d);
+    return d;
+  }
+};
+
 extern "C" int lrnde_ctx_create(lrnde_ctx** out, int device, void* stream) {
   LR_API_BEGIN
   if (!out) lr_fail(LRNDE_EINVAL, "lrnde_ctx_create: out is NULL");
@@ -466,26 +538,19 @@ struct ConvEval {
     ctx->release(part); ctx->release(bpart); ctx->release(coef); ctx->release(dgb);
   }
 
-  // o->model_state (NULL: batch statistics, nothing tracked).  `stage`: device buffer of nstate floats used
-  // when the caller's pointer is a host pointer.  Returns the device pointer in use.
-  float* attach_state(const lrnde_opts* o, float* stage) {
+  // o->model_state (NULL: batch statistics, nothing tracked), staged through the call's `io`.  With `update` and
+  // outside testmode the f evaluations move the running statistics (until bn_update is cleared) and io.finish()
+  // returns st'.model.  Returns the device pointer in use.
+  float* attach_state(const lrnde_opts* o, CallerBufs& io, bool update) {
     bn_state = nullptr; testmode = 0; bn_update = false;
     if (!o) return nullptr;
     if (o->model_testmode && !o->model_state && nstate > 0)
       lr_fail(LRNDE_EINVAL, "model_testmode needs model_state (the running statistics BatchNorm normalises with)");
     if (!o->model_state || nstate == 0) return nullptr;
-    if (o->host_buffers) {
-      LR_CUDA(cudaMemcpyAsync(stage, o->model_state, 4 * nstate, cudaMemcpyHostToDevice, ctx->stream));
-      bn_state = stage;
-    } else bn_state = o->model_state;
     testmode = o->model_testmode ? 1 : 0;
-    bn_update = !testmode;
+    bn_update = update && !testmode;
+    bn_state = bn_update ? io.inout(o->model_state, nstate) : const_cast<float*>(io.in(o->model_state, nstate));
     return bn_state;
-  }
-  void return_state(const lrnde_opts* o) {   // st'.model back into the caller's buffer (host-pointer case)
-    if (bn_state && o && o->host_buffers && !testmode)
-      LR_CUDA(cudaMemcpyAsync(o->model_state, bn_state, 4 * nstate, cudaMemcpyDeviceToHost, ctx->stream));
-    bn_update = false;
   }
 
   void prepare() {
@@ -1784,15 +1849,10 @@ static void lr_validate_opts(const lrnde_opts* o) {
     lr_fail(LRNDE_EINVAL, "unknown precision %d", o->precision);
 }
 
-struct DevBuf {  // pooled device scratch with RAII
-  lrnde_ctx* ctx;
-  float* p;
-  DevBuf(lrnde_ctx* c, size_t nfloat) : ctx(c), p((float*)c->alloc(sizeof(float) * nfloat)) {}
-  ~DevBuf() { ctx->release(p); }
-};
-
 // The returned blocks of the saved solution into u_save (may be NULL) and their times into save_times (host, may be
-// NULL).  u_save is a HOST pointer when the forward call had host_buffers.
+// NULL).  u_save is a HOST pointer when the forward call had host_buffers: then each block goes through one D*B
+// device buffer, with a synchronisation before the next block reuses it, instead of CallerBufs, which would hold
+// nout*D*B of device scratch for the whole call.
 static void lr_write_saves(lrnde_ctx* ctx, lrnde_tape* T, FusedEngine* lean_fe, float* u_save, float* save_times) {
   const SavePlan& plan = T->saves;
   for (size_t i = 0; i < plan.times.size(); ++i)
@@ -1800,15 +1860,15 @@ static void lr_write_saves(lrnde_ctx* ctx, lrnde_tape* T, FusedEngine* lean_fe, 
   if (!u_save || plan.nout == 0) return;
   cudaStream_t st = ctx->stream;
   const size_t DB = T->fwd->h.len;
-  const int host = T->opts.host_buffers;
-  DevBuf dd(ctx, (size_t)plan.nout * (sizeof(LinComb) / 4 + 1)), stage(ctx, host ? DB : 1);
+  const bool per_block = T->opts.host_buffers != 0;
+  DevBuf dd(ctx, (size_t)plan.nout * (sizeof(LinComb) / 4 + 1)), stage(ctx, per_block ? DB : 1);
   for (size_t i = 0; i < plan.times.size(); ++i) {
     const int blk = plan.out[i];
     if (blk < 0) continue;
     LinComb hd;
-    float* dst = host ? stage.p : u_save + (size_t)blk * DB;
+    float* dst = per_block ? stage.p : u_save + (size_t)blk * DB;
     lr_sol_at(ctx, T, lean_fe, std::min(plan.times[i], T->fts.back()), dst, &hd, (const LinComb*)dd.p + blk);
-    if (host) {
+    if (per_block) {
       LR_CUDA(cudaMemcpyAsync(u_save + (size_t)blk * DB, dst, sizeof(float) * DB, cudaMemcpyDeviceToHost, st));
       LR_CUDA(cudaStreamSynchronize(st));   // stage is reused by the next block
     }
@@ -1827,26 +1887,19 @@ extern "C" int lrnde_dynamics_eval(lrnde_ctx* ctx, const lrnde_model* m, const l
   if (!ctx || !m || !ps || !u || !du || B < 1) lr_fail(LRNDE_EINVAL, "lrnde_dynamics_eval: bad args");
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int host = o ? o->host_buffers : 0;
   const size_t DB = (size_t)m->D * B;
-  DevBuf dps(ctx, host ? m->nparams : 1), dun(ctx, host ? DB : 1), dout(ctx, host ? DB : 1);
+  CallerBufs io(ctx, o ? o->host_buffers : 0);
+  const float* psd = io.in(ps, m->nparams);
+  const float* ud = io.in(u, DB);
+  float* outd = io.out(du, DB);
   DevBuf ddesc(ctx, sizeof(LinComb) / 4 + 1);
-  const float* psd = ps;
-  const float* ud = u;
-  float* outd = du;
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(dps.p, ps, 4 * m->nparams, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(dun.p, u, 4 * DB, cudaMemcpyHostToDevice, st));
-    psd = dps.p; ud = dun.p; outd = dout.p;
-  }
   LinComb d;
   memset(&d, 0, sizeof(d));
   d.base = ud; d.t = t; d.dst = outd;
   LR_CUDA(cudaMemcpyAsync(ddesc.p, &d, sizeof(d), cudaMemcpyHostToDevice, st));
   MlpEval ev(ctx, m, psd, B, lr_ode_route(ctx, m, o, B), false);
   ev.prepare();
-  DevBuf dstate(ctx, ev.conv ? std::max<int64_t>(1, ev.conv->nstate) : 1);
-  if (ev.conv) ev.conv->attach_state(o, dstate.p);
+  if (ev.conv) ev.conv->attach_state(o, io, true);
   if (ev.fe) {   // the same two kernels a solve uses for f(u0, t0): Z(u) by the layer-1 GEMM, then chain + kgemm
     Solver tmp(ctx, DB, DB, 2, 1, 1);
     tmp.init_ctrl(t, t + 1.0f, t + 1.0f, 10, 0, 1e-6f, 1e-6f);
@@ -1861,8 +1914,7 @@ extern "C" int lrnde_dynamics_eval(lrnde_ctx* ctx, const lrnde_model* m, const l
     LR_CUDA(cudaStreamSynchronize(st));
   } else
   ev.forward((const LinComb*)ddesc.p, nullptr);
-  if (ev.conv) ev.conv->return_state(o);
-  if (host) LR_CUDA(cudaMemcpyAsync(du, outd, 4 * DB, cudaMemcpyDeviceToHost, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -1873,19 +1925,14 @@ extern "C" int lrnde_dynamics_vjp(lrnde_ctx* ctx, const lrnde_model* m, const lr
   if (!ctx || !m || !ps || !u || !lam || !a || !dps || B < 1) lr_fail(LRNDE_EINVAL, "lrnde_dynamics_vjp: bad args");
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int host = o ? o->host_buffers : 0;
   const size_t DB = (size_t)m->D * B;
-  DevBuf dp(ctx, host ? m->nparams : 1), dun(ctx, host ? DB : 1), dl(ctx, host ? DB : 1), da(ctx, host ? DB : 1),
-      dg(ctx, host ? m->nparams : 1);
+  CallerBufs io(ctx, o ? o->host_buffers : 0);
+  const float* psd = io.in(ps, m->nparams);
+  const float* ud = io.in(u, DB);
+  const float* ld = io.in(lam, DB);
+  float* ad = io.out(a, DB);
+  float* gd = io.out(dps, m->nparams);
   DevBuf ddesc(ctx, 2 * (sizeof(LinComb) / 4 + 1));
-  const float* psd = ps; const float* ud = u; const float* ld = lam;
-  float* ad = a; float* gd = dps;
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(dp.p, ps, 4 * m->nparams, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(dun.p, u, 4 * DB, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(dl.p, lam, 4 * DB, cudaMemcpyHostToDevice, st));
-    psd = dp.p; ud = dun.p; ld = dl.p; ad = da.p; gd = dg.p;
-  }
   LinComb d[2];
   memset(d, 0, sizeof(d));
   d[0].base = ud; d[0].t = t;
@@ -1894,13 +1941,9 @@ extern "C" int lrnde_dynamics_vjp(lrnde_ctx* ctx, const lrnde_model* m, const lr
   LR_CUDA(cudaMemcpyAsync(dd, d, sizeof(d), cudaMemcpyHostToDevice, st));
   MlpEval ev(ctx, m, psd, B, lr_ode_route(ctx, m, o, B), true);
   ev.prepare();
-  DevBuf dstate(ctx, ev.conv ? std::max<int64_t>(1, ev.conv->nstate) : 1);
-  if (ev.conv) { ev.conv->attach_state(o, dstate.p); ev.conv->bn_update = false; }
+  if (ev.conv) ev.conv->attach_state(o, io, false);
   ev.vjp(dd, dd + 1, ad, nullptr, 1.0f, gd, nullptr, 0, 1.0f, 0.0f, nullptr);
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(a, ad, 4 * DB, cudaMemcpyDeviceToHost, st));
-    LR_CUDA(cudaMemcpyAsync(dps, gd, 4 * m->nparams, cudaMemcpyDeviceToHost, st));
-  }
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -1924,8 +1967,7 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
   const int D = m->D;
   const size_t DB = (size_t)D * B;
   const int64_t P = m->nparams;
-  const int host = o->host_buffers;
-  const cudaMemcpyKind in_kind = host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+  CallerBufs io(ctx, o->host_buffers);
 
   auto T = std::make_unique<lrnde_tape>();
   T->ctx = ctx;
@@ -1935,7 +1977,7 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
   T->B = B;
   T->reg_mode = o->reg_mode;
   T->ps = (float*)ctx->alloc(sizeof(float) * P);
-  LR_CUDA(cudaMemcpyAsync(T->ps, ps, sizeof(float) * P, in_kind, st));
+  io.copy_in(T->ps, ps, P);   // kept by the tape
   const bool timing = getenv("LRNDE_TIMING") != nullptr;
   const long tq0 = lr_now_us();
   T->route = lr_ode_route(ctx, m, o, B);
@@ -1953,7 +1995,7 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
   Solver& F = *T->fwd;
   if (ctx->nranks > 1) F.h.total_len = (unsigned long long)D * (unsigned long long)ctx->total_batch;
   F.init_ctrl(o->t0, o->t2, o->t2, o->maxiters, o->pow_mode, o->abstol, o->reltol);
-  LR_CUDA(cudaMemcpyAsync(F.tape, x, sizeof(float) * DB, in_kind, st));
+  io.copy_in(F.tape, x, DB);   // u_0, the first state of the tape
   LR_CUDA(cudaMemcpyAsync(F.ts, &o->t0, sizeof(float), cudaMemcpyHostToDevice, st));
   const long tq2 = lr_now_us();
 
@@ -1966,11 +2008,11 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
   ev.prepare();
   if (ev.conv) {   // st.model: tracked by the main solve's f evaluations only (the closure's st_ at the time
                    // _solve_neuralode_generic returns, neural_ode.jl:44-53)
-    if (ev.conv->nstate > 0 && o->model_state && (o->host_buffers || o->model_testmode))
+    const float* used = ev.conv->attach_state(o, io, true);
+    if (used && ev.conv->testmode) {   // kept by the tape: the backward normalises with the same statistics
       T->bn_state = (float*)ctx->alloc(4 * ev.conv->nstate);
-    float* used = ev.conv->attach_state(o, T->bn_state);
-    if (used && used != T->bn_state && T->bn_state)
       LR_CUDA(cudaMemcpyAsync(T->bn_state, used, 4 * ev.conv->nstate, cudaMemcpyDeviceToDevice, st));
+    }
   }
   const long tq3 = lr_now_us();
   // latent-space engine (lrnde_fused.h): stage chain in H dimensions + one GEMM per attempt for k_2..k_7
@@ -2019,7 +2061,8 @@ extern "C" int lrnde_ode_forward(lrnde_ctx* ctx, const lrnde_model* m, const lrn
     LR_COUNT(ctx);
   }
   const long t_solve = lr_now_us();
-  if (ev.conv) ev.conv->return_state(o);
+  if (ev.conv) ev.conv->bn_update = false;   // the regulariser's evaluations leave st.model alone
+  io.finish();
   const int naccept = F.h.c.naccept, nreject = F.h.c.nreject;
   T->fts.resize(naccept + 1);
   LR_CUDA(cudaMemcpyAsync(T->fts.data(), F.ts, sizeof(float) * (naccept + 1), cudaMemcpyDeviceToHost, st));
@@ -2349,7 +2392,6 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
   const size_t DB = (size_t)D * B;
   const size_t P = (size_t)m->nparams;
   const size_t len = DB + P;
-  const int host = o.host_buffers;
   const long launches0 = ctx->launches;
   const long tb_call = lr_now_us();
   Solver& F = *T->fwd;
@@ -2358,13 +2400,8 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
   const OdeRoute& route = T->route;
 
   // cotangent blocks on the device
-  const int nout = T->saves.nout;
-  DevBuf dstage(ctx, (host && d_u_save) ? DB * (size_t)std::max(nout, 1) : 1);
-  const float* dU = d_u_save;
-  if (host && d_u_save) {
-    LR_CUDA(cudaMemcpyAsync(dstage.p, d_u_save, sizeof(float) * DB * nout, cudaMemcpyHostToDevice, st));
-    dU = dstage.p;
-  }
+  CallerBufs io(ctx, o.host_buffers);
+  const float* dU = io.in(d_u_save, DB * (size_t)T->saves.nout);
   auto cot_blocks = [&](float tval, std::vector<const float*>& out) {
     out.clear();
     if (!dU) return;
@@ -2376,9 +2413,10 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
   if (ev.conv && o.model_testmode) { ev.conv->bn_state = T->bn_state; ev.conv->testmode = 1; }
 
   const bool no_dx = o.no_dx != 0;   // the caller has no use for dL/dx (nothing upstream has parameters)
-  DevBuf out_dx(ctx, (host || !d_x) ? DB : 1), out_dps(ctx, host ? P : 1);
-  float* dx_dev = (host || !d_x) ? out_dx.p : d_x;
-  float* dps_dev = host ? out_dps.p : d_ps;
+  float* dx_dev = io.out(no_dx ? nullptr : d_x, DB);
+  float* dps_dev = io.out(d_ps, P);
+  DevBuf dx_scratch(ctx, dx_dev ? 1 : DB);   // the adjoint solve forms dL/dx even when it is not returned
+  if (!dx_dev) dx_dev = dx_scratch.p;
 
   const long tb_start = lr_now_us();
   int nbwd_stops = 0;
@@ -2526,10 +2564,7 @@ extern "C" int lrnde_ode_backward(lrnde_ctx* ctx, const lrnde_model* m, lrnde_ta
     if (route.reg_hidden) lr_reg_pullback_hidden(ctx, m, T, ev, d_reg, dps_dev);
     else lr_reg_pullback_layers(ctx, m, T, ev, d_reg, dps_dev);
   }
-  if (host) {
-    if (!no_dx) LR_CUDA(cudaMemcpyAsync(d_x, dx_dev, sizeof(float) * DB, cudaMemcpyDeviceToHost, st));
-    LR_CUDA(cudaMemcpyAsync(d_ps, dps_dev, sizeof(float) * P, cudaMemcpyDeviceToHost, st));
-  }
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   if (ev.conv) ctx->bn_check();
   if (stats) {
@@ -2645,17 +2680,15 @@ extern "C" int lrnde_classifier_grad(lrnde_ctx* ctx, const lrnde_model* m, const
     lr_fail(LRNDE_EINVAL, "lrnde_classifier_grad: bad args");
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int host = o->host_buffers;
   const int D = m->D;
   const size_t DB = (size_t)D * B, P = (size_t)m->nparams, PW = (size_t)Cn * (D + 1);
-  DevBuf psd(ctx, host ? P : 1), wcd(ctx, host ? PW : 1), xd(ctx, host ? DB : 1), yd(ctx, host ? (size_t)B : 1);
-  DevBuf ud(ctx, DB), dud(ctx, DB), dpsd(ctx, host ? P : 1), dwd(ctx, host ? PW : 1);
-  const float* psv = ps; const float* wcv = Wc; const float* xv = x; const int32_t* yv = labels;
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(psd.p, ps, 4 * P, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(wcd.p, Wc, 4 * PW, cudaMemcpyHostToDevice, st));
-    psv = psd.p; wcv = wcd.p;
-    // inputs staged by lrnde_prefetch_inputs (oldest matching slot), else copied here
+  CallerBufs io(ctx, o->host_buffers);
+  const float* psv = io.in(ps, P);
+  const float* wcv = io.in(Wc, PW);
+  const float* xv = x; const int32_t* yv = labels;
+  // host x and labels: the copy lrnde_prefetch_inputs staged on the copy stream (oldest matching slot, waited for
+  // through its event), else copied here.  Device x and labels are used in place.
+  if (o->host_buffers) {
     if (ctx->pending.valid && ctx->pending.x == x && ctx->pending.y == labels) lr_flush_prefetch(ctx);   // this very batch
     lrnde_ctx::Staged* hit = nullptr;
     for (auto& sg : ctx->staged)
@@ -2665,14 +2698,14 @@ extern "C" int lrnde_classifier_grad(lrnde_ctx* ctx, const lrnde_model* m, const
       xv = hit->x; yv = hit->y;
       hit->ready = false;   // consumed: this call synchronises before returning, so the slot is free afterwards
     } else {
-      LR_CUDA(cudaMemcpyAsync(xd.p, x, 4 * DB, cudaMemcpyHostToDevice, st));
-      LR_CUDA(cudaMemcpyAsync(yd.p, labels, 4 * (size_t)B, cudaMemcpyHostToDevice, st));
-      xv = xd.p; yv = (const int32_t*)yd.p;
+      xv = io.in(x, DB);
+      yv = io.in(labels, (size_t)B);
     }
     lr_flush_prefetch(ctx);   // the next batch's copy, queued behind this call's own host -> device copies
   }
-  float* dpsv = host ? dpsd.p : d_ps;
-  float* dwv = host ? dwd.p : d_Wc;
+  float* dpsv = io.out(d_ps, P);
+  float* dwv = io.out(d_Wc, PW);
+  DevBuf ud(ctx, DB), dud(ctx, DB);
   const bool timing = getenv("LRNDE_TIMING") != nullptr;
   long tmark = lr_now_us();
   auto mark = [&](const char* what) {
@@ -2701,11 +2734,8 @@ extern "C" int lrnde_classifier_grad(lrnde_ctx* ctx, const lrnde_model* m, const
   mark("backward");
   if (T) lrnde_tape_free(T);
   if (rc != LRNDE_OK) throw LrError(rc);   // the failing call already set the error text
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(d_ps, dpsv, 4 * P, cudaMemcpyDeviceToHost, st));
-    LR_CUDA(cudaMemcpyAsync(d_Wc, dwv, 4 * PW, cudaMemcpyDeviceToHost, st));
-    LR_CUDA(cudaStreamSynchronize(st));
-  }
+  io.finish();
+  LR_CUDA(cudaStreamSynchronize(st));
   mark("stage out");
   *stats = s1;
   stats->nf_bwd = s2.nf_bwd; stats->naccept_bwd = s2.naccept_bwd; stats->nreject_bwd = s2.nreject_bwd;

@@ -33,16 +33,13 @@ extern "C" int lrnde_conv2d_forward(lrnde_ctx* ctx, int32_t in_ch, int32_t out_c
   convops::check_shape("lrnde_conv2d_forward", in_ch, out_ch, width, height, B);
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int host = host_buffers;
   const size_t HW = (size_t)width * height, nx = HW * in_ch * B, ny = HW * out_ch * B;
   const size_t nw = (size_t)9 * in_ch * out_ch, np = nw + (use_bias ? out_ch : 0);
-  DevBuf dp(ctx, host ? np : 1), dx(ctx, host ? nx : 1), dy(ctx, host ? ny : 1), pack(ctx, nw);
-  const float* psd = ps; const float* xd = x; float* yd = y;
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(dp.p, ps, 4 * np, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(dx.p, x, 4 * nx, cudaMemcpyHostToDevice, st));
-    psd = dp.p; xd = dx.p; yd = dy.p;
-  }
+  CallerBufs io(ctx, host_buffers);
+  const float* psd = io.in(ps, np);
+  const float* xd = io.in(x, nx);
+  float* yd = io.out(y, ny);
+  DevBuf pack(ctx, nw);
   conv_pack_kernel<<<lr_ew_blocks(nw), 256, 0, st>>>(psd, in_ch, out_ch, 0, 0, pack.p);
   LR_COUNT(ctx);
   ConvP q;
@@ -51,7 +48,7 @@ extern "C" int lrnde_conv2d_forward(lrnde_ctx* ctx, int32_t in_ch, int32_t out_c
   q.bias = use_bias ? psd + nw : nullptr; q.out_act = lr_map_act(act);
   convops::launch_conv(ctx, q, B);
   LR_CHECK_LAUNCH();
-  if (host) LR_CUDA(cudaMemcpyAsync(y, yd, 4 * ny, cudaMemcpyDeviceToHost, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -64,22 +61,17 @@ extern "C" int lrnde_conv2d_backward(lrnde_ctx* ctx, int32_t in_ch, int32_t out_
   convops::check_shape("lrnde_conv2d_backward", in_ch, out_ch, width, height, B);
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int host = host_buffers;
   const int a = lr_map_act(act);
   const size_t HW = (size_t)width * height, nx = HW * in_ch * B, ny = HW * out_ch * B;
   const size_t nw = (size_t)9 * in_ch * out_ch, np = nw + (use_bias ? out_ch : 0);
-  DevBuf dp(ctx, host ? np : 1), dx(ctx, host ? nx : 1), dg(ctx, ny), pre(ctx, a != ACT_IDENTITY ? ny : 1);
+  CallerBufs io(ctx, host_buffers);
+  const float* psd = io.in(ps, np);
+  const float* xd = io.in(x, nx);
+  float* dg = io.copy_in(d_y, ny);   // owned copy: overwritten by the pullback through the activation
+  float* dpsd = io.out(d_ps, np);
+  float* dxd = io.out(d_x, nx);
+  DevBuf pre(ctx, a != ACT_IDENTITY ? ny : 1);
   DevBuf pack(ctx, nw), packT(ctx, nw), ydummy(ctx, a != ACT_IDENTITY ? ny : 1);
-  DevBuf odx(ctx, (host && d_x) ? nx : 1), odp(ctx, host ? np : 1);
-  const float* psd = ps; const float* xd = x;
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(dp.p, ps, 4 * np, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(dx.p, x, 4 * nx, cudaMemcpyHostToDevice, st));
-    psd = dp.p; xd = dx.p;
-  }
-  LR_CUDA(cudaMemcpyAsync(dg.p, d_y, 4 * ny, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st));
-  float* dpsd = host ? odp.p : d_ps;
-  float* dxd = host ? odx.p : d_x;
   if (a != ACT_IDENTITY) {   // recompute the pre-activation, then delta = d_y * act'(pre)
     conv_pack_kernel<<<lr_ew_blocks(nw), 256, 0, st>>>(psd, in_ch, out_ch, 0, 0, pack.p);
     LR_COUNT(ctx);
@@ -88,7 +80,7 @@ extern "C" int lrnde_conv2d_backward(lrnde_ctx* ctx, int32_t in_ch, int32_t out_
     q.X = xd; q.Wp = pack.p; q.Wd = width; q.Ht = height; q.Cin = in_ch; q.Cout = out_ch; q.Y = ydummy.p; q.out_scale = 1.0f;
     q.bias = use_bias ? psd + nw : nullptr; q.out_act = ACT_IDENTITY; q.pre = pre.p;
     convops::launch_conv(ctx, q, B);
-    bn_bwd_apply_kernel<<<lr_ew_blocks(ny), 256, 0, st>>>(dg.p, pre.p, nullptr, nullptr, nullptr, a, out_ch, HW, ny, nullptr);
+    bn_bwd_apply_kernel<<<lr_ew_blocks(ny), 256, 0, st>>>(dg, pre.p, nullptr, nullptr, nullptr, a, out_ch, HW, ny, nullptr);
     LR_COUNT(ctx);
   }
   // weight gradient (split over the batch, fixed-order reduce) and bias gradient
@@ -105,7 +97,7 @@ extern "C" int lrnde_conv2d_backward(lrnde_ctx* ctx, int32_t in_ch, int32_t out_
     ConvWgOp ox, od;
     memset(&ox, 0, sizeof(ox)); memset(&od, 0, sizeof(od));
     ox.ptr = xd; ox.act = ACT_IDENTITY; ox.C = in_ch; ox.td = 0;
-    od.ptr = dg.p; od.act = ACT_IDENTITY; od.C = out_ch; od.td = 0;
+    od.ptr = dg; od.act = ACT_IDENTITY; od.C = out_ch; od.td = 0;
     w.swapped = swapped ? 1 : 0;
     w.P = swapped ? od : ox; w.Q = swapped ? ox : od;
     w.Wd = width; w.Ht = height; w.B = (int)B; w.CinTot = in_ch; w.Cout = out_ch;
@@ -115,7 +107,7 @@ extern "C" int lrnde_conv2d_backward(lrnde_ctx* ctx, int32_t in_ch, int32_t out_
     wgrad_reduce_kernel<<<lr_ew_blocks(nw), 256, 0, st>>>(part.p, S, nw, dpsd, nullptr, 0, 1.0f, 0.0f, nullptr);
     LR_COUNT(ctx);
     if (use_bias) {
-      channel_sum_kernel<<<out_ch, 256, 0, st>>>(dg.p, out_ch, HW, (int)B, dpsd + nw);
+      channel_sum_kernel<<<out_ch, 256, 0, st>>>(dg, out_ch, HW, (int)B, dpsd + nw);
       LR_COUNT(ctx);
     }
   }
@@ -124,14 +116,11 @@ extern "C" int lrnde_conv2d_backward(lrnde_ctx* ctx, int32_t in_ch, int32_t out_
     LR_COUNT(ctx);
     ConvP q;
     memset(&q, 0, sizeof(q));
-    q.X = dg.p; q.Wp = packT.p; q.Wd = width; q.Ht = height; q.Cin = out_ch; q.Cout = in_ch; q.Y = dxd; q.out_scale = 1.0f;
+    q.X = dg; q.Wp = packT.p; q.Wd = width; q.Ht = height; q.Cin = out_ch; q.Cout = in_ch; q.Y = dxd; q.out_scale = 1.0f;
     convops::launch_conv(ctx, q, B);
   }
   LR_CHECK_LAUNCH();
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(d_ps, dpsd, 4 * np, cudaMemcpyDeviceToHost, st));
-    if (d_x) LR_CUDA(cudaMemcpyAsync(d_x, dxd, 4 * nx, cudaMemcpyDeviceToHost, st));
-  }
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -163,25 +152,19 @@ extern "C" int lrnde_batchnorm_forward(lrnde_ctx* ctx, int32_t C, int64_t HW, in
   if (testmode && !state) lr_fail(LRNDE_EINVAL, "lrnde_batchnorm_forward: testmode needs the running statistics");
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int host = host_buffers;
   const size_t n = (size_t)HW * C * B;
-  DevBuf dp(ctx, host ? 2 * C : 1), dx(ctx, host ? n : 1), dy(ctx, host ? n : 1), ds(ctx, (host && state) ? 2 * C : 1);
+  CallerBufs io(ctx, host_buffers);
+  const float* psd = io.in(ps, 2 * (size_t)C);
+  const float* xd = io.in(x, n);
+  float* yd = io.out(y, n);
+  // running statistics: read in testmode, else updated and returned
+  float* sd = testmode ? const_cast<float*>(io.in(state, 2 * (size_t)C)) : io.inout(state, 2 * (size_t)C);
   DevBuf ab(ctx, 2 * C), stat(ctx, 2 * C);
-  const float* psd = ps; const float* xd = x; float* yd = y; float* sd = state;
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(dp.p, ps, 8 * C, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(dx.p, x, 4 * n, cudaMemcpyHostToDevice, st));
-    if (state) { LR_CUDA(cudaMemcpyAsync(ds.p, state, 8 * C, cudaMemcpyHostToDevice, st)); sd = ds.p; }
-    psd = dp.p; xd = dx.p; yd = dy.p;
-  }
   convops::bn_statistics(ctx, C, (size_t)HW, B, psd, xd, sd, testmode, 1, ab.p, stat.p);
   bn_apply_kernel<<<lr_ew_blocks(n), 256, 0, st>>>(xd, ab.p, lr_map_act(act), C, (size_t)HW, n, yd);
   LR_COUNT(ctx);
   LR_CHECK_LAUNCH();
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(y, yd, 4 * n, cudaMemcpyDeviceToHost, st));
-    if (state && !testmode) LR_CUDA(cudaMemcpyAsync(state, sd, 8 * C, cudaMemcpyDeviceToHost, st));
-  }
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   ctx->bn_check();
   LR_API_END
@@ -196,26 +179,21 @@ extern "C" int lrnde_batchnorm_backward(lrnde_ctx* ctx, int32_t C, int64_t HW, i
   if (testmode && !state) lr_fail(LRNDE_EINVAL, "lrnde_batchnorm_backward: testmode needs the running statistics");
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int host = host_buffers;
   const int a = lr_map_act(act);
   const size_t n = (size_t)HW * C * B;
-  DevBuf dp(ctx, host ? 2 * C : 1), dx(ctx, host ? n : 1), ds(ctx, (host && state) ? 2 * C : 1), g(ctx, host ? n : 1);
-  DevBuf ab(ctx, 2 * C), stat(ctx, 2 * C), coef(ctx, 2 * C), dgb(ctx, host ? 2 * C : 1);
-  const float* psd = ps; const float* xd = x; const float* sd = state;
-  float* gd = d_x;   // the pullback is formed in place over a copy of d_y
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(dp.p, ps, 8 * C, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(dx.p, x, 4 * n, cudaMemcpyHostToDevice, st));
-    if (state) { LR_CUDA(cudaMemcpyAsync(ds.p, state, 8 * C, cudaMemcpyHostToDevice, st)); sd = ds.p; }
-    psd = dp.p; xd = dx.p; gd = g.p;
-  }
-  LR_CUDA(cudaMemcpyAsync(gd, d_y, 4 * n, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st));
+  CallerBufs io(ctx, host_buffers);
+  const float* psd = io.in(ps, 2 * (size_t)C);
+  const float* xd = io.in(x, n);
+  const float* sd = io.in(state, 2 * (size_t)C);
+  float* gd = io.out(d_x, n);   // the pullback is formed in place over a copy of d_y
+  io.copy_in(gd, d_y, n);
+  float* dgbd = io.out(d_ps, 2 * (size_t)C);
+  DevBuf ab(ctx, 2 * C), stat(ctx, 2 * C), coef(ctx, 2 * C);
   convops::bn_statistics(ctx, C, (size_t)HW, B, psd, xd, const_cast<float*>(sd), testmode, 0, ab.p, stat.p);
   int S = (int)std::max<int64_t>(1, std::min<int64_t>(B, 16));
   const int img = (int)((B + S - 1) / S);
   S = (int)((B + img - 1) / img);
   DevBuf bpart(ctx, 4 * (size_t)C * S);
-  float* dgbd = host ? dgb.p : d_ps;
   bn_bwd_stats_kernel<<<dim3(C, S), 256, 0, st>>>(gd, xd, ab.p, stat.p, a, C, (size_t)HW, (int)B, img, (double2*)bpart.p, nullptr);
   LR_COUNT(ctx);
   bn_bwd_finalize_kernel<<<(C + 63) / 64, 64, 0, st>>>((const double2*)bpart.p, S, C, (double)HW * (double)B, coef.p, dgbd,
@@ -224,10 +202,7 @@ extern "C" int lrnde_batchnorm_backward(lrnde_ctx* ctx, int32_t C, int64_t HW, i
   bn_bwd_apply_kernel<<<lr_ew_blocks(n), 256, 0, st>>>(gd, xd, ab.p, stat.p, coef.p, a, C, (size_t)HW, n, nullptr);
   LR_COUNT(ctx);
   LR_CHECK_LAUNCH();
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(d_x, gd, 4 * n, cudaMemcpyDeviceToHost, st));
-    LR_CUDA(cudaMemcpyAsync(d_ps, dgbd, 8 * C, cudaMemcpyDeviceToHost, st));
-  }
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   ctx->bn_check();
   LR_API_END

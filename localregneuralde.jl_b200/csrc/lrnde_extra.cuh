@@ -121,17 +121,16 @@ extern "C" int lrnde_sosri_step(lrnde_ctx* ctx, const lrnde_model* drift,
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const size_t DB = (size_t)drift->D * B;
-  const int host = o->host_buffers;
-  const cudaMemcpyKind kin = host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-  DevBuf psd(ctx, drift->nparams), psg(ctx, diffusion->nparams);
+  // owned copies throughout: the inputs sit together in one pooled buffer, u is a slice of the work buffer
+  CallerBufs io(ctx, o->host_buffers);
+  const float* psd = io.copy_in(ps_drift, drift->nparams);
+  const float* psg = io.copy_in(ps_diffusion, diffusion->nparams);
   DevBuf in(ctx, 3 * DB), work(ctx, 11 * DB);
   DevBuf descs(ctx, 8 * (sizeof(LinComb) / 4 + 1));
   DevBuf red(ctx, 2 * LR_ERR_BLOCKS + 8);
-  LR_CUDA(cudaMemcpyAsync(psd.p, ps_drift, 4 * drift->nparams, kin, st));
-  LR_CUDA(cudaMemcpyAsync(psg.p, ps_diffusion, 4 * diffusion->nparams, kin, st));
-  LR_CUDA(cudaMemcpyAsync(in.p, uprev, 4 * DB, kin, st));
-  LR_CUDA(cudaMemcpyAsync(in.p + DB, dW, 4 * DB, kin, st));
-  LR_CUDA(cudaMemcpyAsync(in.p + 2 * DB, dZ, 4 * DB, kin, st));
+  io.copy_in(in.p, uprev, DB);
+  io.copy_in(in.p + DB, dW, DB);
+  io.copy_in(in.p + 2 * DB, dZ, DB);
   SosriP p;
   p.c = lr_sosri_tab();
   p.uprev = in.p; p.dW = in.p + DB; p.dZ = in.p + 2 * DB;
@@ -154,8 +153,8 @@ extern "C" int lrnde_sosri_step(lrnde_ctx* ctx, const lrnde_model* drift,
   }
   LR_CUDA(cudaMemcpyAsync(descs.p, hd.data(), sizeof(LinComb) * 8, cudaMemcpyHostToDevice, st));
   const LinComb* dd = (const LinComb*)descs.p;
-  MlpEval evf(ctx, drift, psd.p, B, lr_ode_route(ctx, drift, o, B), false);
-  MlpEval evg(ctx, diffusion, psg.p, B, lr_ode_route(ctx, diffusion, o, B), false);
+  MlpEval evf(ctx, drift, psd, B, lr_ode_route(ctx, drift, o, B), false);
+  MlpEval evg(ctx, diffusion, psg, B, lr_ode_route(ctx, diffusion, o, B), false);
   evf.prepare();
   evg.prepare();
   for (int s = 0; s < 4; ++s) {
@@ -172,7 +171,8 @@ extern "C" int lrnde_sosri_step(lrnde_ctx* ctx, const lrnde_model* drift,
   sosri_finish_kernel<<<1, 32, 0, st>>>(p.partials, (double)DB, dt, out_scalar);
   LR_COUNT(ctx);
   LR_CHECK_LAUNCH();
-  LR_CUDA(cudaMemcpyAsync(u, p.u, 4 * DB, host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+  io.copy_out(u, p.u, DB);
+  io.finish();
   LR_CUDA(cudaMemcpyAsync(reg_val, out_scalar, 4, cudaMemcpyDeviceToHost, st));
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
@@ -285,21 +285,17 @@ extern "C" int lrnde_head_ce(lrnde_ctx* ctx, const float* Wc, const float* u,
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const size_t DB = (size_t)D * B, CB = (size_t)Cn * B, PW = (size_t)Cn * (D + 1);
-  const int host = host_buffers;
-  DevBuf w(ctx, host ? PW : 1), ub(ctx, host ? DB : 1), lb(ctx, host ? (size_t)B : 1);
   DevBuf logits(ctx, CB), dlog(ctx, CB), wt(ctx, (size_t)D * Cn);
-  DevBuf dub(ctx, host ? DB : 1), dwb(ctx, host ? PW : 1);
   const int nb = 296;
   DevBuf red(ctx, 2 * nb + 8);
   int* badd = (int*)(red.p + 2 * nb + 4);
   LR_CUDA(cudaMemsetAsync(badd, 0, sizeof(int), st));
-  const float* Wd = Wc; const float* ud = u; const int* ld = labels;
-  if (host) {
-    LR_CUDA(cudaMemcpyAsync(w.p, Wc, 4 * PW, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(ub.p, u, 4 * DB, cudaMemcpyHostToDevice, st));
-    LR_CUDA(cudaMemcpyAsync(lb.p, labels, 4 * (size_t)B, cudaMemcpyHostToDevice, st));
-    Wd = w.p; ud = ub.p; ld = (const int*)lb.p;
-  }
+  CallerBufs io(ctx, host_buffers);
+  const float* Wd = io.in(Wc, PW);
+  const float* ud = io.in(u, DB);
+  const int* ld = io.in(labels, (size_t)B);
+  float* dud = io.out(d_u, DB);
+  float* dWd = io.out(d_Wc, PW);
   const size_t head_smem = sizeof(float) * (size_t)Cn * (D + 1);
   const bool fused_head = Cn <= kHeadMaxC && head_smem <= 160 * 1024 && !getenv("LRNDE_NO_FUSED_HEAD");
   float* lossd = (float*)((double*)red.p + nb);
@@ -311,12 +307,10 @@ extern "C" int lrnde_head_ce(lrnde_ctx* ctx, const float* Wc, const float* u,
     }
     LR_CUDA(cudaMemsetAsync(red.p, 0, sizeof(double) * nb, st));
     const int hb = (int)std::min<int64_t>(nb, (B + 7) / 8);   // at most nb blocks (the partial sums), 8 warps each
-    head_fused_kernel<<<hb, 256, head_smem, st>>>(Wd, ud, ld, Cn, D, (int)B, dlog.p, d_u ? (host ? dub.p : d_u) : nullptr,
-                                                  (double*)red.p, badd);
+    head_fused_kernel<<<hb, 256, head_smem, st>>>(Wd, ud, ld, Cn, D, (int)B, dlog.p, dud, (double*)red.p, badd);
     LR_COUNT(ctx);
     mean_finish_kernel<<<1, 32, 0, st>>>((double*)red.p, nb, (double)B, lossd);
     LR_COUNT(ctx);
-    if (d_u && host) LR_CUDA(cudaMemcpyAsync(d_u, dub.p, 4 * DB, cudaMemcpyDeviceToHost, st));
   } else {
   DenseP p;
   memset(&p, 0, sizeof(p));
@@ -338,11 +332,10 @@ extern "C" int lrnde_head_ce(lrnde_ctx* ctx, const float* Wc, const float* u,
     DenseP q;
     memset(&q, 0, sizeof(q));
     q.A = wt.p; q.lda = D; q.M = D; q.K = Cn; q.X = dlog.p; q.ldx = Cn; q.N = (int)B;
-    q.Y = host ? dub.p : d_u; q.ldy = D; q.act = ACT_IDENTITY; q.dact = -1; q.out_scale = 1.0f;
+    q.Y = dud; q.ldy = D; q.act = ACT_IDENTITY; q.dact = -1; q.out_scale = 1.0f;
     dim3 g2((D + DN_BM - 1) / DN_BM, (unsigned)((B + DN_BN - 1) / DN_BN));
     dense_nn_kernel<<<g2, 256, 0, st>>>(q);
     LR_COUNT(ctx);
-    if (host) LR_CUDA(cudaMemcpyAsync(d_u, dub.p, 4 * DB, cudaMemcpyDeviceToHost, st));
   }
   if (d_Wc) {
     const int naug = D + 1;
@@ -359,14 +352,13 @@ extern "C" int lrnde_head_ce(lrnde_ctx* ctx, const float* Wc, const float* u,
     dim3 g3((Cn + DN_BM - 1) / DN_BM, (naug + DN_BN - 1) / DN_BN, S);
     wgrad_nt_kernel<<<g3, 256, 0, st>>>(wg);
     LR_COUNT(ctx);
-    wgrad_reduce_kernel<<<lr_ew_blocks(PW), 256, 0, st>>>(part.p, S, PW, host ? dwb.p : d_Wc, nullptr,
-                                                          0, 1.0f, 0.0f, nullptr);
+    wgrad_reduce_kernel<<<lr_ew_blocks(PW), 256, 0, st>>>(part.p, S, PW, dWd, nullptr, 0, 1.0f, 0.0f, nullptr);
     LR_COUNT(ctx);
-    if (host) LR_CUDA(cudaMemcpyAsync(d_Wc, dwb.p, 4 * PW, cudaMemcpyDeviceToHost, st));
     LR_CHECK_LAUNCH();
     LR_CUDA(cudaStreamSynchronize(st));
   }
   LR_CHECK_LAUNCH();
+  io.finish();
   int bad_host = 0;
   LR_CUDA(cudaMemcpyAsync(loss, lossd, 4, cudaMemcpyDeviceToHost, st));
   LR_CUDA(cudaMemcpyAsync(&bad_host, badd, sizeof(int), cudaMemcpyDeviceToHost, st));

@@ -282,10 +282,11 @@ extern "C" int lrnde_gru_forward(lrnde_ctx* ctx, int32_t F, int32_t H, int32_t L
   auto take = [&](size_t nfloat) { float* q = (float*)ctx->alloc(sizeof(float) * std::max<size_t>(nfloat, 1)); Tp->owned.push_back(q); return q; };
   const int64_t P = lrnde_gru_nparams(F, H, L);
   const size_t nx = (size_t)F * T * B, ny = (size_t)2 * L * B;
-  const cudaMemcpyKind in_kind = host_buffers ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+  CallerBufs io(ctx, host_buffers);
   float* psd = take(P); float* xd = take(nx); float* yd = take(ny);
-  LR_CUDA(cudaMemcpyAsync(psd, ps, sizeof(float) * P, in_kind, st));
-  LR_CUDA(cudaMemcpyAsync(xd, x, sizeof(float) * nx, in_kind, st));
+  io.copy_in(psd, ps, P);   // ps and x: kept by the tape for the backward
+  io.copy_in(xd, x, nx);
+  io.copy_out(y, yd, ny);
   p.ps = psd; p.x = xd; p.y = yd;
   p.carry = keep_tape ? take((size_t)T * ny) : nullptr;
   const size_t smem = gru_smem_bytes(p, false);
@@ -293,7 +294,7 @@ extern "C" int lrnde_gru_forward(lrnde_ctx* ctx, int32_t F, int32_t H, int32_t L
   gru_forward_kernel<<<Tp->grid, SDE_THREADS, smem, st>>>(p);
   LR_COUNT(ctx);
   LR_CUDA(cudaGetLastError());
-  LR_CUDA(cudaMemcpyAsync(y, yd, sizeof(float) * ny, host_buffers ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   if (keep_tape) *tape_out = Tp.release();
   LR_API_END
@@ -307,21 +308,22 @@ extern "C" int lrnde_gru_backward(lrnde_ctx* ctx, lrnde_gru_tape* Tp, const floa
   GruP p = Tp->p;
   const size_t ny = (size_t)2 * p.L * p.B;
   const int64_t P = lrnde_gru_nparams(p.F, p.nu.out[0], p.L);
-  DevBuf dy(ctx, ny), dps(ctx, P);
+  CallerBufs io(ctx, Tp->host);   // owned copies: pooled (256-byte aligned) arrays that alias no argument
+  p.d_y = io.copy_in(d_y, ny);
+  float* dps = io.copy_out(d_ps, P);
   const int stride = p.nu.wfloats + p.nr.wfloats + p.nn.wfloats;
   DevBuf gpart(ctx, (size_t)Tp->grid * stride);
-  LR_CUDA(cudaMemcpyAsync(dy.p, d_y, sizeof(float) * ny, Tp->host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st));
-  p.d_y = dy.p; p.gpart = gpart.p;
+  p.gpart = gpart.p;
   const size_t smem = gru_smem_bytes(p, true);
   LR_CUDA(cudaFuncSetAttribute(gru_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   gru_backward_kernel<<<Tp->grid, SDE_THREADS, smem, st>>>(p);
   LR_COUNT(ctx);
-  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(p.nu, gpart.p, stride, 0, Tp->grid, dps.p);
-  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(p.nr, gpart.p, stride, p.nu.wfloats, Tp->grid, dps.p);
-  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(p.nn, gpart.p, stride, p.nu.wfloats + p.nr.wfloats, Tp->grid, dps.p);
+  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(p.nu, gpart.p, stride, 0, Tp->grid, dps);
+  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(p.nr, gpart.p, stride, p.nu.wfloats, Tp->grid, dps);
+  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(p.nn, gpart.p, stride, p.nu.wfloats + p.nr.wfloats, Tp->grid, dps);
   LR_COUNT(ctx); LR_COUNT(ctx); LR_COUNT(ctx);
   LR_CUDA(cudaGetLastError());
-  LR_CUDA(cudaMemcpyAsync(d_ps, dps.p, sizeof(float) * P, Tp->host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -452,17 +454,16 @@ extern "C" int lrnde_mlp_forward(lrnde_ctx* ctx, const lrnde_layer_desc* layers,
   cudaStream_t st = ctx->stream;
   MlpOpP p; int grid = 1;
   mlpop_setup(ctx, p, layers, nlayers, N, &grid);
-  const cudaMemcpyKind ik = host_buffers ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-  DevBuf psd(ctx, p.n.nparams), xd(ctx, (size_t)p.in0 * N), yd(ctx, (size_t)p.outL * N);
-  LR_CUDA(cudaMemcpyAsync(psd.p, ps, sizeof(float) * p.n.nparams, ik, st));
-  LR_CUDA(cudaMemcpyAsync(xd.p, x, sizeof(float) * p.in0 * N, ik, st));
-  p.ps = psd.p; p.x = xd.p; p.y = yd.p;
+  CallerBufs io(ctx, host_buffers);   // owned copies: pooled (256-byte aligned) arrays that alias no argument
+  p.ps = io.copy_in(ps, p.n.nparams);
+  p.x = io.copy_in(x, (size_t)p.in0 * N);
+  p.y = io.copy_out(y, (size_t)p.outL * N);
   const size_t smem = mlpop_smem(p, false);
   LR_CUDA(cudaFuncSetAttribute(mlpop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   mlpop_kernel<false><<<grid, SDE_THREADS, smem, st>>>(p);
   LR_COUNT(ctx);
   LR_CUDA(cudaGetLastError());
-  LR_CUDA(cudaMemcpyAsync(y, yd.p, sizeof(float) * p.outL * N, host_buffers ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -476,23 +477,23 @@ extern "C" int lrnde_mlp_backward(lrnde_ctx* ctx, const lrnde_layer_desc* layers
   cudaStream_t st = ctx->stream;
   MlpOpP p; int grid = 1;
   mlpop_setup(ctx, p, layers, nlayers, N, &grid);
-  const cudaMemcpyKind ik = host_buffers ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-  const cudaMemcpyKind ok = host_buffers ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  DevBuf psd(ctx, p.n.nparams), xd(ctx, (size_t)p.in0 * N), dyd(ctx, (size_t)p.outL * N), dxd(ctx, (size_t)p.in0 * N);
-  DevBuf gpart(ctx, (size_t)grid * p.n.wfloats), dpsd(ctx, p.n.nparams);
-  LR_CUDA(cudaMemcpyAsync(psd.p, ps, sizeof(float) * p.n.nparams, ik, st));
-  LR_CUDA(cudaMemcpyAsync(xd.p, x, sizeof(float) * p.in0 * N, ik, st));
-  LR_CUDA(cudaMemcpyAsync(dyd.p, d_y, sizeof(float) * p.outL * N, ik, st));
-  p.ps = psd.p; p.x = xd.p; p.d_y = dyd.p; p.d_x = dxd.p; p.gpart = gpart.p;
+  CallerBufs io(ctx, host_buffers);   // owned copies: pooled (256-byte aligned) arrays that alias no argument
+  p.ps = io.copy_in(ps, p.n.nparams);
+  p.x = io.copy_in(x, (size_t)p.in0 * N);
+  p.d_y = io.copy_in(d_y, (size_t)p.outL * N);
+  DevBuf dxd(ctx, (size_t)p.in0 * N);   // the kernel always writes d_x
+  io.copy_out(d_x, dxd.p, (size_t)p.in0 * N);
+  DevBuf gpart(ctx, (size_t)grid * p.n.wfloats);
+  float* dpsd = io.copy_out(d_ps, p.n.nparams);
+  p.d_x = dxd.p; p.gpart = gpart.p;
   const size_t smem = mlpop_smem(p, true);
   LR_CUDA(cudaFuncSetAttribute(mlpop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   mlpop_kernel<true><<<grid, SDE_THREADS, smem, st>>>(p);
   LR_COUNT(ctx);
-  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(p.n, gpart.p, p.n.wfloats, 0, grid, dpsd.p);
+  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(p.n, gpart.p, p.n.wfloats, 0, grid, dpsd);
   LR_COUNT(ctx);
   LR_CUDA(cudaGetLastError());
-  if (d_x) LR_CUDA(cudaMemcpyAsync(d_x, dxd.p, sizeof(float) * p.in0 * N, ok, st));
-  LR_CUDA(cudaMemcpyAsync(d_ps, dpsd.p, sizeof(float) * p.n.nparams, ok, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -523,20 +524,17 @@ extern "C" int lrnde_reparameterize(lrnde_ctx* ctx, const float* x, int32_t L, i
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const size_t n = (size_t)L * B;
-  const cudaMemcpyKind ik = host_buffers ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-  const cudaMemcpyKind ok = host_buffers ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  DevBuf xd(ctx, 2 * n), yd(ctx, n), dyd(ctx, n), dmd(ctx, n), dld(ctx, n), dxd(ctx, 2 * n);
-  LR_CUDA(cudaMemcpyAsync(xd.p, x, sizeof(float) * 2 * n, ik, st));
-  if (d_y) LR_CUDA(cudaMemcpyAsync(dyd.p, d_y, sizeof(float) * n, ik, st));
-  if (d_mu) LR_CUDA(cudaMemcpyAsync(dmd.p, d_mu, sizeof(float) * n, ik, st));
-  if (d_ls) LR_CUDA(cudaMemcpyAsync(dld.p, d_ls, sizeof(float) * n, ik, st));
-  reparam_kernel<<<lr_ew_blocks(n), 256, 0, st>>>(xd.p, L, (int)B, seed, training, y ? yd.p : nullptr,
-                                                   d_y ? dyd.p : nullptr, d_mu ? dmd.p : nullptr, d_ls ? dld.p : nullptr,
-                                                   d_x ? dxd.p : nullptr);
+  CallerBufs io(ctx, host_buffers);   // owned copies: pooled (256-byte aligned) arrays that alias no argument
+  const float* xd = io.copy_in(x, 2 * n);
+  float* yd = io.copy_out(y, n);
+  const float* dyd = io.copy_in(d_y, n);
+  const float* dmd = io.copy_in(d_mu, n);
+  const float* dld = io.copy_in(d_ls, n);
+  float* dxd = io.copy_out(d_x, 2 * n);
+  reparam_kernel<<<lr_ew_blocks(n), 256, 0, st>>>(xd, L, (int)B, seed, training, yd, dyd, dmd, dld, dxd);
   LR_COUNT(ctx);
   LR_CUDA(cudaGetLastError());
-  if (y) LR_CUDA(cudaMemcpyAsync(y, yd.p, sizeof(float) * n, ok, st));
-  if (d_x) LR_CUDA(cudaMemcpyAsync(d_x, dxd.p, sizeof(float) * 2 * n, ok, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -596,26 +594,23 @@ extern "C" int lrnde_latent_loss(lrnde_ctx* ctx, const float* pred, const float*
   LR_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const size_t n = (size_t)F * T * B, nl = (size_t)L * B;
-  const cudaMemcpyKind ik = host_buffers ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-  const cudaMemcpyKind ok = host_buffers ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  DevBuf pd(ctx, n), dd(ctx, n), md(ctx, n), mud(ctx, nl), lsd(ctx, nl), dpd(ctx, n), dmu(ctx, nl), dls(ctx, nl);
+  CallerBufs io(ctx, host_buffers);   // owned copies: pooled (256-byte aligned) arrays that alias no argument
+  const float* pd = io.copy_in(pred, n);
+  const float* dd = io.copy_in(data, n);
+  const float* md = io.copy_in(mask, n);
+  const float* mud = io.copy_in(mu, nl);
+  const float* lsd = io.copy_in(logsigma2, nl);
+  float* dpd = io.copy_out(d_pred, n);
+  float* dmu = io.copy_out(d_mu, nl);
+  float* dls = io.copy_out(d_logsigma2, nl);
   DevBuf per(ctx, 4 * (size_t)B + 4);
-  LR_CUDA(cudaMemcpyAsync(pd.p, pred, sizeof(float) * n, ik, st));
-  LR_CUDA(cudaMemcpyAsync(dd.p, data, sizeof(float) * n, ik, st));
-  LR_CUDA(cudaMemcpyAsync(md.p, mask, sizeof(float) * n, ik, st));
-  LR_CUDA(cudaMemcpyAsync(mud.p, mu, sizeof(float) * nl, ik, st));
-  LR_CUDA(cudaMemcpyAsync(lsd.p, logsigma2, sizeof(float) * nl, ik, st));
-  latent_loss_kernel<<<(unsigned)B, 256, 0, st>>>(pd.p, dd.p, md.p, mud.p, lsd.p, F * T, L, (int)B, w_kl, (double*)per.p,
-                                                  d_pred ? dpd.p : nullptr, d_mu ? dmu.p : nullptr, dls.p);
+  latent_loss_kernel<<<(unsigned)B, 256, 0, st>>>(pd, dd, md, mud, lsd, F * T, L, (int)B, w_kl, (double*)per.p, dpd, dmu,
+                                                  dls);
   LR_COUNT(ctx);
   LR_CUDA(cudaGetLastError());
   std::vector<double> h(2 * (size_t)B);
   LR_CUDA(cudaMemcpyAsync(h.data(), per.p, sizeof(double) * 2 * B, cudaMemcpyDeviceToHost, st));
-  if (d_pred) LR_CUDA(cudaMemcpyAsync(d_pred, dpd.p, sizeof(float) * n, ok, st));
-  if (d_mu) {
-    LR_CUDA(cudaMemcpyAsync(d_mu, dmu.p, sizeof(float) * nl, ok, st));
-    LR_CUDA(cudaMemcpyAsync(d_logsigma2, dls.p, sizeof(float) * nl, ok, st));
-  }
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   double ll = 0.0, kl = 0.0;
   for (int64_t b = 0; b < B; ++b) { ll += h[2 * b]; kl += h[2 * b + 1]; }

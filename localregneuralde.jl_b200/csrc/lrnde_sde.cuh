@@ -1080,9 +1080,7 @@ extern "C" int lrnde_sde_forward(lrnde_ctx* ctx, const lrnde_model* drift, const
   T->B = B;
   const int D = drift->D;
   const size_t DB = (size_t)D * (size_t)B;
-  const int host = o->host_buffers;
-  const cudaMemcpyKind in_kind = host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-  const cudaMemcpyKind out_kind = host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  CallerBufs io(ctx, o->host_buffers);
 
   // ---- launch shape: S samples per tile, one CTA per SM at most (cooperative launch)
   int n_sm = 0;
@@ -1109,8 +1107,8 @@ extern "C" int lrnde_sde_forward(lrnde_ctx* ctx, const lrnde_model* drift, const
   const int64_t Pf = drift->nparams, Pg = diffusion->nparams;
   T->psf = T->take<float>(Pf);
   T->psg = T->take<float>(Pg);
-  LR_CUDA(cudaMemcpyAsync(T->psf, ps_drift, sizeof(float) * Pf, in_kind, st));
-  LR_CUDA(cudaMemcpyAsync(T->psg, ps_diffusion, sizeof(float) * Pg, in_kind, st));
+  io.copy_in(T->psf, ps_drift, Pf);   // kept by the tape
+  io.copy_in(T->psg, ps_diffusion, Pg);
   size_t budget = (size_t)8 << 30;
   int cap = (int)std::min<size_t>((size_t)o->maxiters, std::max<size_t>(64, budget / (3 * DB * sizeof(float))));
   cap = std::max(cap, 1);
@@ -1128,7 +1126,7 @@ extern "C" int lrnde_sde_forward(lrnde_ctx* ctx, const lrnde_model* drift, const
   T->log_e = T->take<float>(T->log_cap); T->log_a = T->take<unsigned char>(T->log_cap);
   T->out_i = T->take<int>(8); T->out_f = T->take<float>(4);
   LR_CUDA(cudaMemsetAsync(T->out_i, 0, sizeof(int) * 8, st));
-  LR_CUDA(cudaMemcpyAsync(T->tape_u, x, sizeof(float) * DB, in_kind, st));
+  io.copy_in(T->tape_u, x, DB);   // u_0, the first state of the tape
 
   // ---- save times
   std::vector<float> times;
@@ -1218,8 +1216,8 @@ extern "C" int lrnde_sde_forward(lrnde_ctx* ctx, const lrnde_model* drift, const
 
   // ---- outputs
   stats->nsave_out = T->all_steps ? (T->nacc + (o->save_start ? 1 : 0)) : (int)times.size();
-  if (u_save && !times.empty())
-    LR_CUDA(cudaMemcpyAsync(u_save, T->u_save_dev, sizeof(float) * times.size() * DB, out_kind, st));
+  if (!times.empty()) io.copy_out(u_save, T->u_save_dev, times.size() * DB);
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   stats->gpu_launches = (int32_t)(ctx->launches - launches0);
   if (o->keep_tape) *tape_out = T.release();
@@ -1232,9 +1230,9 @@ extern "C" int lrnde_sde_states(lrnde_ctx* ctx, const lrnde_sde_tape* T, int32_t
   if (!ctx || !T || first < 0 || count < 0 || first + count > T->nacc + 1)
     lr_fail(LRNDE_EINVAL, "lrnde_sde_states: range outside the %d stored states", T ? T->nacc + 1 : 0);
   const size_t DB = (size_t)T->nf.D * (size_t)T->B;
-  if (u_out && count)
-    LR_CUDA(cudaMemcpyAsync(u_out, T->tape_u + (size_t)first * DB, sizeof(float) * DB * count,
-                            host_buffers ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, ctx->stream));
+  CallerBufs io(ctx, host_buffers);
+  if (count) io.copy_out(u_out, T->tape_u + (size_t)first * DB, DB * count);
+  io.finish();
   if (t_out) for (int i = 0; i < count; ++i) t_out[i] = T->step_t[first + i];
   LR_CUDA(cudaStreamSynchronize(ctx->stream));
   LR_API_END
@@ -1261,17 +1259,15 @@ extern "C" int lrnde_sde_backward(lrnde_ctx* ctx, lrnde_sde_tape* T, const float
   cudaStream_t st = ctx->stream;
   const int D = T->nf.D;
   const size_t DB = (size_t)D * (size_t)T->B;
-  const int host = T->opts.host_buffers;
+  CallerBufs io(ctx, T->opts.host_buffers);
   // cotangent blocks: one per saved state (all-steps mode: one per returned state, in order)
   int nblk = T->all_steps ? (T->nacc + (T->opts.save_start ? 1 : 0)) : T->nsave_dev;
   std::vector<int> step(std::max(nblk, 1));
   std::vector<float> theta(std::max(nblk, 1), 1.0f);
   const int* step_dev = T->save_step;
   const float* theta_dev = T->save_theta;
-  DevBuf dsave(ctx, std::max<size_t>(1, (size_t)nblk * DB));
-  if (d_u_save && nblk)
-    LR_CUDA(cudaMemcpyAsync(dsave.p, d_u_save, sizeof(float) * nblk * DB,
-                            host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st));
+  DevBuf dsave(ctx, std::max<size_t>(1, (size_t)nblk * DB));   // the kernel reads a zero block for a NULL d_u_save
+  if (d_u_save && nblk) io.copy_in(dsave.p, d_u_save, (size_t)nblk * DB);
   else if (nblk) LR_CUDA(cudaMemsetAsync(dsave.p, 0, sizeof(float) * nblk * DB, st));
   DevBuf stepb(ctx, nblk + 1), thetab(ctx, nblk + 1);
   if (T->all_steps) {
@@ -1286,8 +1282,10 @@ extern "C" int lrnde_sde_backward(lrnde_ctx* ctx, lrnde_sde_tape* T, const float
   LR_CUDA(cudaFuncSetAttribute(sde_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
   const int gstride = T->nf.wfloats + T->ng.wfloats;
   DevBuf gpart(ctx, (size_t)T->grid * gstride);
-  DevBuf dx(ctx, DB);
-  DevBuf dpf(ctx, T->nf.nparams), dpg(ctx, T->ng.nparams);
+  DevBuf dx(ctx, DB);   // the kernel always writes d_x
+  float* dpf = io.copy_out(d_ps_drift, T->nf.nparams);
+  float* dpg = io.copy_out(d_ps_diffusion, T->ng.nparams);
+  io.copy_out(d_x, dx.p, DB);
   SdeBwdP q;
   memset(&q, 0, sizeof(q));
   q.nf = T->nf; q.ng = T->ng; q.tab = T->tab; q.psf = T->psf; q.psg = T->psg;
@@ -1302,15 +1300,12 @@ extern "C" int lrnde_sde_backward(lrnde_ctx* ctx, lrnde_sde_tape* T, const float
   q.eest_reg = T->eest_reg; q.d_reg = d_reg;
   sde_backward_kernel<<<T->grid, SDE_THREADS, smem_b, st>>>(q);
   LR_COUNT(ctx);
-  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(T->nf, gpart.p, gstride, 0, T->grid, dpf.p);
+  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(T->nf, gpart.p, gstride, 0, T->grid, dpf);
   LR_COUNT(ctx);
-  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(T->ng, gpart.p, gstride, T->nf.wfloats, T->grid, dpg.p);
+  sde_grad_reduce_kernel<<<64, 256, 0, st>>>(T->ng, gpart.p, gstride, T->nf.wfloats, T->grid, dpg);
   LR_COUNT(ctx);
   LR_CUDA(cudaGetLastError());
-  const cudaMemcpyKind out_kind = host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  LR_CUDA(cudaMemcpyAsync(d_ps_drift, dpf.p, sizeof(float) * T->nf.nparams, out_kind, st));
-  LR_CUDA(cudaMemcpyAsync(d_ps_diffusion, dpg.p, sizeof(float) * T->ng.nparams, out_kind, st));
-  if (d_x) LR_CUDA(cudaMemcpyAsync(d_x, dx.p, sizeof(float) * DB, out_kind, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   LR_API_END
 }
@@ -1357,21 +1352,21 @@ extern "C" int lrnde_sde_aux_step(lrnde_ctx* ctx, const lrnde_model* drift, cons
   p.tiles_per_cta = (ntiles + max_grid - 1) / max_grid;
   const int grid = (ntiles + p.tiles_per_cta - 1) / p.tiles_per_cta;
   p.t = t; p.dt = dt; p.abstol = abstol; p.reltol = reltol; p.delta = delta;
-  const cudaMemcpyKind in_kind = host_buffers ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-  DevBuf psf(ctx, drift->nparams), psg(ctx, diffusion->nparams), up(ctx, DB), dw(ctx, DB), un(ctx, DB);
+  CallerBufs io(ctx, host_buffers);   // owned copies: pooled (256-byte aligned) arrays that alias no argument
+  p.psf = io.copy_in(ps_drift, drift->nparams);
+  p.psg = io.copy_in(ps_diffusion, diffusion->nparams);
+  p.uprev = io.copy_in(uprev, DB);
+  p.dW = io.copy_in(dW, DB);
+  p.u = io.copy_out(u, DB);
   DevBuf parts(ctx, 2 * (size_t)grid + 2);
-  LR_CUDA(cudaMemcpyAsync(psf.p, ps_drift, sizeof(float) * drift->nparams, in_kind, st));
-  LR_CUDA(cudaMemcpyAsync(psg.p, ps_diffusion, sizeof(float) * diffusion->nparams, in_kind, st));
-  LR_CUDA(cudaMemcpyAsync(up.p, uprev, sizeof(float) * DB, in_kind, st));
-  LR_CUDA(cudaMemcpyAsync(dw.p, dW, sizeof(float) * DB, in_kind, st));
-  p.psf = psf.p; p.psg = psg.p; p.uprev = up.p; p.dW = dw.p; p.u = un.p; p.partials = (double*)parts.p;
+  p.partials = (double*)parts.p;
   LR_CUDA(cudaFuncSetAttribute(sde_aux_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   sde_aux_step_kernel<<<grid, SDE_THREADS, smem, st>>>(p);
   LR_COUNT(ctx);
   LR_CUDA(cudaGetLastError());
   std::vector<double> hp(grid);
   LR_CUDA(cudaMemcpyAsync(hp.data(), parts.p, sizeof(double) * grid, cudaMemcpyDeviceToHost, st));
-  LR_CUDA(cudaMemcpyAsync(u, un.p, sizeof(float) * DB, host_buffers ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+  io.finish();
   LR_CUDA(cudaStreamSynchronize(st));
   double tot = 0.0;
   for (double v : hp) tot += v;

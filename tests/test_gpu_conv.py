@@ -419,6 +419,25 @@ def test_device_resident_tensors_match_host_buffers(pkg):
     b_h, s_h = pkg.batchnorm_forward(xi, bn_ps, state)
     b_d, s_d = pkg.batchnorm_forward(torch.from_numpy(xi).to(dev), torch.from_numpy(bn_ps).to(dev), state)
     assert np.array_equal(b_d.cpu().numpy(), b_h) and np.array_equal(s_d["running"].cpu().numpy(), s_h["running"])
+    # the pullbacks; d_y is passed as the very tensor the library reads (the wrappers' WHCN -> BCHW conversion is a
+    # no-op on a permuted contiguous tensor), so it must come back untouched although both calls transform a copy
+    # of it in place
+    def whcn_view(a):
+        return torch.from_numpy(np.ascontiguousarray(a.transpose(3, 2, 1, 0))).to(dev).permute(3, 2, 1, 0)
+    gy = rng.standard_normal((8, 8, 5, 4)).astype(np.float32)
+    gy_d = whcn_view(gy)
+    gy_before = gy_d.clone()
+    cx_h, cp_h = pkg.conv2d_backward(xi, pa, gy, activation="gelu")
+    cx_d, cp_d = pkg.conv2d_backward(torch.from_numpy(xi).to(dev), torch.from_numpy(pa).to(dev), gy_d, activation="gelu")
+    assert np.array_equal(cx_d.cpu().numpy(), cx_h) and np.array_equal(cp_d.cpu().numpy(), cp_h)
+    assert torch.equal(gy_d, gy_before)
+    gb = rng.standard_normal(xi.shape).astype(np.float32)
+    gb_d = whcn_view(gb)
+    gb_before = gb_d.clone()
+    bx_h, bp_h = pkg.batchnorm_backward(xi, bn_ps, gb, activation="relu")
+    bx_d, bp_d = pkg.batchnorm_backward(torch.from_numpy(xi).to(dev), torch.from_numpy(bn_ps).to(dev), gb_d, activation="relu")
+    assert np.array_equal(bx_d.cpu().numpy(), bx_h) and np.array_equal(bp_d.cpu().numpy(), bp_h)
+    assert torch.equal(gb_d, gb_before)
 
 
 @pytest.mark.parametrize("mode,kwargs", [("unbiased", dict(saveat=[0.25, 0.6, 1.0])), ("biased", {}), ("none", dict(saveat=[0.5, 1.0]))])

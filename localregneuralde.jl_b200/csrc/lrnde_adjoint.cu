@@ -13,18 +13,20 @@
 
 #include "lrnde_fused_dev.cuh"
 
-// hidden-space work arrays ([B][LR_ZROW] each)
+// hidden-space work arrays ([B][LR_ZROW] each, padded to whole 64-sample tiles).  Written by: interp = (0), pre = (1),
+// chain = (2); stage 7 of an attempt is stage 1 of the next ring slot.
 enum {
-  LA_ALPHA = 0,   // + slot: W2^T lambda of the ring slot
-  LA_S1 = 2,      // + 3 * slot + {0: delta_1, 1: [h_1;t;1], 2: c_1}: stage 1 (FSAL) of the ring slot
-  LA_DEL = 8,     // + j - 2, j = 2..6: delta_j
-  LA_CC = 13,     // + j - 2: c_j (rows Kaug, Kaug + 1 = tau_j, 1)
-  LA_HH = 18,     // + j - 2: [h_j ; tau_j ; 1]
-  LA_EPS = 23,    // + j - 2, j = 2..7: eps_j = sum_i a_ji delta_i  (eps_7 = Delta_b)
-  LA_DBT = 29,    // Delta_btilde
-  LA_HBB = 30,    // sum_j b_j [h_j;tau_j;1]
-  LA_HBT = 31,    // sum_j btilde_j [h_j;tau_j;1]
-  LA_NARR = 32
+  LA_ALPHA = 0,   // + slot: W2^T lambda of the ring slot (pre in single mode, chain)
+  LA_S1 = 2,      // + 3 * slot + {0: delta_1 (pre single / chain), 1: [h_1;t;1] (pre), 2: c_1 (interp)}: stage 1 (FSAL)
+  LA_DEL = 8,     // + j - 2, j = 2..6: delta_j (chain)
+  LA_CC = 13,     // + j - 2: c_j (rows Kaug, Kaug + 1 = tau_j, 1) (interp)
+  LA_HH = 18,     // + j - 2: [h_j ; tau_j ; 1] (pre)
+  LA_EPS = 23,    // + j - 2, j = 2..7: eps_j = sum_i a_ji delta_i  (eps_7 = Delta_b) (chain)
+  LA_DBT = 29,    // Delta_btilde (chain)
+  LA_HBB = 30,    // sum_j b_j [h_j;tau_j;1] (pre)
+  LA_HBT = 31,    // sum_j btilde_j [h_j;tau_j;1] (pre)
+  LA_SS = 32,     // + j - 2, j = 2..7: s_j = act'(p_j), 0 in rows >= H (pre)
+  LA_NARR = 38
 };
 
 #ifdef LRNDE_UMMA_TRACE
@@ -46,14 +48,15 @@ using namespace fused;
 template <int ACT>
 __device__ __forceinline__ void act_pair(float x, float& h, float& s) {
   if (ACT == ACT_TANH) { h = tanhf(x); s = 1.0f - h * h; }
+  else if (ACT == ACT_SIGMOID) { h = 1.0f / (1.0f + expf(-x)); s = h * (1.0f - h); }
   else { h = lr_act(ACT, x); s = lr_dact(ACT, x); }
 }
 
 // ---------------------------------------------------------------------------------------------------------
 // (0) interpolant kernel: c_j = C_n + dt_n sum_i b_i(theta_j) H(k_i), the dense interpolant of the forward solution in
 // hidden space at every stage time of the attempt, written as the stored copy of c_j (rows Kaug, Kaug + 1 = tau_j, 1,
-// the rest 0).  It does not depend on lambda, so it runs ahead of the chain kernel over the whole batch, and the
-// stages that fall in the same forward interval share one read of that interval's 8 tape arrays.
+// the rest 0).  It does not depend on lambda, so it runs over the whole batch ahead of the pre kernel, and the stages
+// that fall in the same forward interval share one read of that interval's 8 tape arrays.
 // Thread = 4 hidden rows of one sample (a warp reads one sample's row of 512 bytes).
 // ---------------------------------------------------------------------------------------------------------
 struct AInterpP {
@@ -124,28 +127,11 @@ __global__ void __launch_bounds__(256) adj_interp_kernel(AInterpP p) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// (1) chain kernel: one CTA = 64 samples as two independent halves of 32 (while the tensor core works for one half
-// the other half's warps do their element-wise arithmetic).  Thread of a compute warp = one hidden row x 16 samples.
-// TMEM: [Mz hi | Mz lo | Mh^T hi | Mh^T lo] as A operands (8 KS columns each), then one 32-column accumulator per half
-// (p = Mz c first, Mh^T eps once p has been read).  c_j comes from adj_interp_kernel's stored copy.
+// Shared by the two tensor-core kernels below: one CTA works on 64 samples as two independent halves of 32 (while the
+// tensor core works for one half the other half's warps do their element-wise arithmetic).  Thread of a compute warp =
+// one hidden row x 16 samples; an [M = 128 rows] x [K = KS * 8] matrix sits in tensor memory as the A operand (hi and lo
+// images, 8 KS columns each), the 32-sample B operand tile is formed in shared memory.
 // ---------------------------------------------------------------------------------------------------------
-constexpr int kTapeBufs = 3;                       // ring of [64 samples][LR_ZROW] tiles of c_j
-constexpr int kTapeBufBytes = kNT * LR_ZROW * 4;   // 32 KB
-struct AChainP {
-  SolveDev* S;
-  int single;            // 1: stage-1 quantities of the current state (alpha from alpha_in, time / interpolant yint[0])
-  const float* Mz;
-  const float* w1t;      // layer-1 time column (nullptr without TDChain)
-  const float* b1;
-  const float* Zx;
-  const float* alpha_in;
-  float* ws;
-  size_t zlen;
-  float* hbuf;
-  uint32_t unit_bytes;
-  int B, H, td, Kaug, KS, nfull, ntail, passes;
-};
-
 __device__ __forceinline__ void issue_group(uint32_t d, uint32_t a_hi, uint32_t a_lo, uint32_t b0, int nfull, int ntail,
                                             int passes, uint32_t idesc) {
   uint32_t first = 0u;
@@ -175,44 +161,132 @@ __device__ __forceinline__ void issue_group(uint32_t d, uint32_t a_hi, uint32_t 
   }
 }
 
+// The per-thread view of a compute warp (warps 2 .. 17): TMEM lane quarter q, hidden row hrow, half cg and the first of
+// its 16 samples inside the tile; tile_put16 writes the thread's 16 values as (tile row = sample, k = hrow) of a [hi | lo]
+// operand image: byte offset = oA + r * oS + ((osw ^ m(r)) << 4) with m(r) = r & 7 (SWIZZLE_128B chunks of 32 k) or
+// (r >> 2) & 1 (SWIZZLE_32B K-steps of the tail); lo image at + oLo.
+struct ComputeLane {
+  int q, cg, hrow, rbase;
+  bool rowv, rowc, in_full, in_img;
+  uint32_t oA, osw;
+  __device__ __forceinline__ ComputeLane(int warp, int lane, int H, int Kaug, int KS, int nfull) {
+    q = warp & 3;
+    const int sub = (warp - 2) >> 2;
+    cg = sub >> 1;
+    hrow = q * 32 + lane;
+    rbase = (sub & 1) * 16;
+    rowv = hrow < H;
+    rowc = hrow < Kaug;
+    in_full = hrow < nfull * 32;
+    in_img = hrow < KS * 8;
+    if (in_full) {
+      osw = (uint32_t)(lane >> 2);
+      oA = (uint32_t)(q * 8192 + (lane & 3) * 4) + (uint32_t)rbase * 128u;
+    } else {
+      const int kt = hrow - nfull * 32, t = kt >> 3, kk = kt & 7;
+      osw = (uint32_t)((kk >> 2) & 1);
+      oA = (uint32_t)(nfull * 8192 + t * 2048 + (kk & 3) * 4) + (uint32_t)rbase * 32u;
+    }
+  }
+  __device__ __forceinline__ void tile_put16(uint8_t* tile, const float (&val)[16], int passes) const {
+    if (!in_img) return;
+    const uint32_t oS = in_full ? 128u : 32u, oLo = in_full ? 4096u : 1024u;
+    // tf32 split without branches: passes == 1 keeps the value (no rounding, lo = 0)
+    const uint32_t rnd = (passes == 3) ? 0x1000u : 0u, msk = (passes == 3) ? 0xFFFFE000u : 0xFFFFFFFFu;
+#pragma unroll
+    for (int i = 0; i < 16; ++i) {
+      const uint32_t m = in_full ? (uint32_t)(i & 7) : (uint32_t)((i >> 2) & 1);
+      const uint32_t o = oA + (uint32_t)i * oS + ((osw ^ m) << 4);
+      const float hi = __uint_as_float((__float_as_uint(val[i]) + rnd) & msk);
+      const float lo = __uint_as_float((__float_as_uint(val[i] - hi) + rnd) & msk);
+      *reinterpret_cast<float*>(tile + o) = hi;
+      *reinterpret_cast<float*>(tile + o + oLo) = lo;
+    }
+  }
+};
+
+// A operand -> tensor memory: element (hrow, k) of a [128][128] fp32 matrix, k < KS * 8, as hi at column k and lo at
+// column 8 KS + k (warp `sub` of a lane quarter writes the K-steps sub, sub + 4, ...).  transposed: Mh^T = Mz[:H, :H]^T.
+__device__ __forceinline__ void a_operand_to_tmem(const float* Mz, bool transposed, int H, int KS, int passes, int warp,
+                                                  int hrow, uint32_t tlane) {
+  const int sub = (warp - 2) >> 2;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int ks = sub + 4 * j;
+    if (ks < KS) {
+      float a[8], hi[8], lo[8];
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const int k = ks * 8 + e;
+        a[e] = transposed ? ((hrow < H && k < H) ? __ldg(Mz + k * 128 + hrow) : 0.0f)   // Mh^T[hrow][k] = Mz[k][hrow]
+                          : __ldg(Mz + hrow * 128 + k);                                  // Mz[hrow][k]  (zero padded)
+      }
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        if (passes == 3) { hi[e] = tf32_rna(a[e]); lo[e] = tf32_rna(a[e] - hi[e]); }
+        else { hi[e] = a[e]; lo[e] = 0.0f; }
+      }
+      tmem_st8(tlane + (uint32_t)(ks * 8), hi);
+      tmem_st8(tlane + (uint32_t)(8 * KS + ks * 8), lo);
+    }
+  }
+  tmem_st_wait();
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// (1) pre kernel: everything of a stage that does not depend on lambda, over the whole batch:
+//       p_j = Zx + Mz c_j + w1t tau_j + b1,  [h_j ; tau_j ; 1],  s_j = act'(p_j)   (rows >= H of s_j are 0)
+//     and, per sample, sum_j b_j [h_j;tau_j;1] and sum_j btilde_j [h_j;tau_j;1] over the seven stages of the attempt
+//     (stage 1 from the ring slot).  A CTA takes whole 64-sample tiles (all their stages, so the two sums stay in
+//     registers), tile = blockIdx.x + i * gridDim.x; the stages are independent, so the c tile of the next stage is
+//     formed while the tensor core works on the current one (two [hi | lo] tiles and two accumulators per half).
+//     TMEM: [Mz hi | Mz lo] (8 KS columns each), then four 32-column accumulators (half cg, buffer b at 32 (2 cg + b)).
+//     SINGLE (stage 1 of the current state, c_1 from yint[0]): also delta_1 = s_1 .* alpha_in and alpha of the slot.
+// ---------------------------------------------------------------------------------------------------------
+struct APreP {
+  SolveDev* S;
+  const float* Mz;
+  const float* w1t;      // layer-1 time column (nullptr without TDChain)
+  const float* b1;
+  const float* Zx;
+  const float* alpha_in;
+  float* ws;
+  size_t zlen;
+  int H, td, Kaug, KS, nfull, ntail, passes, ntiles;
+};
+
 template <int ACT, bool SINGLE>
-__global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
+__global__ void __launch_bounds__(kThreads, 1) adj_pre_kernel(APreP p) {
   SolveDev* S = p.S;
   if (SINGLE ? S->failed : S->done) return;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  __shared__ uint64_t a_ready, bfull[2], pdone[2], pread[2], xdone[2], out_full, tfull[kTapeBufs], tempty[kTapeBufs];
+  __shared__ uint64_t a_ready, bfull[2][2], pdone[2][2];
   __shared__ uint32_t tmem_slot;
-  __shared__ LinComb sd[6], sy[7];
-  __shared__ float s_bt[7];
+  __shared__ float s_tau[6], s_cb[7], s_ct[7];
   __shared__ int s_slot, s_next;
 
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
   const int lane = threadIdx.x & 31;
-  const int n0 = blockIdx.x * kNT;
   const int nst = SINGLE ? 1 : 6;
+  const int nk = ((p.ntiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x) * nst;   // stages of this CTA
   const uint32_t tileB = (uint32_t)(p.nfull * 8192 + p.ntail * 2048);   // [hi | lo] images of a 32-sample operand tile
-  uint8_t* tC[2] = {smem, smem + tileB};
-  uint8_t* tE[2] = {smem + 2 * (size_t)tileB, smem + 3 * (size_t)tileB};
-  uint8_t* tbuf = smem + 4 * (size_t)tileB;        // kTapeBufs tape tiles (tileB is a multiple of 1024)
+  auto tile = [&](int cg, int b) { return smem + (size_t)(2 * cg + b) * tileB; };
 
   if (threadIdx.x == 0) {
     mbar_init(&a_ready, (uint32_t)kEpiWarps);
-    mbar_init(&out_full, (uint32_t)kEpiWarps);
-    for (int b = 0; b < kTapeBufs; ++b) { mbar_init(&tfull[b], 1u); mbar_init(&tempty[b], (uint32_t)kEpiWarps); }
-    for (int c = 0; c < 2; ++c) {
-      mbar_init(&bfull[c], (uint32_t)(kEpiWarps / 2));
-      mbar_init(&pdone[c], 1u);
-      mbar_init(&pread[c], (uint32_t)(kEpiWarps / 2));
-      mbar_init(&xdone[c], 1u);
-    }
+    for (int c = 0; c < 2; ++c)
+      for (int b = 0; b < 2; ++b) { mbar_init(&bfull[c][b], (uint32_t)(kEpiWarps / 2)); mbar_init(&pdone[c][b], 1u); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     s_slot = S->slot; s_next = (S->slot + 1) % S->cap;
   }
-  if (threadIdx.x >= 64 && threadIdx.x < 70) sd[threadIdx.x - 64] = S->st[threadIdx.x - 64];
-  if (threadIdx.x >= 96 && threadIdx.x < 103) sy[threadIdx.x - 96] = S->yint[threadIdx.x - 96];
-  if (threadIdx.x >= 128 && threadIdx.x < 135) s_bt[threadIdx.x - 128] = S->err.coef[threadIdx.x - 128];
-  if (warp == 1) {
+  if (threadIdx.x >= 32 && threadIdx.x < 32 + nst) s_tau[threadIdx.x - 32] = S->yint[SINGLE ? 0 : threadIdx.x - 31].t;
+  if (threadIdx.x >= 64 && threadIdx.x < 71) {   // weights of stage s = 0..6 in the two sums (b_7 = 0)
+    const int s = threadIdx.x - 64;
+    s_cb[s] = (s < 6) ? S->st[5].coef[s] : 0.0f;
+    s_ct[s] = S->err.coef[s];
+  }
+  if (warp == 1) {   // 16 KS + 128 <= 352 columns (KS <= 14)
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(512u)
                  : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -221,330 +295,120 @@ __global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = tmem_slot;
-  const uint32_t c_acc = tmem_base + (uint32_t)(32 * p.KS);
+  const uint32_t c_acc = tmem_base + (uint32_t)(16 * p.KS);
   auto arr = [&](int idx) -> float* { return p.ws + (size_t)idx * p.zlen; };
-  const bool tr = (threadIdx.x == 64) && !SINGLE;
-  if (tr) ATRACE(0, 0);
 
-  if (warp == 0) {
-    // ---------------- c_j in: the stored copy adj_interp_kernel wrote, one tile per stage, bulk-copied onto a ring
-    // (it does not depend on lambda: it runs ahead)
-    {
-      const int nvalid = min(kNT, p.B - n0);
-      const uint32_t bytes = (uint32_t)nvalid * LR_ZROW * 4u;
-      for (int it = 0; it < nst; ++it) {
-        const int b = it % kTapeBufs;
-        const float* src = SINGLE ? arr(LA_S1 + 3 * s_slot + 2) : (it == 5 ? arr(LA_S1 + 3 * s_next + 2) : arr(LA_CC + it));
-        mbar_wait(&tempty[b], (uint32_t)(((it / kTapeBufs) & 1) ^ 1));
-        if (elect_one_sync()) {
-          mbar_arrive_expect_tx(&tfull[b], bytes);
-          bulk_g2s(tbuf + (size_t)b * kTapeBufBytes, src + (size_t)n0 * LR_ZROW, bytes, &tfull[b]);
-        }
-        __syncwarp();
-      }
-    }
-    // ---------------- Delta_b / Delta_bt operand images out (units of 16 samples for the lambda GEMM)
-    if (!SINGLE) {
-      mbar_wait(&out_full, 0);
-      if (elect_one_sync()) {
-        for (int sg = 0; sg < 4; ++sg) {
-          uint8_t* g = reinterpret_cast<uint8_t*>(p.hbuf) + ((size_t)blockIdx.x * 4 + sg) * p.unit_bytes;
-          const int cg = sg >> 1, half = sg & 1;
-          for (int c = 0; c < p.nfull; ++c)
-            for (int lo = 0; lo < 2; ++lo) {
-              bulk_s2g(g + (size_t)c * 8192 + lo * 4096, tE[cg] + (size_t)c * 8192 + lo * 4096 + half * 2048, 2048);
-              bulk_s2g(g + (size_t)c * 8192 + lo * 4096 + 2048, tC[cg] + (size_t)c * 8192 + lo * 4096 + half * 2048, 2048);
-            }
-          for (int t = 0; t < p.ntail; ++t)
-            for (int lo = 0; lo < 2; ++lo) {
-              const size_t o = (size_t)p.nfull * 8192 + (size_t)t * 2048 + lo * 1024;
-              bulk_s2g(g + o, tE[cg] + o + half * 512, 512);
-              bulk_s2g(g + o + 512, tC[cg] + o + half * 512, 512);
-            }
-        }
-        bulk_commit();
-        bulk_wait0();
-      }
-      __syncwarp();
-    }
-  } else if (warp == 1) {
-    // ---------------- tcgen05.mma issue (M = 128 hidden rows x N = 32 samples, A from tensor memory)
+  if (warp == 1) {
+    // ---------------- tcgen05.mma issue (M = 128 hidden rows x N = 32 samples, A from tensor memory): p = Mz c
     constexpr uint32_t idesc = make_idesc(128, kNT / 2);
     mbar_wait(&a_ready, 0);
     tc_fence_after();
     const uint32_t mz_hi = tmem_base, mz_lo = tmem_base + (uint32_t)(8 * p.KS);
-    const uint32_t mt_hi = tmem_base + (uint32_t)(16 * p.KS), mt_lo = tmem_base + (uint32_t)(24 * p.KS);
-    for (int st = 0; st < nst; ++st) {
-      const uint32_t ph = (uint32_t)(st & 1);
+    for (int k = 0; k < nk; ++k) {
+      const int b = k & 1;
       for (int cg = 0; cg < 2; ++cg) {
-        mbar_wait(&bfull[cg], ph);
+        mbar_wait(&bfull[cg][b], (uint32_t)((k >> 1) & 1));
         tc_fence_after();
         if (elect_one_sync()) {
-          if (cg == 0 && !SINGLE) ATRACE(7, st);
-          issue_group(c_acc + (uint32_t)(cg * 32), mz_hi, mz_lo, smem_u32(tC[cg]), p.nfull, p.ntail, p.passes, idesc);
-          mma_commit(&pdone[cg]);
-          if (cg == 0 && !SINGLE) ATRACE(8, st);
+          issue_group(c_acc + (uint32_t)((2 * cg + b) * 32), mz_hi, mz_lo, smem_u32(tile(cg, b)), p.nfull, p.ntail, p.passes,
+                      idesc);
+          mma_commit(&pdone[cg][b]);
         }
         __syncwarp();
       }
-      if (!SINGLE) {
-        for (int cg = 0; cg < 2; ++cg) {
-          mbar_wait(&pread[cg], ph);
-          tc_fence_after();
-          if (elect_one_sync()) {
-            issue_group(c_acc + (uint32_t)(cg * 32), mt_hi, mt_lo, smem_u32(tE[cg]), p.nfull, p.ntail, p.passes, idesc);
-            mma_commit(&xdone[cg]);
-          }
-          __syncwarp();
-        }
-      }
     }
-  } else {
-    // ---------------- compute warps: lane = hidden row, registers = 16 samples
-    const int q = warp & 3, sub = (warp - 2) >> 2;
-    const int cg = sub >> 1;
-    const int hrow = q * 32 + lane;
-    const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16);
-    const int rbase = (sub & 1) * 16;              // first row of this thread inside its half's 32-row tiles
-    const int nb = n0 + cg * 32 + rbase;           // first sample of this thread
-    const bool rowv = hrow < p.H;
-    const bool rowc = hrow < p.Kaug;
-    // A operands -> tensor memory (warp `sub` of a lane quarter writes the K-steps sub, sub + 4, ...)
-    {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int ks = sub + 4 * j;
-        if (ks < p.KS) {
-          float a1[8], a2[8], hi[8], lo[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) {
-            const int k = ks * 8 + e;
-            a1[e] = __ldg(p.Mz + hrow * 128 + k);                                    // Mz[hrow][k]  (zero padded)
-            a2[e] = (rowv && k < p.H) ? __ldg(p.Mz + k * 128 + hrow) : 0.0f;           // Mh^T[hrow][k] = Mz[k][hrow]
-          }
-#pragma unroll
-          for (int e = 0; e < 8; ++e) {
-            if (p.passes == 3) { hi[e] = tf32_rna(a1[e]); lo[e] = tf32_rna(a1[e] - hi[e]); }
-            else { hi[e] = a1[e]; lo[e] = 0.0f; }
-          }
-          tmem_st8(tlane + (uint32_t)(ks * 8), hi);
-          tmem_st8(tlane + (uint32_t)(8 * p.KS + ks * 8), lo);
-#pragma unroll
-          for (int e = 0; e < 8; ++e) {
-            if (p.passes == 3) { hi[e] = tf32_rna(a2[e]); lo[e] = tf32_rna(a2[e] - hi[e]); }
-            else { hi[e] = a2[e]; lo[e] = 0.0f; }
-          }
-          tmem_st8(tlane + (uint32_t)(16 * p.KS + ks * 8), hi);
-          tmem_st8(tlane + (uint32_t)(24 * p.KS + ks * 8), lo);
-        }
-      }
-    }
-    tmem_st_wait();
+  } else if (warp >= 2) {
+    const ComputeLane L(warp, lane, p.H, p.Kaug, p.KS, p.nfull);
+    const uint32_t tlane = tmem_base + ((uint32_t)(L.q * 32) << 16);
+    a_operand_to_tmem(p.Mz, false, p.H, p.KS, p.passes, warp, L.hrow, tlane);
     tc_fence_before();
     __syncwarp();
     if (lane == 0) mbar_arrive(&a_ready);
-    if (tr) ATRACE(0, 1);
 
-    // operand-image position of (tile row r, k = hrow): byte offset = oA + r * oS + ((osw ^ m(r)) << 4) with
-    // m(r) = r & 7 (SWIZZLE_128B chunks of 32 k) or (r >> 2) & 1 (SWIZZLE_32B K-steps of the tail); lo image at + oLo
-    const bool in_full = hrow < p.nfull * 32;
-    const bool in_img = hrow < p.KS * 8;
-    uint32_t oA, oS, oLo, osw;
-    if (in_full) {
-      oS = 128u; oLo = 4096u; osw = (uint32_t)(lane >> 2);
-      oA = (uint32_t)(q * 8192 + (lane & 3) * 4) + (uint32_t)rbase * oS;
-    } else {
-      const int kt = hrow - p.nfull * 32, t = kt >> 3, kk = kt & 7;
-      oS = 32u; oLo = 1024u; osw = (uint32_t)((kk >> 2) & 1);
-      oA = (uint32_t)(p.nfull * 8192 + t * 2048 + (kk & 3) * 4) + (uint32_t)rbase * oS;
-    }
-    // tf32 split without branches: passes == 1 keeps the value (no rounding, lo = 0)
-    const uint32_t rnd = (p.passes == 3) ? 0x1000u : 0u, msk = (p.passes == 3) ? 0xFFFFE000u : 0xFFFFFFFFu;
-    auto tile_put16 = [&](uint8_t* tile, const float (&val)[16]) {
-      if (!in_img) return;
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const uint32_t m = in_full ? (uint32_t)(i & 7) : (uint32_t)((i >> 2) & 1);
-        const uint32_t o = oA + (uint32_t)i * oS + ((osw ^ m) << 4);
-        const float hi = __uint_as_float((__float_as_uint(val[i]) + rnd) & msk);
-        const float lo = __uint_as_float((__float_as_uint(val[i] - hi) + rnd) & msk);
-        *reinterpret_cast<float*>(tile + o) = hi;
-        *reinterpret_cast<float*>(tile + o + oLo) = lo;
-      }
-    };
-    const float w1t = (p.td && rowv && p.w1t) ? p.w1t[hrow] : 0.0f;
-    const float b1 = rowv ? p.b1[hrow] : 0.0f;
+    const float w1t = (p.td && L.rowv && p.w1t) ? p.w1t[L.hrow] : 0.0f;
+    const float b1 = L.rowv ? p.b1[L.hrow] : 0.0f;
     const int slot = s_slot, next = s_next;
-    const float dt = sd[0].scale;
-    const float* alpha_n = SINGLE ? p.alpha_in : arr(LA_ALPHA + slot);
-    // element of (first sample, this row) in a [Bpad][LR_ZROW] array.  The work arrays are padded to whole 64-sample
-    // tiles, so samples beyond B are computed and stored like the others (never read back): no bounds tests below
-    const size_t e0 = (size_t)nb * LR_ZROW + hrow;
-    uint8_t* const tCc = tC[cg];
-    uint8_t* const tEc = tE[cg];
-    const float* ring_row = reinterpret_cast<const float*>(tbuf) + (cg * 32 + rbase) * LR_ZROW + hrow;
-
-    float c[16], ep[16], dprev[16];
+    // element of (first sample of this thread, this row) for the k-th stage of the CTA.  The work arrays are padded to
+    // whole 64-sample tiles, so samples beyond B are computed and stored like the others (never read back)
+    auto e0_of = [&](int k) -> size_t {
+      const int t = (int)blockIdx.x + (k / nst) * (int)gridDim.x;
+      return (size_t)(t * kNT + L.cg * 32 + L.rbase) * LR_ZROW + L.hrow;
+    };
+    // c_j: adj_interp_kernel's stored copy
+    auto c_src = [&](int j) -> const float* {
+      return SINGLE ? arr(LA_S1 + 3 * slot + 2) : (j == 5 ? arr(LA_S1 + 3 * next + 2) : arr(LA_CC + j));
+    };
+    float c[16], zx[16], v[16], hb[16], ht[16];
+    auto put_stage = [&](int k) {   // c of the k-th stage -> operand tile, then hand it to the MMA warp
+      const float* src = c_src(k % nst) + e0_of(k);
 #pragma unroll
-    for (int i = 0; i < 16; ++i) { c[i] = 0.0f; ep[i] = 0.0f; dprev[i] = 0.0f; }
-    if (!SINGLE && rowv) {   // delta_1 (FSAL) of the current state
-      const float* d1 = arr(LA_S1 + 3 * slot + 0) + e0;
-#pragma unroll
-      for (int i = 0; i < 16; ++i) dprev[i] = __ldcg(d1 + (size_t)i * LR_ZROW);
-    }
-    float v[16], ss[16];
-    // software pipeline: iteration jj runs the front of stage jj (operand tiles), then the lambda-independent part of
-    // stage jj + 1 (known part of eps) while the tensor core works, then the back of stage jj (p, activation, alpha,
-    // delta).  jj = -1 only prefetches.
-    for (int jj = -1; jj < nst; ++jj) {
-      const LinComb& yd = SINGLE ? sy[0] : sy[jj < 0 ? 1 : jj + 1];
-      const float tau = yd.t;
-      const bool last = (!SINGLE && jj == 5);
-      float* dst_del = SINGLE ? arr(LA_S1 + 3 * slot + 0) : (last ? arr(LA_S1 + 3 * next + 0) : arr(LA_DEL + max(jj, 0)));
-      float* dst_hh = SINGLE ? arr(LA_S1 + 3 * slot + 1) : (last ? arr(LA_S1 + 3 * next + 1) : arr(LA_HH + max(jj, 0)));
-      if (jj >= 0) {
-        if (tr) ATRACE(1, jj);
-        // ---- operand tiles: c_j (dense interpolant of the forward solution in hidden space, adj_interp_kernel) from
-        //      the ring, and eps_j = (partial sum prefetched during the previous stage) + a_{j,j-1} delta_{j-1}
-        {
-          const int b = jj % kTapeBufs;
-          mbar_wait(&tfull[b], (uint32_t)((jj / kTapeBufs) & 1));
-          const float* tb = ring_row + (size_t)b * (kTapeBufBytes / 4);
-#pragma unroll
-          for (int i = 0; i < 16; ++i) c[i] = rowc ? tb[i * LR_ZROW] : 0.0f;
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&tempty[b]);
-        }
-        tile_put16(tCc, c);
-        if (!SINGLE) {
-          const float cl = sd[jj].coef[jj];
-          float* dst_eps = arr(LA_EPS + jj) + e0;
-#pragma unroll
-          for (int i = 0; i < 16; ++i) { v[i] = fmaf(cl, dprev[i], ep[i]); dst_eps[(size_t)i * LR_ZROW] = v[i]; }
-          tile_put16(tEc, v);
-        }
-        tc_fence_before();
-        fence_proxy_async();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&bfull[cg]);
-        if (tr) ATRACE(2, jj);
-      }
-      if (jj + 1 < nst) {
-        if (!SINGLE && jj >= 0) {   // known part of eps_{j+1}: delta_1 .. delta_j (the newest one is in registers)
-#pragma unroll
-          for (int i = 0; i < 16; ++i) ep[i] = sd[jj + 1].coef[jj] * dprev[i];
-          if (rowv) {
-            for (int s = 0; s < jj; ++s) {
-              const float* src = ((s == 0) ? arr(LA_S1 + 3 * slot + 0) : arr(LA_DEL + s - 1)) + e0;
-              const float cf = sd[jj + 1].coef[s];
-#pragma unroll
-              for (int i = 0; i < 16; ++i) ep[i] = fmaf(cf, __ldcg(src + (size_t)i * LR_ZROW), ep[i]);
-            }
-          }
-        }
-      }
-      if (jj >= 0) {
-        if (tr) ATRACE(3, jj);
-#pragma unroll
-        for (int i = 0; i < 16; ++i) ss[i] = rowv ? __ldcg(p.Zx + e0 + (size_t)i * LR_ZROW) : 0.0f;   // Zx
-        // ---- p_j = Zx + Mz c_j + w1t tau_j + b1 ; h_j, s_j
-        mbar_wait(&pdone[cg], (uint32_t)(jj & 1));
-        if (tr) ATRACE(4, jj);
-        tc_fence_after();
-        tmem_ld16(c_acc + ((uint32_t)(q * 32) << 16) + (uint32_t)(cg * 32 + rbase), v);
-        tc_fence_before();
-        __syncwarp();
-        if (!SINGLE && lane == 0) mbar_arrive(&pread[cg]);
-        const float hconst = (p.td && hrow == p.H) ? tau : ((hrow == p.H + p.td) ? 1.0f : 0.0f);
-        const float pb = p.td ? fmaf(w1t, tau, b1) : b1;
+      for (int i = 0; i < 16; ++i) c[i] = L.rowc ? __ldcg(src + (size_t)i * LR_ZROW) : 0.0f;
+      L.tile_put16(tile(L.cg, k & 1), c, p.passes);
+      tc_fence_before();
+      fence_proxy_async();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&bfull[L.cg][k & 1]);
+    };
+    if (nk > 0) put_stage(0);
+    for (int k = 0; k < nk; ++k) {
+      const int j = k % nst;
+      const size_t e0 = e0_of(k);
+      if (!SINGLE && j == 0) {   // the two sums start with stage 1 (FSAL) of the ring slot
+        const float* h1 = arr(LA_S1 + 3 * slot + 1) + e0;
 #pragma unroll
         for (int i = 0; i < 16; ++i) {
-          float h, sg;
-          act_pair<ACT>(v[i] + ss[i] + pb, h, sg);
-          ss[i] = rowv ? sg : 0.0f;
-          dst_hh[e0 + (size_t)i * LR_ZROW] = rowv ? h : hconst;
-        }
-        // ---- alpha_j = alpha_n - dt Mh^T eps_j ; delta_j = s_j .* alpha_j
-        float an[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) an[i] = rowv ? __ldcg(alpha_n + e0 + (size_t)i * LR_ZROW) : 0.0f;
-        if (tr) ATRACE(5, jj);
-        if (!SINGLE) {
-          mbar_wait(&xdone[cg], (uint32_t)(jj & 1));
-          if (tr) ATRACE(6, jj);
-          tc_fence_after();
-          tmem_ld16(c_acc + ((uint32_t)(q * 32) << 16) + (uint32_t)(cg * 32 + rbase), v);
-          tc_fence_before();
-        }
-        float* dst_alpha = (SINGLE ? arr(LA_ALPHA + slot) : arr(LA_ALPHA + next)) + e0;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          const float aj = SINGLE ? an[i] : fmaf(-dt, v[i], an[i]);
-          dprev[i] = ss[i] * aj;
-          dst_del[e0 + (size_t)i * LR_ZROW] = dprev[i];
-          if (SINGLE || last) dst_alpha[(size_t)i * LR_ZROW] = rowv ? aj : 0.0f;
+          const float hv = L.rowc ? __ldcg(h1 + (size_t)i * LR_ZROW) : 0.0f;
+          hb[i] = fmaf(s_cb[0], hv, 0.0f);
+          ht[i] = fmaf(s_ct[0], hv, 0.0f);
         }
       }
-    }
-    if (tr) ATRACE(0, 3);
-    if (!SINGLE) {
-      // ---- Delta_bt = sum_j btilde_j delta_j ; sum_j b_j H_j ; sum_j btilde_j H_j  (stage 7 in registers / own stores)
-      const LinComb& d7 = sd[5];   // coef = a_7i = b_i
-      // which = 0: delta_j, 1: [h_j;tau_j;1]; three source arrays per round trip
-      auto gather3 = [&](int s0, int ns, int which, float (&t)[3][16]) {
+      if (k + 1 < nk) put_stage(k + 1);   // the next stage's tile while the tensor core works on this one
 #pragma unroll
-        for (int k = 0; k < 3; ++k) {
-          const int s = min(s0 + k, 6);
-          const float* src = ((s == 0) ? arr(LA_S1 + 3 * slot + which)
-                                       : (s == 6 ? arr(LA_S1 + 3 * next + which) : arr((which ? LA_HH : LA_DEL) + s - 1))) + e0;
+      for (int i = 0; i < 16; ++i) zx[i] = L.rowv ? __ldcg(p.Zx + e0 + (size_t)i * LR_ZROW) : 0.0f;
+      mbar_wait(&pdone[L.cg][k & 1], (uint32_t)((k >> 1) & 1));
+      tc_fence_after();
+      tmem_ld16(tlane + (uint32_t)(16 * p.KS + (2 * L.cg + (k & 1)) * 32 + L.rbase), v);
+      tc_fence_before();
+      const float tau = s_tau[j];
+      const float hconst = (p.td && L.hrow == p.H) ? tau : ((L.hrow == p.H + p.td) ? 1.0f : 0.0f);
+      const float pb = p.td ? fmaf(w1t, tau, b1) : b1;
+      const bool last = (!SINGLE && j == 5);
+      float* dst_hh = (SINGLE ? arr(LA_S1 + 3 * slot + 1) : (last ? arr(LA_S1 + 3 * next + 1) : arr(LA_HH + j))) + e0;
+      float* dst_s = arr(LA_SS + j) + e0;
+      float* dst_del = arr(LA_S1 + 3 * slot + 0) + e0;
+      float* dst_alpha = arr(LA_ALPHA + slot) + e0;
 #pragma unroll
-          for (int i = 0; i < 16; ++i) t[k][i] = (k < ns) ? __ldcg(src + (size_t)i * LR_ZROW) : 0.0f;
-        }
-      };
-      float t[3][16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) { v[i] = s_bt[6] * dprev[i]; ss[i] = 0.0f; c[i] = 0.0f; }
-      for (int round = 0; round < 5; ++round) {     // rounds 0, 1: delta_1..6 ; rounds 2..4: H_1..7
-        const int which = round < 2 ? 0 : 1;
-        const int s0 = which ? (round - 2) * 3 : round * 3;
-        const int ns = which ? min(3, 7 - s0) : 3;
-        if (which ? rowc : rowv) {
-          gather3(s0, ns, which, t);
-#pragma unroll
-          for (int k = 0; k < 3; ++k) {
-            const int s = min(s0 + k, 6);
-            const float ct = (k < ns) ? s_bt[s] : 0.0f;
-            const float cb = (k < ns && s < 6) ? d7.coef[s] : 0.0f;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              if (which) { c[i] = fmaf(cb, t[k][i], c[i]); ss[i] = fmaf(ct, t[k][i], ss[i]); }
-              else v[i] = fmaf(ct, t[k][i], v[i]);
-            }
-          }
-        }
-        if (round == 1) {    // Delta_bt complete: stored, and its operand image (tile C is free: p of stage 7 has been read)
-          float* dbt = arr(LA_DBT) + e0;
-#pragma unroll
-          for (int i = 0; i < 16; ++i) dbt[(size_t)i * LR_ZROW] = v[i];
-          tile_put16(tCc, v);
-          fence_proxy_async();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&out_full);
-        }
-      }
-      if (tr) ATRACE(0, 4);
-      float* hbb = arr(LA_HBB) + e0;
-      float* hbt = arr(LA_HBT) + e0;
+      for (int i = 0; i < 16; ++i) v[i] = v[i] + zx[i] + pb;
 #pragma unroll
       for (int i = 0; i < 16; ++i) {
-        hbb[(size_t)i * LR_ZROW] = rowc ? c[i] : 0.0f;
-        hbt[(size_t)i * LR_ZROW] = rowc ? ss[i] : 0.0f;
+        float h, sg;
+        act_pair<ACT>(v[i], h, sg);
+        const float sj = L.rowv ? sg : 0.0f;
+        const float hv = L.rowv ? h : hconst;
+        dst_hh[(size_t)i * LR_ZROW] = hv;
+        if (SINGLE) {   // alpha_1 = alpha_n ; delta_1 = s_1 .* alpha_1
+          const float an = L.rowv ? __ldcg(p.alpha_in + e0 + (size_t)i * LR_ZROW) : 0.0f;
+          dst_del[(size_t)i * LR_ZROW] = sj * an;
+          dst_alpha[(size_t)i * LR_ZROW] = an;
+        } else {
+          dst_s[(size_t)i * LR_ZROW] = sj;
+          hb[i] = fmaf(s_cb[j + 1], hv, hb[i]);
+          ht[i] = fmaf(s_ct[j + 1], hv, ht[i]);
+        }
+      }
+      if (last) {
+        float* hbb = arr(LA_HBB) + e0;
+        float* hbt = arr(LA_HBT) + e0;
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+          hbb[(size_t)i * LR_ZROW] = L.rowc ? hb[i] : 0.0f;
+          hbt[(size_t)i * LR_ZROW] = L.rowc ? ht[i] : 0.0f;
+        }
       }
     }
     tc_fence_before();
   }
   __syncthreads();
-  if (threadIdx.x == 0 && !SINGLE) ATRACE(0, 5);
   if (warp == 1) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
@@ -552,7 +416,246 @@ __global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// (3) pairacc kernel: batch contractions  acc[2a + v] += sum_b P[:, b] (s_v Q_v[:, b])^T  (v = 0, 1) on the tensor cores.
+// (2) chain kernel: the lambda recurrence of the six stages, one MMA round trip per stage and half:
+//       eps_j = sum_i a_ji delta_i -> alpha_j = alpha_n - dt Mh^T eps_j -> delta_j = s_j .* alpha_j
+//     s_j comes from (1) on a bulk-copy ring, the part of eps_{j+1} that is already known is formed while the tensor
+//     core works.  TMEM: [Mh^T hi | Mh^T lo] (8 KS columns each), then one 32-column accumulator per half.
+// ---------------------------------------------------------------------------------------------------------
+constexpr int kTapeBufs = 3;                       // ring of [64 samples][LR_ZROW] tiles of s_j
+constexpr int kTapeBufBytes = kNT * LR_ZROW * 4;   // 32 KB
+struct AChainP {
+  SolveDev* S;
+  const float* Mz;
+  float* ws;
+  size_t zlen;
+  float* hbuf;
+  uint32_t unit_bytes;
+  int H, Kaug, KS, nfull, ntail, passes;
+};
+
+__global__ void __launch_bounds__(kThreads, 1) adj_chain_kernel(AChainP p) {
+  SolveDev* S = p.S;
+  if (S->done) return;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
+  __shared__ uint64_t a_ready, bfull[2], xdone[2], out_full, tfull[kTapeBufs], tempty[kTapeBufs];
+  __shared__ uint32_t tmem_slot;
+  __shared__ LinComb sd[6];
+  __shared__ float s_bt[7];
+  __shared__ int s_slot, s_next;
+
+  const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
+  const int lane = threadIdx.x & 31;
+  const int n0 = blockIdx.x * kNT;
+  constexpr int nst = 6;
+  const uint32_t tileB = (uint32_t)(p.nfull * 8192 + p.ntail * 2048);   // [hi | lo] images of a 32-sample operand tile
+  auto tC = [&](int cg) { return smem + (size_t)cg * tileB; };         // Delta_bt images of the two halves
+  auto tE = [&](int cg) { return smem + (size_t)(2 + cg) * tileB; };   // eps_j images (eps_7 = Delta_b)
+  uint8_t* tbuf = smem + 4 * (size_t)tileB;        // kTapeBufs s_j tiles (tileB is a multiple of 1024)
+
+  if (threadIdx.x == 0) {
+    mbar_init(&a_ready, (uint32_t)kEpiWarps);
+    mbar_init(&out_full, (uint32_t)kEpiWarps);
+    for (int b = 0; b < kTapeBufs; ++b) { mbar_init(&tfull[b], 1u); mbar_init(&tempty[b], (uint32_t)kEpiWarps); }
+    for (int c = 0; c < 2; ++c) {
+      mbar_init(&bfull[c], (uint32_t)(kEpiWarps / 2));
+      mbar_init(&xdone[c], 1u);
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    s_slot = S->slot; s_next = (S->slot + 1) % S->cap;
+  }
+  if (threadIdx.x >= 64 && threadIdx.x < 70) sd[threadIdx.x - 64] = S->st[threadIdx.x - 64];
+  if (threadIdx.x >= 128 && threadIdx.x < 135) s_bt[threadIdx.x - 128] = S->err.coef[threadIdx.x - 128];
+  if (warp == 1) {   // 16 KS + 64 <= 288 columns (KS <= 14)
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(512u)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = tmem_slot;
+  const uint32_t c_acc = tmem_base + (uint32_t)(16 * p.KS);
+  auto arr = [&](int idx) -> float* { return p.ws + (size_t)idx * p.zlen; };
+  const bool tr = (threadIdx.x == 64);
+  if (tr) ATRACE(0, 0);
+
+  if (warp == 0) {
+    // ---------------- s_j in: one whole (padded) tile per stage, bulk-copied onto a ring
+    {
+      constexpr uint32_t bytes = (uint32_t)kTapeBufBytes;
+      for (int it = 0; it < nst; ++it) {
+        const int b = it % kTapeBufs;
+        mbar_wait(&tempty[b], (uint32_t)(((it / kTapeBufs) & 1) ^ 1));
+        if (elect_one_sync()) {
+          mbar_arrive_expect_tx(&tfull[b], bytes);
+          bulk_g2s(tbuf + (size_t)b * kTapeBufBytes, arr(LA_SS + it) + (size_t)n0 * LR_ZROW, bytes, &tfull[b]);
+        }
+        __syncwarp();
+      }
+    }
+    // ---------------- Delta_b / Delta_bt operand images out (units of 16 samples for the lambda GEMM)
+    mbar_wait(&out_full, 0);
+    if (elect_one_sync()) {
+      for (int sg = 0; sg < 4; ++sg) {
+        uint8_t* g = reinterpret_cast<uint8_t*>(p.hbuf) + ((size_t)blockIdx.x * 4 + sg) * p.unit_bytes;
+        const int cg = sg >> 1, half = sg & 1;
+        for (int c = 0; c < p.nfull; ++c)
+          for (int lo = 0; lo < 2; ++lo) {
+            bulk_s2g(g + (size_t)c * 8192 + lo * 4096, tE(cg) + (size_t)c * 8192 + lo * 4096 + half * 2048, 2048);
+            bulk_s2g(g + (size_t)c * 8192 + lo * 4096 + 2048, tC(cg) + (size_t)c * 8192 + lo * 4096 + half * 2048, 2048);
+          }
+        for (int t = 0; t < p.ntail; ++t)
+          for (int lo = 0; lo < 2; ++lo) {
+            const size_t o = (size_t)p.nfull * 8192 + (size_t)t * 2048 + lo * 1024;
+            bulk_s2g(g + o, tE(cg) + o + half * 512, 512);
+            bulk_s2g(g + o + 512, tC(cg) + o + half * 512, 512);
+          }
+      }
+      bulk_commit();
+      bulk_wait0();
+    }
+    __syncwarp();
+  } else if (warp == 1) {
+    // ---------------- tcgen05.mma issue (M = 128 hidden rows x N = 32 samples, A from tensor memory): Mh^T eps_j
+    constexpr uint32_t idesc = make_idesc(128, kNT / 2);
+    mbar_wait(&a_ready, 0);
+    tc_fence_after();
+    const uint32_t mt_hi = tmem_base, mt_lo = tmem_base + (uint32_t)(8 * p.KS);
+    for (int st = 0; st < nst; ++st) {
+      for (int cg = 0; cg < 2; ++cg) {
+        mbar_wait(&bfull[cg], (uint32_t)(st & 1));
+        tc_fence_after();
+        if (elect_one_sync()) {
+          if (cg == 0) ATRACE(7, st);
+          issue_group(c_acc + (uint32_t)(cg * 32), mt_hi, mt_lo, smem_u32(tE(cg)), p.nfull, p.ntail, p.passes, idesc);
+          mma_commit(&xdone[cg]);
+          if (cg == 0) ATRACE(8, st);
+        }
+        __syncwarp();
+      }
+    }
+  } else {
+    // ---------------- compute warps: lane = hidden row, registers = 16 samples
+    const ComputeLane L(warp, lane, p.H, p.Kaug, p.KS, p.nfull);
+    const int cg = L.cg;
+    const uint32_t tlane = tmem_base + ((uint32_t)(L.q * 32) << 16);
+    a_operand_to_tmem(p.Mz, true, p.H, p.KS, p.passes, warp, L.hrow, tlane);
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&a_ready);
+    if (tr) ATRACE(0, 1);
+
+    const bool rowv = L.rowv;
+    const int slot = s_slot, next = s_next;
+    const float dt = sd[0].scale;
+    // element of (first sample, this row) in a [Bpad][LR_ZROW] array (padded to whole tiles: no bounds tests below)
+    const size_t e0 = (size_t)(n0 + cg * 32 + L.rbase) * LR_ZROW + L.hrow;
+    const float* ring_row = reinterpret_cast<const float*>(tbuf) + (cg * 32 + L.rbase) * LR_ZROW + L.hrow;
+
+    const float* alpha_n = arr(LA_ALPHA + slot) + e0;
+    float ep[16], dprev[16], an[16], v[16], ss[16];
+    {
+      const float* d1 = arr(LA_S1 + 3 * slot + 0) + e0;     // delta_1 (FSAL) of the current state
+#pragma unroll
+      for (int i = 0; i < 16; ++i) { ep[i] = 0.0f; dprev[i] = rowv ? __ldcg(d1 + (size_t)i * LR_ZROW) : 0.0f; }
+    }
+    for (int jj = 0; jj < nst; ++jj) {
+      const bool last = (jj == 5);
+      if (tr) ATRACE(1, jj);
+      // ---- operand tile: eps_j = (partial sum prefetched during the previous stage) + a_{j,j-1} delta_{j-1}
+      {
+        const float cl = sd[jj].coef[jj];
+        float* dst_eps = arr(LA_EPS + jj) + e0;
+#pragma unroll
+        for (int i = 0; i < 16; ++i) { v[i] = fmaf(cl, dprev[i], ep[i]); dst_eps[(size_t)i * LR_ZROW] = v[i]; }
+        L.tile_put16(tE(cg), v, p.passes);
+        tc_fence_before();
+        fence_proxy_async();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&bfull[cg]);
+      }
+      if (tr) ATRACE(2, jj);
+      if (jj + 1 < nst) {   // known part of eps_{j+1}: delta_1 .. delta_j (the newest one is in registers)
+#pragma unroll
+        for (int i = 0; i < 16; ++i) ep[i] = sd[jj + 1].coef[jj] * dprev[i];
+        if (rowv) {
+          for (int s = 0; s < jj; ++s) {
+            const float* src = ((s == 0) ? arr(LA_S1 + 3 * slot + 0) : arr(LA_DEL + s - 1)) + e0;
+            const float cf = sd[jj + 1].coef[s];
+#pragma unroll
+            for (int i = 0; i < 16; ++i) ep[i] = fmaf(cf, __ldcg(src + (size_t)i * LR_ZROW), ep[i]);
+          }
+        }
+      }
+      if (tr) ATRACE(3, jj);
+      // ---- alpha_j = alpha_n - dt Mh^T eps_j ; delta_j = s_j .* alpha_j
+#pragma unroll
+      for (int i = 0; i < 16; ++i) an[i] = rowv ? __ldcg(alpha_n + (size_t)i * LR_ZROW) : 0.0f;
+      mbar_wait(&xdone[cg], (uint32_t)(jj & 1));
+      if (tr) ATRACE(6, jj);
+      tc_fence_after();
+      tmem_ld16(c_acc + ((uint32_t)(L.q * 32) << 16) + (uint32_t)(cg * 32 + L.rbase), v);
+      tc_fence_before();
+      // ---- s_j from the ring (read after the MMA wait: not live across it)
+      {
+        const int b = jj % kTapeBufs;
+        mbar_wait(&tfull[b], (uint32_t)((jj / kTapeBufs) & 1));
+        const float* tb = ring_row + (size_t)b * (kTapeBufBytes / 4);
+#pragma unroll
+        for (int i = 0; i < 16; ++i) ss[i] = tb[i * LR_ZROW];
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&tempty[b]);
+      }
+      float* dst_del = (last ? arr(LA_S1 + 3 * next + 0) : arr(LA_DEL + jj)) + e0;
+      float* dst_alpha = arr(LA_ALPHA + next) + e0;
+#pragma unroll
+      for (int i = 0; i < 16; ++i) {
+        const float aj = fmaf(-dt, v[i], an[i]);
+        dprev[i] = ss[i] * aj;
+        dst_del[(size_t)i * LR_ZROW] = dprev[i];
+        if (last) dst_alpha[(size_t)i * LR_ZROW] = rowv ? aj : 0.0f;
+      }
+    }
+    if (tr) ATRACE(0, 3);
+    // ---- Delta_bt = sum_j btilde_j delta_j (stage 7 in registers), three source arrays per round trip
+#pragma unroll
+    for (int i = 0; i < 16; ++i) v[i] = s_bt[6] * dprev[i];
+    if (rowv) {
+      for (int s0 = 0; s0 < 6; s0 += 3) {
+        float t[3][16];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+          const float* src = ((s0 + k == 0) ? arr(LA_S1 + 3 * slot + 0) : arr(LA_DEL + s0 + k - 1)) + e0;
+#pragma unroll
+          for (int i = 0; i < 16; ++i) t[k][i] = __ldcg(src + (size_t)i * LR_ZROW);
+        }
+#pragma unroll
+        for (int k = 0; k < 3; ++k)
+#pragma unroll
+          for (int i = 0; i < 16; ++i) v[i] = fmaf(s_bt[s0 + k], t[k][i], v[i]);
+      }
+    }
+    float* dbt = arr(LA_DBT) + e0;
+#pragma unroll
+    for (int i = 0; i < 16; ++i) dbt[(size_t)i * LR_ZROW] = v[i];
+    L.tile_put16(tC(cg), v, p.passes);
+    fence_proxy_async();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&out_full);
+    if (tr) ATRACE(0, 4);
+    tc_fence_before();
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) ATRACE(0, 5);
+  if (warp == 1) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// (4) pairacc kernel: batch contractions  acc[2a + v] += sum_b P[:, b] (s_v Q_v[:, b])^T  (v = 0, 1) on the tensor cores.
 // Operands are [rows, B] arrays with the rows of a sample contiguous = MN-major for the MMA (same operand images as
 // umma::wgrad_kernel).  Jobs (blockIdx): 0 = the hidden-space terms (P = c_j / H_j, Q = delta_j / eps_j scaled by
 // b_j and btilde_j; 4 accumulators), 1 = x (Delta_b, Delta_bt)^T per 128-feature tile, 2 = lambda_n (HB_b, HB_bt)^T.
@@ -782,7 +885,7 @@ __global__ void __launch_bounds__(kThreads, 1) pairacc_kernel(PairAccP q) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// (4) fixed-order reduction of the partial blocks, then the mu block of the attempt
+// (5) fixed-order reduction of the partial blocks, then the mu block of the attempt
 // ---------------------------------------------------------------------------------------------------------
 struct AReduceP {
   SolveDev* S;
@@ -995,7 +1098,7 @@ LatentAdjoint::LatentAdjoint(lrnde_ctx* c, const lrnde_model* mm, const float* p
     : ctx(c), m(mm), ps(p), B(b), passes(npasses) {
   lrf_shape(m, &sh);
   ntiles = (int)((B + fused::kNT - 1) / fused::kNT);
-  zlen = (size_t)LR_ZROW * (size_t)ntiles * fused::kNT;   // work arrays padded to whole 64-sample tiles (adj_chain_kernel)
+  zlen = (size_t)LR_ZROW * (size_t)ntiles * fused::kNT;   // work arrays padded to whole 64-sample tiles (adj_pre_kernel)
   nunits = (int)((B + 15) / 16);
   unit_bytes = (size_t)sh.nfull * 8192 + (size_t)sh.ntail * 2048;
   const int maxc = std::max(1, 148 / sh.n_mt);
@@ -1023,19 +1126,21 @@ LatentAdjoint::LatentAdjoint(lrnde_ctx* c, const lrnde_model* mm, const float* p
   RP = (float*)ctx->alloc(sizeof(float) * 4 * 16384);
   RX = (float*)ctx->alloc(sizeof(float) * (size_t)ntile_d * 2 * 16384);
   RL = (float*)ctx->alloc(sizeof(float) * (size_t)ntile_d * 2 * 16384);
+  int dev = 0, nsm = 0;
+  LR_CUDA(cudaGetDevice(&dev));
+  LR_CUDA(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev));
+  pre_ctas = std::max(1, std::min(ntiles, nsm));
   static bool attr_set = false;
   if (!attr_set) {
-    constexpr int kChainSmem = 4 * (3 * 8192 + 3 * 2048) + ladj::kTapeBufs * ladj::kTapeBufBytes + 1024;   // KS <= 14: at most 3 full chunks + 3 tail K-steps
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_IDENTITY, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_IDENTITY, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_TANH, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_TANH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_GELU, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_GELU, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_SIGMOID, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_SIGMOID, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_RELU, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
-    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel<ACT_RELU, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
+    // KS <= 14: at most 3 full chunks + 3 tail K-steps per operand tile
+    constexpr int kTiles4 = 4 * (3 * 8192 + 3 * 2048);
+    constexpr int kChainSmem = kTiles4 + ladj::kTapeBufs * ladj::kTapeBufBytes + 1024, kPreSmem = kTiles4 + 1024;
+    LR_CUDA(cudaFuncSetAttribute(ladj::adj_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmem));
+#define LRA_PRE_ATTR(A) do { \
+      LR_CUDA(cudaFuncSetAttribute(ladj::adj_pre_kernel<A, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPreSmem)); \
+      LR_CUDA(cudaFuncSetAttribute(ladj::adj_pre_kernel<A, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPreSmem)); } while (0)
+    LRA_PRE_ATTR(ACT_IDENTITY); LRA_PRE_ATTR(ACT_TANH); LRA_PRE_ATTR(ACT_GELU); LRA_PRE_ATTR(ACT_SIGMOID); LRA_PRE_ATTR(ACT_RELU);
+#undef LRA_PRE_ATTR
     LR_CUDA(cudaFuncSetAttribute(ladj::pairacc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ladj::pairacc_smem()));
     attr_set = true;
   }
@@ -1056,36 +1161,48 @@ void LatentAdjoint::prepare(const float* mz_plain) {
   LRA_COUNT(ctx);
 }
 
+// (0) interpolant, (1) pre kernel and, for an attempt, (2) the chain kernel; single: stage 1 of the current state only
 static void lra_launch_chain(LatentAdjoint& E, SolveDev* S, int single) {
   const FusedShape& sh = E.sh;
   const LayerInfo& L1 = E.m->layers[0];
-  ladj::AChainP cp;
-  memset(&cp, 0, sizeof(cp));
-  cp.S = S; cp.single = single; cp.Mz = E.Mz_ext ? E.Mz_ext : E.Mz;
-  cp.w1t = sh.td ? E.ps + L1.w_off + (size_t)sh.D * sh.H : nullptr;
-  cp.b1 = E.ps + L1.b_off;
-  cp.Zx = E.Zx; cp.alpha_in = E.alpha_in; cp.ws = E.ws; cp.zlen = E.zlen;
-  cp.hbuf = E.hbuf; cp.unit_bytes = (uint32_t)E.unit_bytes;
-  cp.B = (int)E.B; cp.H = sh.H; cp.td = sh.td; cp.Kaug = sh.Kaug; cp.KS = sh.KS; cp.nfull = sh.nfull; cp.ntail = sh.ntail;
-  cp.passes = E.passes;
-  const size_t smem_c = 4 * ((size_t)sh.nfull * 8192 + (size_t)sh.ntail * 2048) + ladj::kTapeBufs * ladj::kTapeBufBytes + 1024;
+  const float* Mz = E.Mz_ext ? E.Mz_ext : E.Mz;
+  const size_t tiles4 = 4 * ((size_t)sh.nfull * 8192 + (size_t)sh.ntail * 2048);
   cudaStream_t st = E.ctx->stream;
   ladj::AInterpP ip;
   ip.S = S; ip.single = single; ip.ws = E.ws; ip.zlen = E.zlen; ip.B = (int)E.B; ip.Kaug = sh.Kaug;
   ip.nunit = E.ntiles * fused::kNT * (LR_ZROW / 4);
   ladj::adj_interp_kernel<<<(ip.nunit + 255) / 256, 256, 0, st>>>(ip);
   LRA_COUNT(E.ctx);
-#define LRA_CHAIN(A) do { if (single) ladj::adj_chain_kernel<A, true><<<E.ntiles, fused::kThreads, smem_c, st>>>(cp); \
-                         else ladj::adj_chain_kernel<A, false><<<E.ntiles, fused::kThreads, smem_c, st>>>(cp); } while (0)
+  ladj::APreP pp;
+  memset(&pp, 0, sizeof(pp));
+  pp.S = S; pp.Mz = Mz;
+  pp.w1t = sh.td ? E.ps + L1.w_off + (size_t)sh.D * sh.H : nullptr;
+  pp.b1 = E.ps + L1.b_off;
+  pp.Zx = E.Zx; pp.alpha_in = E.alpha_in; pp.ws = E.ws; pp.zlen = E.zlen;
+  pp.H = sh.H; pp.td = sh.td; pp.Kaug = sh.Kaug; pp.KS = sh.KS; pp.nfull = sh.nfull; pp.ntail = sh.ntail;
+  pp.passes = E.passes; pp.ntiles = E.ntiles;
+  const size_t smem_p = tiles4 + 1024;
+#define LRA_PRE(A) do { if (single) ladj::adj_pre_kernel<A, true><<<E.pre_ctas, fused::kThreads, smem_p, st>>>(pp); \
+                       else ladj::adj_pre_kernel<A, false><<<E.pre_ctas, fused::kThreads, smem_p, st>>>(pp); } while (0)
   switch (sh.act) {
-    case ACT_TANH: LRA_CHAIN(ACT_TANH); break;
-    case ACT_GELU: LRA_CHAIN(ACT_GELU); break;
-    case ACT_SIGMOID: LRA_CHAIN(ACT_SIGMOID); break;
-    case ACT_RELU: LRA_CHAIN(ACT_RELU); break;
-    default: LRA_CHAIN(ACT_IDENTITY); break;
+    case ACT_TANH: LRA_PRE(ACT_TANH); break;
+    case ACT_GELU: LRA_PRE(ACT_GELU); break;
+    case ACT_SIGMOID: LRA_PRE(ACT_SIGMOID); break;
+    case ACT_RELU: LRA_PRE(ACT_RELU); break;
+    default: LRA_PRE(ACT_IDENTITY); break;
   }
-#undef LRA_CHAIN
+#undef LRA_PRE
   LRA_COUNT(E.ctx);
+  if (!single) {
+    ladj::AChainP cp;
+    memset(&cp, 0, sizeof(cp));
+    cp.S = S; cp.Mz = Mz; cp.ws = E.ws; cp.zlen = E.zlen;
+    cp.hbuf = E.hbuf; cp.unit_bytes = (uint32_t)E.unit_bytes;
+    cp.H = sh.H; cp.Kaug = sh.Kaug; cp.KS = sh.KS; cp.nfull = sh.nfull; cp.ntail = sh.ntail; cp.passes = E.passes;
+    const size_t smem_c = tiles4 + ladj::kTapeBufs * ladj::kTapeBufBytes + 1024;
+    ladj::adj_chain_kernel<<<E.ntiles, fused::kThreads, smem_c, st>>>(cp);
+    LRA_COUNT(E.ctx);
+  }
   LR_CUDA(cudaGetLastError());
 }
 

@@ -13,12 +13,15 @@
 //                     sum_j w_j dW2a_j = lambda_n (sum_j w_j [h_j;tau_j;1])^T - dt W1^T (sum_j w_j eps_j [h_j;tau_j;1]^T)
 // so an attempt touches D-dimensional data only to read lambda_n and x and to write lambda_{n+1}:
 //   (0) adj_interp_kernel  c_j of the six stages from the forward hidden tape (lambda-independent: one pass over the
-//                          whole batch, one read of each forward interval's tape per attempt), stored for (1) and (3)
-//   (1) adj_chain_kernel   the six stages in hidden space (tcgen05, Mz / Mh^T as TMEM A operands; c_j from (0))
-//   (2) kgemm_kernel<2,1>  [W1^T Delta_b, W1^T Delta_bt] with the lambda_{n+1} / residual epilogue (lrnde_fused.cu)
-//   (3) pairacc_kernel     every batch contraction of the mu block (tcgen05, MN-major operands, split over the batch)
-//   (4) adj_reduce_kernel + adj_mu_kernel   fixed-order reduction, mu_{n+1}, residual of the mu block
-//   (5) controller_kernel  (unchanged)
+//                          whole batch, one read of each forward interval's tape per attempt), stored for (1) and (4)
+//   (1) adj_pre_kernel     the rest of the lambda-independent stage work over the whole batch: p_j = Zx + Mz c_j + ...
+//                          (tcgen05, Mz as TMEM A operand), [h_j;tau_j;1], s_j and the sums sum_j w_j [h_j;tau_j;1]
+//   (2) adj_chain_kernel   the lambda recurrence of the six stages in hidden space: one Mh^T eps_j MMA round trip per
+//                          stage (tcgen05, Mh^T as TMEM A operand; s_j from (1))
+//   (3) kgemm_kernel<2,1>  [W1^T Delta_b, W1^T Delta_bt] with the lambda_{n+1} / residual epilogue (lrnde_fused.cu)
+//   (4) pairacc_kernel     every batch contraction of the mu block (tcgen05, MN-major operands, split over the batch)
+//   (5) adj_reduce_kernel + adj_mu_kernel   fixed-order reduction, mu_{n+1}, residual of the mu block
+//   (6) controller_kernel  (unchanged)
 #pragma once
 #include "lrnde_fused.h"
 
@@ -31,6 +34,7 @@ struct LatentAdjoint {
   FusedShape sh;
   size_t zlen = 0;
   int ntiles = 0, nunits = 0, nclusters = 1;
+  int pre_ctas = 1;           // adj_pre_kernel: CTAs (one per SM), each takes whole 64-sample tiles
   int ntile_d = 0;            // 128-row feature tiles of a [D, B] array
   int nP = 1, chunkP = 32;    // pairacc: CTAs / samples per CTA of the hidden-space terms
   int nD = 1, chunkD = 32;    // pairacc: batch splits / samples per split of the D-dimensional terms
@@ -50,10 +54,11 @@ struct LatentAdjoint {
   LatentAdjoint(lrnde_ctx* c, const lrnde_model* mm, const float* p, int64_t b, int npasses);
   ~LatentAdjoint();
   void prepare(const float* mz_plain = nullptr);
-  // stage-1 quantities (delta_1, [h_1;t;1], c_1) of the current state from alpha_in and S->yint[0]
+  // stage-1 quantities (delta_1, [h_1;t;1], c_1, alpha) of the current state from alpha_in and S->yint[0]: (0), (1)
   void begin(SolveDev* S);
-  // one Tsit5 attempt of the adjoint from the descriptors of S (st, yint, err): launches (0) - (4)
+  // one Tsit5 attempt of the adjoint from the descriptors of S (st, yint, err): launches (0) - (5)
   void attempt(SolveDev* S);
-  // profiling: the launches of attempt() one by one (0 interpolant + chain, 1 lambda GEMM, 2 pairacc, 3 reduce + mu)
+  // profiling: the launches of attempt() one by one (0 interpolant + pre + chain, 1 lambda GEMM, 2 pairacc,
+  // 3 reduce + mu)
   void attempt_part(SolveDev* S, int which);
 };

@@ -18,7 +18,7 @@ buf = (C.c_longlong * 1024)()
 L.lrnde_debug_trace_adj(buf, 1024)
 a = np.array(buf[:]).reshape(64, 16)
 t0 = a[0, 0]
-names = ["misc[start,A in TMEM,c0 done,stages done,dbt done,end]", "stage top", "tiles written", "prefetch done", "p ready",
-         "act done", "xi ready", "mma1 issue", "mma1 issued", "cc stored", "tile C put", "eps stored+put"]
+names = ["misc[start,A in TMEM,-,stages done,dbt done,end]", "stage top", "eps tile put", "prefetch done", "-", "-",
+         "xi ready", "mma issue", "mma issued"]
 for i, nm in enumerate(names):
     print(f"{nm:56s}", " ".join(f"{int(v - t0):7d}" if v else "      ." for v in a[i][:6]))
